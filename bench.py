@@ -2,6 +2,7 @@
 """Benchmark of the B200-native neural_raytracing hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision f16|bf16|f32]
+                    [--dump-outputs DIR]
 
 Workload at N = 1 (BASELINE.json configs[1]): nerf_synthetic-shape NeRF volumetric render, 800x800 rays,
 64 coarse + 128 importance-resampled fine samples per ray, random-init NeRFLE-architecture MLPs
@@ -23,6 +24,18 @@ Prints ONE JSON line (rank 0):
 
 `--impl reference` times only that CPU restatement (the reference is pure Python/PyTorch and does
 not exist on the GPU box; oracle/ is its pinned restatement) and prints the same line shape.
+
+`--steps K` is the number of timed steps behind `value` and `ms_per_step`.  The secondary legs pick their own counts:
+`e2e` (and `e2e.from_camera`) times max(3, min(K, 10)) steps; at N > 1 the eager per-kernel split and
+`single_gpu_same_run` time max(3, K // 2) steps; the configs under `also` and the 4K render have fixed counts.
+
+`--dump-outputs DIR` writes what the last timed step computed, float32, once per run:
+  N = 1   rgb.npy     the radiance of the frame, [640000, 3]
+  N > 1   loss.npy    the loss of rank 0's slice; grad.npy the all-reduced flat gradient and params.npy the flat
+                      parameters after the AdamW update (both in the layout of training.FlatParameters)
+The inputs are fixed by seeds, so two builds run with the same arguments can be compared output for output: the
+render is reproducible bit for bit; the training step's weight gradients are accumulated with atomics, so its outputs
+agree from run to run only to the order of fp32 summation (about 1e-3 of the largest element).
 """
 import argparse
 import json
@@ -846,8 +859,15 @@ def run_multi_gpu(args, rank, world, local_rank):
     barrier()
 
     # ---- the headline: K timed steps, barrier + synchronize on both sides, CUDA events, max over ranks ----
-    ms = max_over_ranks(_time_steps(torch, tb.step, args.steps, args.warmup, barrier))
+    last = [None]
+
+    def timed_step():
+        last[0] = tb.step()
+    ms = max_over_ranks(_time_steps(torch, timed_step, args.steps, args.warmup, barrier))
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss=last[0], grad=tb.flat.grad, params=tb.flat.flat)
+    del last
     # per-kernel split: the library's event brackets do not fire inside a graph replay, so the same step is also run
     # eagerly (its kernels are the ones the graph holds)
     n_eager = max(3, args.steps // 2)
@@ -1048,26 +1068,41 @@ def ncu_traffic():
     return None
 
 
+def dump_outputs(directory, **arrays):
+    """Writes each tensor as DIR/<name>.npy in float32."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline number (value, ms_per_step); the secondary legs pick their own counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--precision", default="f16", choices=["f16", "bf16", "f32"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the supplementary configs reported under `also`")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    multi_gpu = world > 1 or os.environ.get("NRT_BENCH_FORCE_CFG5") == "1"     # (the env switch is a development aid)
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference arm times a sample of the rays only")
 
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
-    if world > 1 or os.environ.get("NRT_BENCH_FORCE_CFG5") == "1":     # (the env switch is a development aid)
+    if multi_gpu:
         run_multi_gpu(args, rank, world, local_rank)
         return
 
@@ -1109,8 +1144,9 @@ def main():
 
     sampler = ClockSampler(local_rank)
     sampler.start()            # nvidia-smi needs ~1 s to come up: start it before the warm-up
+    # the warm-up also keeps each step's rgb alive until the next one returns, so the timed loop reuses cached blocks
     for _ in range(args.warmup):
-        step()
+        rgb = step()
     barrier()
     ops.profile_collect()
     ops.profile_enable(True)
@@ -1119,12 +1155,15 @@ def main():
     for a, b in evs:
         flush.zero_()          # L2 flush, outside the event bracket
         a.record()
-        step()
+        rgb = step()
         b.record()
     barrier()
     clocks = sampler.stop()
     prof = ops.profile_collect()
     ops.profile_enable(False)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rgb=rgb)
+    del rgb
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
     if world > 1:

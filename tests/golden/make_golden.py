@@ -183,7 +183,8 @@ def gen_nerfle():
 
 def gen_nerfle_train():
     """nerfle.py:104-116-style step on the UNMODIFIED reference: NeRFLE forward -> mse -> backward.  Stores the loss and
-    the gradient of every Linear (flattened in module order) for the point-light and the environment-light model."""
+    the gradient of every Linear (flattened in module order, synth.pack_grad, with its float64 norm as `<key>_norm`)
+    for the point-light and the environment-light model."""
     out = {}
     random.random = lambda: FIXED_RANDOM
     for tag, envmap in (("pt", False), ("le", True)):
@@ -208,13 +209,16 @@ def gen_nerfle_train():
         out[tag + "_rgb"] = rgb.detach().numpy()
         for name, mod in (("first", n.first), ("second", n.second)):
             lins = [mod.init] + list(mod.layers) + [mod.out]
-            out["%s_g_%s_w" % (tag, name)] = np.concatenate([l.weight.grad.numpy().ravel() for l in lins])
-            out["%s_g_%s_b" % (tag, name)] = np.concatenate([l.bias.grad.numpy().ravel() for l in lins])
+            for kind in ("w", "b"):
+                key = "%s_g_%s_%s" % (tag, name, kind)
+                grad = np.concatenate([(l.weight if kind == "w" else l.bias).grad.numpy().ravel() for l in lins])
+                out[key], out[key + "_scale"] = synth.pack_grad(grad)
+                out[key + "_norm"] = np.array(np.linalg.norm(grad.astype(np.float64)), np.float64)
     out["fixed_random"] = np.array(FIXED_RANDOM, np.float64)
     out["src"] = np.array("shapes/nerf.py:175-214 NeRFLE.forward + torch autograd of F.mse_loss (scripts/nerfle.py:113-116)")
     np.savez_compressed(os.path.join(HERE, "nerfle_train.npz"), **out)
     print("nerfle_train.npz: loss pt %.6f le %.6f, |g first| %.3e" % (out["pt_loss"], out["le_loss"],
-                                                                      np.linalg.norm(out["pt_g_first_w"])))
+                                                                      out["pt_g_first_w_norm"]))
 
 
 def gen_composite():
@@ -660,7 +664,7 @@ def gen_dtu16():
     (training_utils.py:385-405) -- pathtrace_sample, masked_loss(mask_weight=10) + eikonal_loss(raw_normals) --
     forward and backward.  The SSIM term of masked_loss comes from the absent, unpinned pytorch_msssim: it is patched
     to the constant 1 (-log 1 = 0) for the run, i.e. "masked_loss without SSIM" (SURVEY 8d cfg4).  Gradients are kept
-    as scenes.grad_block() of every parameter tensor."""
+    as scenes.grad_block() of every parameter tensor, stored with synth.pack_grad."""
     import pytorch3d.pathtracer as P
     import pytorch3d.pathtracer.utils as RU
     import pytorch3d.pathtracer.shapes.sdfs, pytorch3d.pathtracer.bsdf, pytorch3d.pathtracer.lights  # noqa: F401
@@ -694,7 +698,7 @@ def gen_dtu16():
         for pname, p in mod.named_parameters():
             assert p.grad is not None, (gname, pname)
             key = "g_%s.%s" % (gname, pname)
-            out[key] = scenes.grad_block(p.grad).numpy().copy()
+            out[key], out[key + "_scale"] = synth.pack_grad(scenes.grad_block(p.grad).numpy())
             out["n_" + key[2:]] = np.array(float(p.grad.norm()), np.float64)
             names.append(key)
     out["g_reflectance"] = np.stack([b.reflectance.grad.numpy() for b in bsdf.bsdfs[10:]])

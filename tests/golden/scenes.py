@@ -109,5 +109,6 @@ def dtu_targets(n_views, crop, device="cpu"):
 
 def grad_block(t):
     """The part of a gradient tensor the fixtures keep: the first 16 output rows of a weight matrix, everything of a
-    vector / small tensor (keeps the dtu16 fixture at ~1 MB; every kept element is an independent check)."""
+    vector / small tensor (with synth.pack_grad this keeps the dtu16 fixture under 1 MB; every kept element is an
+    independent check)."""
     return t[:16] if t.dim() == 2 and t.shape[0] > 16 else t

@@ -122,3 +122,20 @@ class GoldenRatioSampler:
         i = torch.arange(n, dtype=torch.float64) + 1 + 977 * self.calls
         self.calls += 1
         return ((i * 0.6180339887498949) % 1.0).float().reshape(tuple(shape)).to(device)
+
+
+def pack_grad(x):
+    """A reference gradient as float16 times a power-of-two float32 scale (stored as `<key>` and `<key>_scale`): every
+    element is kept, at half the bytes of float32, so the gradient fixtures stay under 1 MB.  The scale maps the largest
+    magnitude into [2**14, 2**15]: every element above 2**-29 of it keeps 11 significant bits (relative error <= 2**-11),
+    smaller ones lose precision down to zero, and decoding is exact.  On the stored reference gradients this moves every
+    cosine (whole vector and per tensor) by less than 1e-7; the norm checks use norms stored in float64."""
+    x = np.asarray(x, np.float32)
+    m = float(np.abs(x).max()) if x.size else 0.0
+    scale = np.float32(2.0 ** (int(np.ceil(np.log2(m))) - 15)) if m > 0 else np.float32(1.0)
+    return (x / scale).astype(np.float16), scale
+
+
+def unpack_grad(g, key):
+    """float64 value of a gradient stored with pack_grad."""
+    return g[key].astype(np.float64) * float(g[key + "_scale"])

@@ -88,7 +88,7 @@ def fixture_cosines():
             for name, mod in (("first", n.first), ("second", n.second)):
                 lins = [mod.init] + list(mod.layers) + [mod.out]
                 for kind in ("w", "b"):
-                    ref_all = g["%s_g_%s_%s" % (tag, name, kind)].astype(np.float64)
+                    ref_all = synth.unpack_grad(g, "%s_g_%s_%s" % (tag, name, kind))
                     got_all = torch.cat([(l.weight if kind == "w" else l.bias).grad.reshape(-1) for l in lins]).cpu().numpy().astype(np.float64)
                     cos = float(got_all @ ref_all / (np.linalg.norm(got_all) * np.linalg.norm(ref_all)))
                     # per tensor
