@@ -170,6 +170,14 @@ int nrt_nerfle_train_forward(const nrt_mlp_t* first, const nrt_mlp_t* second, in
                              const int32_t* view_of_ray, float* sigma, float* rgb, float* latent,
                              void* ws_first, size_t ws_first_bytes, void* ws_second, size_t ws_second_bytes,
                              void* stream);
+/* The same forward with per-sample distances ts [S,R] (sample m = s * R + ray at distance ts[m]), e.g. the merged
+ * coarse + fine distances of nrt_nerfle_sample_hierarchical.  Extension: the reference uses one shared ts (nerf.py:178).
+ * The backward is nrt_nerfle_train_backward unchanged (it needs no distances). */
+int nrt_nerfle_train_forward_ts(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                int64_t R, const float* ts, int S, const float* light_code, int light_dim,
+                                const int32_t* view_of_ray, float* sigma, float* rgb, float* latent,
+                                void* ws_first, size_t ws_first_bytes, void* ws_second, size_t ws_second_bytes,
+                                void* stream);
 int nrt_nerfle_train_backward(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, int64_t R, int S,
                               int light_dim, const float* rgb, const float* g_sigma, const float* g_rgb,
                               const void* dgrad_blob_first, const void* dgrad_blob_second, void* ws_first,
@@ -252,6 +260,16 @@ int nrt_composite_forward(const float* sigma_raw, const float* rgb, const float*
 int nrt_composite_backward(const float* sigma_raw, const float* rgb, const float* ts, int S,
                            int64_t R, const float* g_out, float* g_sigma_raw, float* g_rgb,
                            void* stream);
+/* The same pair with per-sample distances ts [S,R] (sample s of ray r at ts[s*R + r]; the hierarchical samples of
+ * nrt_nerfle_sample_hierarchical), keeping every quirk above (nerf.py:205-213): alpha from the absolute t, the
+ * roll-by-one that gives sample 0 the total transmittance, the last transmittance forced to 1, and a backward built
+ * from suffix recurrences without dividing by the clamped 1 - alpha.  With ts[s*R + r] = ts_shared[s] the results
+ * equal nrt_composite_forward / _backward bit for bit. */
+int nrt_composite_forward_ts(const float* sigma_raw, const float* rgb, const float* ts, int S,
+                             int64_t R, float* out, void* stream);
+int nrt_composite_backward_ts(const float* sigma_raw, const float* rgb, const float* ts, int S,
+                              int64_t R, const float* g_out, float* g_sigma_raw, float* g_rgb,
+                              void* stream);
 
 /* ---- a18: NeRFLE.forward fused volumetric render (nerf.py:175-214) ------------------- */
 /* rays [R,6]; ts [S] sample distances (the reference uses linspace(0, 2+U*0.1, 64));
@@ -272,6 +290,25 @@ int nrt_nerfle_render(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
                       void* workspace, size_t workspace_bytes, void* stream);
 size_t nrt_nerfle_render_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
                                    int64_t R, const nrt_nerf_sampling_t* sampling);
+/* Hierarchical sample distances for TRAINING on what nrt_nerfle_render renders (extension of nerf.py:178, which uses
+ * one shared uniform ts; the render's hierarchical mode is pinned by oracle/port.py): the first half of that render --
+ * stratified coarse distances in [t_near, t_far), the coarse pass keeping per-sample sigma (at `prec`), inverse-CDF
+ * resampling of n_fine distances -- then the coarse and fine lists merged in ascending order (coarse first on ties, as
+ * the render's merged compositing orders them) into ts_out [n_coarse + n_fine, R], SAMPLE-major (m = s * R + ray, the
+ * layout of nrt_nerfle_train_forward_ts and nrt_composite_forward_ts).  n_fine = 0 is the render's single stratified
+ * pass: ts_out is the stratified distances, no coarse pass runs.  Needs n_coarse >= 1 (>= 3 when n_fine > 0),
+ * n_coarse + n_fine <= NRT_MAX_HIER_SAMPLES and t_near < t_far.
+ * seed_dev: a device uint64 read by the kernels in place of sampling->jitter_seed (NULL: use jitter_seed), so that a
+ * CUDA-graph replay draws new jitter after the caller advanced it; 0 means no jitter (bin centres, u = 0.5).
+ * Jitter is hashed with the ray's index in the call, so equal seeds give the distances of nrt_nerfle_render.
+ * workspace: nrt_nerfle_sample_hierarchical_workspace bytes (256-byte aligned). */
+#define NRT_MAX_HIER_SAMPLES 512
+size_t nrt_nerfle_sample_hierarchical_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
+                                                int64_t R, const nrt_nerf_sampling_t* sampling);
+int nrt_nerfle_sample_hierarchical(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                   int64_t R, const nrt_nerf_sampling_t* sampling, const uint64_t* seed_dev,
+                                   const float* light_code, int light_dim, const int32_t* view_of_ray,
+                                   float* ts_out, void* workspace, size_t workspace_bytes, void* stream);
 /* Host-buffer variant: copies rays H2D, renders, copies rgb D2H, synchronises. */
 int nrt_nerfle_render_host(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
                            const float* rays_host, int64_t R, const float* ts_host, int S,

@@ -13,6 +13,7 @@ ACT_LEAKY_RELU, ACT_SOFTPLUS = 0, 1
 OUT_NONE, OUT_SIGMOID, OUT_SOFTPLUS, OUT_TANH = 0, 1, 2, 3
 PREC_F32, PREC_F16, PREC_BF16 = 0, 1, 2
 MAX_LAYERS = 20
+MAX_HIER_SAMPLES = 512     # NRT_MAX_HIER_SAMPLES: n_coarse + n_fine the merge kernels hold in shared memory
 
 c_int, c_i64, c_f32, c_f64, c_vp, c_sz = (ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_double,
                                           ctypes.c_void_p, ctypes.c_size_t)
@@ -86,6 +87,8 @@ SIGNATURES = {
     "nrt_mlp_backward_tc": (c_int, [_PM, c_int, c_int, c_i64, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp, c_vp, c_vp]),
     "nrt_nerfle_train_forward": (c_int, [_PM, _PM, c_int, c_vp, c_i64, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp,
                                          c_vp, c_sz, c_vp, c_sz, c_vp]),
+    "nrt_nerfle_train_forward_ts": (c_int, [_PM, _PM, c_int, c_vp, c_i64, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp,
+                                            c_vp, c_sz, c_vp, c_sz, c_vp]),
     "nrt_nerfle_train_backward": (c_int, [_PM, _PM, c_int, c_i64, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                           c_vp, c_vp, c_vp, c_vp]),
     "nrt_sdf_eval": (c_int, [_PS, c_int, c_vp, c_i64, c_vp, c_vp]),
@@ -102,8 +105,13 @@ SIGNATURES = {
     "nrt_sdf_min_scan": (c_int, [_PS, c_int, c_vp, c_i64, c_f64, c_int, c_vp, c_vp, c_vp, c_vp]),
     "nrt_composite_forward": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),
     "nrt_composite_backward": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_vp]),
+    "nrt_composite_forward_ts": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp]),
+    "nrt_composite_backward_ts": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "nrt_nerfle_render": (c_int, [_PM, _PM, c_int, c_vp, c_i64, c_vp, _PN, c_vp, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "nrt_nerfle_render_workspace": (c_sz, [_PM, _PM, c_int, c_i64, _PN]),
+    "nrt_nerfle_sample_hierarchical_workspace": (c_sz, [_PM, _PM, c_int, c_i64, _PN]),
+    "nrt_nerfle_sample_hierarchical": (c_int, [_PM, _PM, c_int, c_vp, c_i64, _PN, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_sz,
+                                               c_vp]),
     "nrt_nerfle_render_host": (c_int, [_PM, _PM, c_int, c_vp, c_i64, c_vp, c_int, _PN, c_vp, c_int, c_vp, c_vp]),
     "nrt_camera_rays": (c_int, [_PC, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "nrt_set_camera_rays_mode": (c_int, [c_int]),

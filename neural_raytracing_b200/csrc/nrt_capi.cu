@@ -171,7 +171,7 @@ static const char* kTagNames[TAG_COUNT] = {
     "composite_fwd", "composite_bwd", "mlp_tc_nerf_first", "mlp_tc_nerf_second", "mlp_tc_generic", "mlp_tc_pack",
     "stratified_ts", "sample_pdf", "merge_composite", "mlp_bwd_f32", "sdf_value_grad_f32", "shade",
     "sdf_eval_tc", "sdf_march_tc", "sdf_shadow_tc", "sdf_min_scan_tc", "mlp_tc_train_fwd", "mlp_tc_dgrad",
-    "mlp_tc_wgrad", "mlp_tc_wide", "camera_rays"};
+    "mlp_tc_wgrad", "mlp_tc_wide", "camera_rays", "merge_ts", "composite_ts_fwd", "composite_ts_bwd"};
 static std::mutex g_prof_mu;
 static long long g_launches[TAG_COUNT] = {0};
 static bool g_prof_on = false;

@@ -78,7 +78,7 @@ enum NrtTag {
   TAG_COMPOSITE_FWD, TAG_COMPOSITE_BWD, TAG_TC_NERF_FIRST, TAG_TC_NERF_SECOND, TAG_TC_MLP, TAG_TC_PACK,
   TAG_STRATIFIED_TS, TAG_SAMPLE_PDF, TAG_MERGE_COMPOSITE, TAG_MLP_BWD_F32, TAG_SDF_GRAD_F32, TAG_SHADE,
   TAG_TC_SDF_EVAL, TAG_TC_MARCH, TAG_TC_SHADOW, TAG_TC_MIN_SCAN, TAG_TC_TRAIN_FWD, TAG_TC_DGRAD, TAG_TC_WGRAD, TAG_TC_MLP_WIDE,
-  TAG_CAMERA_RAYS, TAG_COUNT
+  TAG_CAMERA_RAYS, TAG_MERGE_TS, TAG_COMPOSITE_TS_FWD, TAG_COMPOSITE_TS_BWD, TAG_COUNT
 };
 void nrt_prof_begin(int tag, cudaStream_t st);
 void nrt_prof_end(int tag, cudaStream_t st);

@@ -462,6 +462,14 @@ k_nerfle(MlpDev m1, MlpDev m2, NerfArgs a) {
 // a19 standalone: compositing over materialised sample-major sigma/rgb (HBM-bound).
 // One thread per ray walks the samples front to back; reads are coalesced across rays.
 // ------------------------------------------------------------------------------------------
+// PER_RAY: ts is [S,R] (one distance per sample, nrt_composite_forward_ts) instead of the shared [S]; the arithmetic is
+// the same, so equal distances give equal bits.
+template <bool PER_RAY>
+__device__ __forceinline__ float comp_t(const float* __restrict__ ts, int s, int64_t R, int64_t r) {
+  return PER_RAY ? __ldg(ts + (int64_t)s * R + r) : __ldg(ts + s);
+}
+
+template <bool PER_RAY>
 __global__ void k_composite_fwd(const float* __restrict__ sigma_raw, const float* __restrict__ rgb,
                                 const float* __restrict__ ts, int S, int64_t R, float* __restrict__ out) {
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -470,7 +478,7 @@ __global__ void k_composite_fwd(const float* __restrict__ sigma_raw, const float
   float a0 = 0.f, r0 = 0.f, g0 = 0.f, b0 = 0.f;
   for (int s = 0; s < S; ++s) {
     const float sigma = fmaxf(__ldg(sigma_raw + (int64_t)s * R + r), 0.0f);
-    const float alpha = 1.0f - nrt_expf(-sigma * __ldg(ts + s));
+    const float alpha = 1.0f - nrt_expf(-sigma * comp_t<PER_RAY>(ts, s, R, r));
     const float* c = rgb + ((int64_t)s * R + r) * 3;
     const float cr = __ldg(c), cg = __ldg(c + 1), cb = __ldg(c + 2);
     if (s == 0) { a0 = alpha; r0 = cr; g0 = cg; b0 = cb; }
@@ -495,6 +503,7 @@ __global__ void k_composite_fwd(const float* __restrict__ sigma_raw, const float
 // both built back to front without dividing by x (which may be 1e-10).  The clamp passes
 // gradient where 1-a >= 1e-10 and the relu where raw > 0 (torch semantics).  g_sigma doubles
 // as scratch for P_{s-1} between the forward and the backward sweep.
+template <bool PER_RAY>
 __global__ void k_composite_bwd(const float* __restrict__ sigma_raw, const float* __restrict__ rgb,
                                 const float* __restrict__ ts, int S, int64_t R,
                                 const float* __restrict__ g_out, float* __restrict__ g_sigma,
@@ -508,7 +517,7 @@ __global__ void k_composite_bwd(const float* __restrict__ sigma_raw, const float
     const int64_t off = (int64_t)s * R + r;
     g_sigma[off] = cp;  // P_{s-1}
     const float sigma = fmaxf(__ldg(sigma_raw + off), 0.0f);
-    const float alpha = 1.0f - nrt_expf(-sigma * __ldg(ts + s));
+    const float alpha = 1.0f - nrt_expf(-sigma * comp_t<PER_RAY>(ts, s, R, r));
     if (s == 0) {
       a0 = alpha;
       D0 = go0 * __ldg(rgb + off * 3) + go1 * __ldg(rgb + off * 3 + 1) + go2 * __ldg(rgb + off * 3 + 2);
@@ -524,7 +533,7 @@ __global__ void k_composite_bwd(const float* __restrict__ sigma_raw, const float
     const float Pprev = g_sigma[off];
     const float raw = __ldg(sigma_raw + off);
     const float sigma = fmaxf(raw, 0.0f);
-    const float t = __ldg(ts + s);
+    const float t = comp_t<PER_RAY>(ts, s, R, r);
     const float e = nrt_expf(-sigma * t);
     const float alpha = 1.0f - e;
     const float om = 1.0f - alpha;
@@ -730,7 +739,7 @@ extern "C" int nrt_composite_forward(const float* sigma_raw, const float* rgb, c
   if (R == 0) return NRT_OK;
   NRT_REQUIRE(sigma_raw && rgb && ts && out, "nrt_composite_forward: null pointer");
   NrtProfScope _ps(TAG_COMPOSITE_FWD, (cudaStream_t)stream);
-  k_composite_fwd<<<nrt_cdiv(R, 128), 128, 0, (cudaStream_t)stream>>>(sigma_raw, rgb, ts, S, R, out);
+  k_composite_fwd<false><<<nrt_cdiv(R, 128), 128, 0, (cudaStream_t)stream>>>(sigma_raw, rgb, ts, S, R, out);
   NRT_CUDA(cudaGetLastError());
   return NRT_OK;
 }
@@ -742,8 +751,33 @@ extern "C" int nrt_composite_backward(const float* sigma_raw, const float* rgb, 
   if (R == 0) return NRT_OK;
   NRT_REQUIRE(sigma_raw && rgb && ts && g_out && g_sigma_raw && g_rgb, "nrt_composite_backward: null pointer");
   NrtProfScope _ps(TAG_COMPOSITE_BWD, (cudaStream_t)stream);
-  k_composite_bwd<<<nrt_cdiv(R, 128), 128, 0, (cudaStream_t)stream>>>(sigma_raw, rgb, ts, S, R, g_out,
-                                                                      g_sigma_raw, g_rgb);
+  k_composite_bwd<false><<<nrt_cdiv(R, 128), 128, 0, (cudaStream_t)stream>>>(sigma_raw, rgb, ts, S, R, g_out,
+                                                                             g_sigma_raw, g_rgb);
+  NRT_CUDA(cudaGetLastError());
+  return NRT_OK;
+}
+
+// the same pair over per-sample distances ts [S,R] (hierarchical sampling, nrt_nerfle_sample_hierarchical)
+extern "C" int nrt_composite_forward_ts(const float* sigma_raw, const float* rgb, const float* ts, int S,
+                                        int64_t R, float* out, void* stream) {
+  NRT_REQUIRE(S >= 1 && R >= 0, "nrt_composite_forward_ts: bad arguments");
+  if (R == 0) return NRT_OK;
+  NRT_REQUIRE(sigma_raw && rgb && ts && out, "nrt_composite_forward_ts: null pointer");
+  NrtProfScope _ps(TAG_COMPOSITE_TS_FWD, (cudaStream_t)stream);
+  k_composite_fwd<true><<<nrt_cdiv(R, 128), 128, 0, (cudaStream_t)stream>>>(sigma_raw, rgb, ts, S, R, out);
+  NRT_CUDA(cudaGetLastError());
+  return NRT_OK;
+}
+
+extern "C" int nrt_composite_backward_ts(const float* sigma_raw, const float* rgb, const float* ts, int S,
+                                         int64_t R, const float* g_out, float* g_sigma_raw, float* g_rgb,
+                                         void* stream) {
+  NRT_REQUIRE(S >= 1 && R >= 0, "nrt_composite_backward_ts: bad arguments");
+  if (R == 0) return NRT_OK;
+  NRT_REQUIRE(sigma_raw && rgb && ts && g_out && g_sigma_raw && g_rgb, "nrt_composite_backward_ts: null pointer");
+  NrtProfScope _ps(TAG_COMPOSITE_TS_BWD, (cudaStream_t)stream);
+  k_composite_bwd<true><<<nrt_cdiv(R, 128), 128, 0, (cudaStream_t)stream>>>(sigma_raw, rgb, ts, S, R, g_out,
+                                                                            g_sigma_raw, g_rgb);
   NRT_CUDA(cudaGetLastError());
   return NRT_OK;
 }

@@ -66,10 +66,13 @@ __device__ __forceinline__ float hash_u01(uint64_t seed, uint64_t a, uint64_t b)
   return (float)(h >> 8) * (1.0f / 16777216.0f);
 }
 
-// four consecutive samples of one ray per thread (S % 4 == 0: one 16-byte store per thread, coalesced), else one
+// four consecutive samples of one ray per thread (S % 4 == 0: one 16-byte store per thread, coalesced), else one.
+// seed_dev (training under CUDA graphs, nrt_nerfle_sample_hierarchical): when not NULL the seed is read from device memory
+// instead of the by-value `seed`, so that a captured launch draws new jitter whenever the caller advances it.
 template <int V>
 __global__ void k_stratified_ts(int64_t R, int64_t r_off, int S, float t_near, float t_far, uint64_t seed,
-                                float* __restrict__ ts) {
+                                const uint64_t* __restrict__ seed_dev, float* __restrict__ ts) {
+  if (seed_dev) seed = *seed_dev;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int SV = S / V;
   if (i >= R * SV) return;
@@ -99,8 +102,9 @@ template <bool EXACT>
 __global__ void __launch_bounds__(kPdfWarps * 32)
 k_sample_pdf(const float* __restrict__ sigma_c, const float* __restrict__ ts_c_shared,
              const float* __restrict__ ts_c_per_ray, int Sc, int Sf, int64_t R, int64_t r_off,
-             uint64_t seed, float* __restrict__ ts_f) {
+             uint64_t seed, const uint64_t* __restrict__ seed_dev, float* __restrict__ ts_f) {
   extern __shared__ float sm[];
+  if (seed_dev) seed = *seed_dev;       // as in k_stratified_ts
   const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* s_t = sm + (size_t)wid * 3 * Sc;
   float* s_cdf = s_t + Sc;     // inclusive cdf over the interior samples (index = sample)
@@ -283,7 +287,83 @@ __global__ void k_merge_composite(const float* __restrict__ sig_c, const float* 
   if (lane == 0) { out[r * 3] = acc0; out[r * 3 + 1] = acc1; out[r * 3 + 2] = acc2; }
 }
 
+// ---- merged distances only (training: nrt_nerfle_sample_hierarchical), written SAMPLE-major ----------
+// The same ranks as k_merge_composite (coarse first on ties), one warp per ray, but the output is ts_out [S, R_out] with
+// m = s * R_out + ray, the layout of the training kernels.  A block merges kMergeTsRays rays into a shared-memory tile
+// [S][kMergeTsRays + 1] and then writes every sample row as kMergeTsRays consecutive floats (coalesced across rays).  The
+// padding column makes the row-wise reads of the write-out conflict-free; the per-ray column writes hit rows i + rank,
+// which can be 32 apart within one warp instruction and then share a bank (rare, a few extra cycles).  With Sf = 0 the
+// kernel is the transpose of the stratified distances.  Reads 4 B + writes 4 B per sample.
+constexpr int kMergeTsWarps = 8, kMergeTsRays = 32;
+static size_t merge_ts_smem(int S) { return ((size_t)S * (kMergeTsRays + 1) + (size_t)kMergeTsWarps * S) * sizeof(float); }
+__global__ void __launch_bounds__(kMergeTsWarps * 32)
+k_merge_ts(const float* __restrict__ ts_c, int Sc, const float* __restrict__ ts_f, int Sf, int64_t n, int64_t R_out,
+           int64_t r_off, float* __restrict__ ts_out) {
+  extern __shared__ float sm[];
+  const int S = Sc + Sf;
+  const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  constexpr int LD = kMergeTsRays + 1;
+  float* s_out = sm;
+  float* s_tc = sm + (size_t)S * LD + (size_t)wid * S;
+  float* s_tf = s_tc + Sc;
+  const int64_t rb = (int64_t)blockIdx.x * kMergeTsRays;
+  for (int k = wid; k < kMergeTsRays; k += kMergeTsWarps) {
+    const int64_t r = rb + k;
+    if (r >= n) break;
+    for (int i = lane; i < Sc; i += 32) s_tc[i] = ts_c[r * Sc + i];
+    for (int j = lane; j < Sf; j += 32) s_tf[j] = ts_f[r * Sf + j];
+    __syncwarp();
+    for (int i = lane; i < Sc; i += 32) {
+      const float t = s_tc[i];
+      int lo = 0, hi = Sf;
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (s_tf[mid] < t) lo = mid + 1; else hi = mid; }
+      s_out[(i + lo) * LD + k] = t;
+    }
+    for (int j = lane; j < Sf; j += 32) {
+      const float t = s_tf[j];
+      int lo = 0, hi = Sc;
+      while (lo < hi) { const int mid = (lo + hi) >> 1; if (s_tc[mid] <= t) lo = mid + 1; else hi = mid; }
+      s_out[(j + lo) * LD + k] = t;
+    }
+    __syncwarp();
+  }
+  __syncthreads();
+  const int nr = (int)min((int64_t)kMergeTsRays, n - rb);
+  for (int e = threadIdx.x; e < S * kMergeTsRays; e += blockDim.x) {
+    const int s = e / kMergeTsRays, k = e - s * kMergeTsRays;
+    if (k < nr) ts_out[(int64_t)s * R_out + r_off + rb + k] = s_out[s * LD + k];
+  }
+}
+
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+
+// the two sampling launches shared by the render and by nrt_nerfle_sample_hierarchical (seed_dev NULL: sampling->jitter_seed)
+static int launch_stratified(int64_t n, int64_t r0, int Sc, const nrt_nerf_sampling_t* sampling, const uint64_t* seed_dev,
+                             float* ts_c, cudaStream_t st) {
+  NrtProfScope _ps(TAG_STRATIFIED_TS, st);
+  if (Sc % 4 == 0)
+    k_stratified_ts<4><<<nrt_cdiv(n * (Sc / 4), 256), 256, 0, st>>>(n, r0, Sc, sampling->t_near, sampling->t_far,
+                                                                   sampling->jitter_seed, seed_dev, ts_c);
+  else
+    k_stratified_ts<1><<<nrt_cdiv(n * Sc, 256), 256, 0, st>>>(n, r0, Sc, sampling->t_near, sampling->t_far,
+                                                             sampling->jitter_seed, seed_dev, ts_c);
+  NRT_CUDA(cudaGetLastError());
+  return NRT_OK;
+}
+
+static int launch_sample_pdf(int prec, const float* sig_c, const float* ts_shared, const float* ts_pr, int Sc, int Sf,
+                             int64_t n, int64_t r0, uint64_t seed, const uint64_t* seed_dev, float* ts_f, cudaStream_t st) {
+  { NrtProfScope _ps(TAG_SAMPLE_PDF, st);
+  const int grid = (int)std::min<int64_t>((n + kPdfWarps - 1) / kPdfWarps, (int64_t)nrt_sm_count() * 16);
+  if (prec == NRT_PREC_F32)
+    k_sample_pdf<true><<<grid, kPdfWarps * 32, (size_t)kPdfWarps * 3 * Sc * sizeof(float), st>>>(
+        sig_c, ts_shared, ts_pr, Sc, Sf, n, r0, seed, seed_dev, ts_f);
+  else
+    k_sample_pdf<false><<<grid, kPdfWarps * 32, (size_t)kPdfWarps * 3 * Sc * sizeof(float), st>>>(
+        sig_c, ts_shared, ts_pr, Sc, Sf, n, r0, seed, seed_dev, ts_f); }
+  NRT_CUDA(cudaGetLastError());
+  return NRT_OK;
+}
 
 // rays are rendered in chunks of this many so that the scratch (per-sample sigma / rgb / latent: ~150 B x 192 per ray)
 // stays a few GB regardless of the image size (65,536-ray chunks measured 2 % slower: 3.3x the launches)
@@ -370,14 +450,8 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
     const float* ts_pr = nullptr;
     if (jitter || ts == nullptr) {
       // per-ray (stratified) distances; without jitter this is the bin-centre grid
-      NrtProfScope _ps(TAG_STRATIFIED_TS, st);
-      if (Sc % 4 == 0)
-        k_stratified_ts<4><<<nrt_cdiv(n * (Sc / 4), 256), 256, 0, st>>>(n, r0, Sc, sampling->t_near, sampling->t_far,
-                                                                       sampling->jitter_seed, ts_c);
-      else
-        k_stratified_ts<1><<<nrt_cdiv(n * Sc, 256), 256, 0, st>>>(n, r0, Sc, sampling->t_near, sampling->t_far,
-                                                                 sampling->jitter_seed, ts_c);
-      NRT_CUDA(cudaGetLastError());
+      const int rs = launch_stratified(n, r0, Sc, sampling, nullptr, ts_c, st);
+      if (rs != NRT_OK) return rs;
       ts_shared = nullptr; ts_pr = ts_c;
     }
     int rc;
@@ -392,15 +466,8 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
                    sig_c, rgb_c, tcws, tcws_bytes, st, kcam, r0);
     if (rc != NRT_OK) return rc;
     if (Sf > 0) {
-      { NrtProfScope _ps(TAG_SAMPLE_PDF, st);
-      const int grid = (int)std::min<int64_t>((n + kPdfWarps - 1) / kPdfWarps, (int64_t)nrt_sm_count() * 16);
-      if (prec == NRT_PREC_F32)
-        k_sample_pdf<true><<<grid, kPdfWarps * 32, (size_t)kPdfWarps * 3 * Sc * sizeof(float), st>>>(
-            sig_c, ts_shared, ts_pr, Sc, Sf, n, r0, sampling->jitter_seed, ts_f);
-      else
-        k_sample_pdf<false><<<grid, kPdfWarps * 32, (size_t)kPdfWarps * 3 * Sc * sizeof(float), st>>>(
-            sig_c, ts_shared, ts_pr, Sc, Sf, n, r0, sampling->jitter_seed, ts_f); }
-      NRT_CUDA(cudaGetLastError());
+      rc = launch_sample_pdf(prec, sig_c, ts_shared, ts_pr, Sc, Sf, n, r0, sampling->jitter_seed, nullptr, ts_f, st);
+      if (rc != NRT_OK) return rc;
       rc = nerf_pass(first, second, prec, c_rays, n, nullptr, ts_f, Sf, light_code, light_dim, c_view, nullptr,
                      sig_f, rgb_f, tcws, tcws_bytes, st, kcam, r0);
       if (rc != NRT_OK) return rc;
@@ -424,6 +491,77 @@ extern "C" int nrt_nerfle_render(const nrt_mlp_t* first, const nrt_mlp_t* second
   NRT_REQUIRE(R <= 0 || rays != nullptr, "nrt_nerfle_render: null rays");
   return render_impl(first, second, prec, rays, nullptr, R, ts, sampling, light_code, light_dim, view_of_ray, out_rgb,
                      workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- hierarchical sample distances for training (extension of nerf.py:178, see nrt_b200.h) -----------------------
+// The first half of render_impl: stratified coarse distances, the coarse pass keeping per-sample sigma, k_sample_pdf;
+// then k_merge_ts writes the merged ascending distances sample-major.  n_fine = 0 is the render's single stratified pass:
+// no coarse pass, the stratified distances are written sample-major as they are.  Chunked like the render, jitter hashed
+// with the global ray index, so the distances are those the render composites over (same prec, same seed).
+extern "C" size_t nrt_nerfle_sample_hierarchical_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
+                                                           int64_t R, const nrt_nerf_sampling_t* sampling) {
+  if (sampling == nullptr || R < 0) return 0;
+  const int64_t C = std::min<int64_t>(R, kRayChunk);
+  const int Sc = sampling->n_coarse, Sf = sampling->n_fine;
+  size_t total = 256 + align256((size_t)C * Sc * 4);
+  if (Sf == 0) return total;
+  total += align256((size_t)C * Sc * 4) + align256((size_t)C * Sc * 12) + align256((size_t)C * Sf * 4);
+  if (prec != NRT_PREC_F32) total += align256(nrt_nerfle_pass_tc_workspace(first, second, C, Sc));
+  return total;
+}
+
+extern "C" int nrt_nerfle_sample_hierarchical(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                              int64_t R, const nrt_nerf_sampling_t* sampling, const uint64_t* seed_dev,
+                                              const float* light_code, int light_dim, const int32_t* view_of_ray,
+                                              float* ts_out, void* workspace, size_t workspace_bytes, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  NRT_REQUIRE(R >= 0, "nrt_nerfle_sample_hierarchical: negative R");
+  NRT_REQUIRE(sampling != nullptr, "nrt_nerfle_sample_hierarchical: sampling descriptor is NULL");
+  const int Sc = sampling->n_coarse, Sf = sampling->n_fine;
+  NRT_REQUIRE(Sc >= 1 && Sf >= 0, "nrt_nerfle_sample_hierarchical: bad sample counts %d/%d", Sc, Sf);
+  NRT_REQUIRE(Sf == 0 || Sc >= 3, "nrt_nerfle_sample_hierarchical: hierarchical sampling needs n_coarse >= 3");
+  NRT_REQUIRE(Sc + Sf <= NRT_MAX_HIER_SAMPLES, "nrt_nerfle_sample_hierarchical: n_coarse + n_fine = %d exceeds %d",
+              Sc + Sf, NRT_MAX_HIER_SAMPLES);
+  NRT_REQUIRE(sampling->t_far > sampling->t_near, "nrt_nerfle_sample_hierarchical: needs t_near < t_far");
+  if (R == 0) return NRT_OK;
+  NRT_REQUIRE(rays != nullptr && ts_out != nullptr, "nrt_nerfle_sample_hierarchical: null rays/ts_out");
+  const int64_t C = std::min<int64_t>(R, kRayChunk);
+  const size_t need = nrt_nerfle_sample_hierarchical_workspace(first, second, prec, R, sampling);
+  NRT_REQUIRE(workspace != nullptr && workspace_bytes >= need,
+              "nrt_nerfle_sample_hierarchical: workspace of %zu bytes required, got %zu", need, workspace_bytes);
+  char* wp = (char*)workspace;
+  auto take = [&](size_t bytes) { char* p = wp; wp += align256(bytes); return (void*)p; };
+  float* ts_c = (float*)take((size_t)C * Sc * 4);
+  float *sig_c = nullptr, *rgb_c = nullptr, *ts_f = nullptr;
+  if (Sf > 0) {
+    sig_c = (float*)take((size_t)C * Sc * 4);
+    rgb_c = (float*)take((size_t)C * Sc * 12);
+    ts_f = (float*)take((size_t)C * Sf * 4);
+  }
+  void* tcws = nullptr; size_t tcws_bytes = 0;
+  if (Sf > 0 && prec != NRT_PREC_F32) {
+    tcws_bytes = nrt_nerfle_pass_tc_workspace(first, second, C, Sc);
+    tcws = take(tcws_bytes);
+  }
+  const size_t msmem = merge_ts_smem(Sc + Sf);
+  NRT_CUDA(cudaFuncSetAttribute(k_merge_ts, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem));
+  for (int64_t r0 = 0; r0 < R; r0 += C) {
+    const int64_t n = std::min<int64_t>(C, R - r0);
+    const int32_t* c_view = view_of_ray ? view_of_ray + r0 : nullptr;
+    int rc = launch_stratified(n, r0, Sc, sampling, seed_dev, ts_c, st);
+    if (rc != NRT_OK) return rc;
+    if (Sf > 0) {
+      rc = nerf_pass(first, second, prec, rays + r0 * 6, n, nullptr, ts_c, Sc, light_code, light_dim, c_view, nullptr,
+                     sig_c, rgb_c, tcws, tcws_bytes, st);
+      if (rc != NRT_OK) return rc;
+      rc = launch_sample_pdf(prec, sig_c, nullptr, ts_c, Sc, Sf, n, r0, sampling->jitter_seed, seed_dev, ts_f, st);
+      if (rc != NRT_OK) return rc;
+    }
+    { NrtProfScope _ps(TAG_MERGE_TS, st);
+    k_merge_ts<<<nrt_cdiv(n, kMergeTsRays), kMergeTsWarps * 32, msmem, st>>>(ts_c, Sc, ts_f, Sf, n, R, r0, ts_out); }
+    NRT_CUDA(cudaGetLastError());
+  }
+  return NRT_OK;
 }
 
 // ---- f4: the frame from a camera (main.py:57-88 for a volumetric shape as one call) ------------------------------

@@ -390,11 +390,13 @@ static int train_backward_io(const nrt_mlp_t* m, const MlpDev& d, IO io, int64_t
 // compositing kernels directly; the 64-d latent travels between the two MLPs as fp32 (the second MLP splits it into
 // hi + lo operands for its Fourier-phase GEMM), and so does its gradient on the way back.
 // ---------------------------------------------------------------------------------------------
+// PER_SAMPLE: ts [S,R] holds one distance per sample (t = ts[m], hierarchical sampling) instead of the shared ts [S]
+template <bool PER_SAMPLE>
 struct IoNerfTrainFirst {
   const float* rays; const float* ts; int64_t R; float* sigma; float* latent;
   __device__ __forceinline__ void load(int64_t m, float* v) const {
     const int64_t s = m / R, ray = m - s * R;
-    const float t = __ldg(ts + s);
+    const float t = __ldg(ts + (PER_SAMPLE ? m : s));
     const float* r = rays + ray * 6;
     v[0] = __ldg(r) + t * __ldg(r + 3); v[1] = __ldg(r + 1) + t * __ldg(r + 4); v[2] = __ldg(r + 2) + t * __ldg(r + 5);
   }
@@ -637,11 +639,12 @@ static int nerfle_train_nets(const nrt_mlp_t* first, const nrt_mlp_t* second, in
   return NRT_OK;
 }
 
-extern "C" int nrt_nerfle_train_forward(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays, int64_t R,
-                                        const float* ts, int S, const float* light_code, int light_dim,
-                                        const int32_t* view_of_ray, float* sigma, float* rgb, float* latent,
-                                        void* ws_first, size_t ws_first_bytes, void* ws_second, size_t ws_second_bytes,
-                                        void* stream) {
+template <bool PER_SAMPLE>
+static int nerfle_train_forward_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays, int64_t R,
+                                     const float* ts, int S, const float* light_code, int light_dim,
+                                     const int32_t* view_of_ray, float* sigma, float* rgb, float* latent,
+                                     void* ws_first, size_t ws_first_bytes, void* ws_second, size_t ws_second_bytes,
+                                     cudaStream_t st) {
   MlpDev d1, d2;
   int id2 = 0;
   int rc = nerfle_train_nets(first, second, light_dim, &d1, &d2, &id2);
@@ -657,9 +660,8 @@ extern "C" int nrt_nerfle_train_forward(const nrt_mlp_t* first, const nrt_mlp_t*
   const Layout y2 = make_layout(d2.in_size, d2.latent, d2.freqs, d2.hidden, d2.L, d2.skip, d2.out);
   const TrainWs w1 = carve_ws(y1, d1.hidden, d1.L, M, ws_first), w2 = carve_ws(y2, d2.hidden, d2.L, M, ws_second);
   NRT_REQUIRE(ws_first_bytes >= w1.bytes && ws_second_bytes >= w2.bytes, "training workspace too small");
-  cudaStream_t st = (cudaStream_t)stream;
   const int fmt = prec == NRT_PREC_BF16 ? 1 : 0;
-  IoNerfTrainFirst io1{rays, ts, R, sigma, latent};
+  IoNerfTrainFirst<PER_SAMPLE> io1{rays, ts, R, sigma, latent};
   rc = fmt == 0 ? train_forward_io<NetNerfFirst, 0>(first, io1, M, w1, st) : train_forward_io<NetNerfFirst, 1>(first, io1, M, w1, st);
   if (rc != NRT_OK) return rc;
   if (id2 == 2) {
@@ -668,6 +670,24 @@ extern "C" int nrt_nerfle_train_forward(const nrt_mlp_t* first, const nrt_mlp_t*
   }
   IoNerfTrainSecond<48> io2{rays, latent, light_code, view_of_ray, R, rgb};
   return fmt == 0 ? train_forward_io<NetNerfSecondLE, 0>(second, io2, M, w2, st) : train_forward_io<NetNerfSecondLE, 1>(second, io2, M, w2, st);
+}
+
+extern "C" int nrt_nerfle_train_forward(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays, int64_t R,
+                                        const float* ts, int S, const float* light_code, int light_dim,
+                                        const int32_t* view_of_ray, float* sigma, float* rgb, float* latent,
+                                        void* ws_first, size_t ws_first_bytes, void* ws_second, size_t ws_second_bytes,
+                                        void* stream) {
+  return nerfle_train_forward_impl<false>(first, second, prec, rays, R, ts, S, light_code, light_dim, view_of_ray, sigma, rgb,
+                                          latent, ws_first, ws_first_bytes, ws_second, ws_second_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int nrt_nerfle_train_forward_ts(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays, int64_t R,
+                                           const float* ts, int S, const float* light_code, int light_dim,
+                                           const int32_t* view_of_ray, float* sigma, float* rgb, float* latent,
+                                           void* ws_first, size_t ws_first_bytes, void* ws_second, size_t ws_second_bytes,
+                                           void* stream) {
+  return nerfle_train_forward_impl<true>(first, second, prec, rays, R, ts, S, light_code, light_dim, view_of_ray, sigma, rgb,
+                                         latent, ws_first, ws_first_bytes, ws_second, ws_second_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int nrt_nerfle_train_backward(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, int64_t R, int S,

@@ -238,11 +238,17 @@ def mlp_backward_tc(m: PackedMLP, M: int, out: torch.Tensor, g_out: torch.Tensor
 def nerfle_train_forward(first: PackedMLP, second: PackedMLP, rays: torch.Tensor, ts: torch.Tensor, light_code: torch.Tensor,
                          view_of_ray: Optional[torch.Tensor] = None, prec=PREC_F16):
     """Both NeRFLE MLPs under autograd on the tensor cores (nrt_nerfle_train_forward): rays [R,6], ts [S] ->
-    sigma [S,R], rgb [S,R,3] (sample-major) and the opaque state for nerfle_train_backward."""
+    sigma [S,R], rgb [S,R,3] (sample-major) and the opaque state for nerfle_train_backward.  A 2-D ts [S,R] gives every
+    sample its own distance (nrt_nerfle_train_forward_ts; the hierarchical samples of nerfle_sample_hierarchical)."""
     prec = prec_id(prec)
     r2 = _chk(rays, "rays").reshape(-1, 6)
-    R, S = r2.shape[0], ts.numel()
-    t = _chk(ts, "ts").reshape(S)
+    R = r2.shape[0]
+    per_sample = ts.dim() == 2
+    S = ts.shape[0] if per_sample else ts.numel()
+    if per_sample and ts.shape[1] != R:
+        raise NrtError("ts [S,R] has %d columns for %d rays" % (ts.shape[1], R))
+    t = _chk(ts, "ts").reshape(ts.shape if per_sample else (S,))
+    entry = N.lib().nrt_nerfle_train_forward_ts if per_sample else N.lib().nrt_nerfle_train_forward
     code = _chk(light_code, "light_code").reshape(-1, light_code.shape[-1])
     view = _chk(view_of_ray, "view_of_ray", torch.int32) if view_of_ray is not None else None
     dev = rays.device
@@ -257,9 +263,8 @@ def nerfle_train_forward(first: PackedMLP, second: PackedMLP, rays: torch.Tensor
             N.check(int(min(n1, n2)))
         ws1 = torch.empty(int(n1), dtype=torch.uint8, device=dev)
         ws2 = torch.empty(int(n2), dtype=torch.uint8, device=dev)
-        N.check(N.lib().nrt_nerfle_train_forward(ctypes.byref(c1), ctypes.byref(c2), prec, _ptr(r2), R, _ptr(t), S, _ptr(code),
-                                                 code.shape[-1], _ptr(view), _ptr(sigma), _ptr(rgb), _ptr(lat), _ptr(ws1),
-                                                 ws1.numel(), _ptr(ws2), ws2.numel(), _stream()))
+        N.check(entry(ctypes.byref(c1), ctypes.byref(c2), prec, _ptr(r2), R, _ptr(t), S, _ptr(code), code.shape[-1], _ptr(view),
+                      _ptr(sigma), _ptr(rgb), _ptr(lat), _ptr(ws1), ws1.numel(), _ptr(ws2), ws2.numel(), _stream()))
     return sigma, rgb, (ws1, ws2, R, S, code.shape[-1])
 
 
@@ -473,6 +478,40 @@ def composite_backward(sigma_raw, rgb, ts, g_out):
     return g_s, g_c.reshape(rgb.shape)
 
 
+def _ts_per_sample(ts, S, R):
+    t = _chk(ts, "ts")
+    if t.numel() != S * R:
+        raise NrtError("ts must hold one distance per sample, [%d,%d]; got %s" % (S, R, tuple(ts.shape)))
+    return t.reshape(S, R)
+
+
+def composite_forward_ts(sigma_raw: torch.Tensor, rgb: torch.Tensor, ts: torch.Tensor) -> torch.Tensor:
+    """composite_forward with per-sample distances: sigma_raw [S,...], rgb [S,...,3], ts [S,...] -> [...,3]
+    (nrt_composite_forward_ts; the reference's quirks kept)."""
+    sg = _chk(sigma_raw, "sigma_raw")
+    S, R = sg.shape[0], sg[0].numel()
+    c = _chk(rgb, "rgb").reshape(S, R, 3)
+    t = _ts_per_sample(ts, S, R)
+    out = torch.empty((R, 3), dtype=torch.float32, device=sg.device)
+    with torch.cuda.device(sg.device):
+        N.check(N.lib().nrt_composite_forward_ts(_ptr(sg), _ptr(c), _ptr(t), S, R, _ptr(out), _stream()))
+    return out.reshape(tuple(sigma_raw.shape[1:]) + (3,))
+
+
+def composite_backward_ts(sigma_raw, rgb, ts, g_out):
+    sg = _chk(sigma_raw, "sigma_raw")
+    S, R = sg.shape[0], sg[0].numel()
+    c = _chk(rgb, "rgb").reshape(S, R, 3)
+    t = _ts_per_sample(ts, S, R)
+    go = _chk(g_out, "g_out").reshape(R, 3)
+    g_s = torch.empty_like(sg)
+    g_c = torch.empty_like(c)
+    with torch.cuda.device(sg.device):
+        N.check(N.lib().nrt_composite_backward_ts(_ptr(sg), _ptr(c), _ptr(t), S, R, _ptr(go), _ptr(g_s), _ptr(g_c),
+                                                  _stream()))
+    return g_s, g_c.reshape(rgb.shape)
+
+
 def shading_frame(normals: torch.Tensor, rays: Optional[torch.Tensor] = None):
     """coordinate_system(normals) [..,3,3] and, if rays are given, wi = to_local(frame, -r_d)
     (interaction.py:9-27, 38-41; sdfs.py:158-159)."""
@@ -649,6 +688,43 @@ def nerfle_render(first: PackedMLP, second: PackedMLP, rays: torch.Tensor, ts: O
                                           ctypes.byref(samp), _ptr(lc), lc.shape[-1], _ptr(vor), _ptr(out),
                                           _ptr(ws), ws.numel(), _stream()))
     return out.reshape(batch + (3,))
+
+
+_sample_ws_cache = {}
+
+
+def nerfle_sample_hierarchical(first: PackedMLP, second: PackedMLP, rays: torch.Tensor, light_code: torch.Tensor,
+                               view_of_ray: Optional[torch.Tensor] = None, prec=PREC_F32, n_coarse=64, n_fine=128,
+                               t_near=0.0, t_far=2.05, jitter_seed=0, seed: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The merged coarse + fine distances nerfle_render(n_coarse, n_fine, ...) composites over, for training on them
+    (nrt_nerfle_sample_hierarchical): rays [...,6] -> ts [n_coarse + n_fine, R], ascending per ray, sample-major.
+    `seed`, a one-element int64 CUDA tensor, replaces jitter_seed when given: the kernels read it on the device."""
+    prec = prec_id(prec)
+    r2 = _chk(rays, "rays").reshape(-1, 6)
+    R = r2.shape[0]
+    lc = _chk(light_code, "light_code")
+    lc = lc.reshape(-1, lc.shape[-1])
+    vor = _chk(view_of_ray.reshape(-1), "view_of_ray", torch.int32) if view_of_ray is not None else None
+    sd = None
+    if seed is not None:
+        sd = _chk(seed, "seed", torch.int64)
+        if sd.numel() != 1:
+            raise NrtError("seed must hold one int64")
+    out = torch.empty((int(n_coarse) + int(n_fine), R), dtype=torch.float32, device=rays.device)
+    samp = N.NrtNerfSampling(int(n_coarse), int(n_fine), float(t_near), float(t_far), int(jitter_seed))
+    with torch.cuda.device(rays.device):
+        c1, c2 = first.c_struct(prec), second.c_struct(prec)
+        nbytes = N.lib().nrt_nerfle_sample_hierarchical_workspace(ctypes.byref(c1), ctypes.byref(c2), prec, R,
+                                                                  ctypes.byref(samp))
+        key = (rays.device.index, torch.cuda.current_stream().cuda_stream)
+        ws = _sample_ws_cache.get(key)
+        if ws is None or ws.numel() < nbytes:
+            ws = torch.empty(int(nbytes), dtype=torch.uint8, device=rays.device)
+            _sample_ws_cache[key] = ws
+        N.check(N.lib().nrt_nerfle_sample_hierarchical(ctypes.byref(c1), ctypes.byref(c2), prec, _ptr(r2), R,
+                                                       ctypes.byref(samp), _ptr(sd), _ptr(lc), lc.shape[-1], _ptr(vor),
+                                                       _ptr(out), _ptr(ws), ws.numel(), _stream()))
+    return out
 
 
 def nerfle_render_host(first: PackedMLP, second: PackedMLP, rays_host: torch.Tensor, ts_host: torch.Tensor,

@@ -43,6 +43,74 @@ def composite(sigma_raw, rgb, ts):
     return composite_reference_ops(sigma_raw, rgb, ts)
 
 
+class _CompositeTs(torch.autograd.Function):
+    """_Composite with per-sample distances ts [S,...] (hierarchical sampling)."""
+
+    @staticmethod
+    def forward(ctx, sigma_raw, rgb, ts):
+        s, c, t = sigma_raw.contiguous().float(), rgb.contiguous().float(), ts.contiguous().float()
+        ctx.save_for_backward(s, c, t)
+        return ops.composite_forward_ts(s, c, t)
+
+    @staticmethod
+    def backward(ctx, g):
+        s, c, t = ctx.saved_tensors
+        gs, gc = ops.composite_backward_ts(s, c, t, g.contiguous().float())
+        return gs, gc, None
+
+
+class HierarchicalSampling:
+    """Opt-in NeRF sampling for NeRFLE: n_coarse stratified distances in [t_near, t_far) (jittered within their bins when
+    `jitter`), a coarse pass, n_fine distances drawn by inverse-CDF resampling of the coarse weights, and compositing over
+    all n_coarse + n_fine samples in ascending order (n_fine = 0: one stratified pass).  An extension: the reference uses
+    64 shared uniform distances (nerf.py:178).  Assign an instance to `NeRFLE.sampling`.  CUDA only: the sampling, the
+    resampling and the compositing over per-sample distances exist as CUDA kernels alone, so a NeRFLE whose rays are on
+    the CPU raises NrtError while `sampling` is set.
+
+    Seeds: gradient-free renders use `render_seed` (fixed, so a frame renders the same image every time); training
+    reads the device tensor `train_seed(device)` and advances it by one per forward, so a step captured by
+    training.GraphedStep draws new coarse and fine jitter on every replay."""
+
+    def __init__(self, n_coarse=64, n_fine=128, t_near=0.0, t_far=2.05, jitter=True):
+        n_coarse, n_fine, t_near, t_far = int(n_coarse), int(n_fine), float(t_near), float(t_far)
+        if n_coarse < 1 or n_fine < 0:
+            raise ValueError("HierarchicalSampling: n_coarse must be >= 1 and n_fine >= 0, got %d / %d" % (n_coarse, n_fine))
+        if n_fine > 0 and n_coarse < 3:
+            raise ValueError("HierarchicalSampling: n_coarse must be >= 3 when n_fine > 0 (the resampling uses the interior "
+                             "coarse samples), got %d" % n_coarse)
+        if not t_far > t_near:
+            raise ValueError("HierarchicalSampling: t_far (%g) must be greater than t_near (%g)" % (t_far, t_near))
+        for name, k in (("n_coarse", n_coarse), ("n_fine", n_fine)):
+            if k > 0 and 64 % k != 0 and k % 64 != 0:
+                raise ValueError("HierarchicalSampling: %s = %d must divide 64 or be a multiple of 64 (the sample tiling of "
+                                 "the fp32 NeRFLE kernel that renders it and runs the fp32 coarse pass)" % (name, k))
+        if n_coarse + n_fine > ops.N.MAX_HIER_SAMPLES:
+            raise ValueError("HierarchicalSampling: n_coarse + n_fine = %d exceeds %d, the samples per ray the merge kernels "
+                             "hold in shared memory" % (n_coarse + n_fine, ops.N.MAX_HIER_SAMPLES))
+        self.n_coarse, self.n_fine, self.t_near, self.t_far, self.jitter = n_coarse, n_fine, t_near, t_far, bool(jitter)
+        self.render_seed = 0x5EED if self.jitter else 0
+        self.seed = None      # device int64 [1], created on the module's device by train_seed()
+
+    @property
+    def n_samples(self):
+        return self.n_coarse + self.n_fine
+
+    def train_seed(self, device):
+        """The device seed of the differentiable forward (None without jitter)."""
+        if not self.jitter:
+            return None
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        if self.seed is None or self.seed.device != device:
+            self.seed = torch.ones(1, dtype=torch.int64, device=device)
+        return self.seed
+
+    def __repr__(self):
+        return "HierarchicalSampling(n_coarse=%d, n_fine=%d, t_near=%g, t_far=%g, jitter=%s)" % (
+            self.n_coarse, self.n_fine, self.t_near, self.t_far, self.jitter)
+
+
 class _NerfleFused(torch.autograd.Function):
     """first MLP -> [latent | r_d | light] -> second MLP -> sigmoid on the tensor-core training kernels, nothing but
     sigma [S,...] and rgb [S,...,3] materialised in fp32 (ops.nerfle_train_forward / _backward).  Gradients reach the
@@ -60,7 +128,7 @@ class _NerfleFused(torch.autograd.Function):
         ctx.n1 = len(module.first._flat_params())
         ctx.save_for_backward(rgb)
         lead = tuple(rays.shape[:-1])
-        return sigma.reshape((ts.numel(),) + lead), rgb.reshape((ts.numel(),) + lead + (3,))
+        return sigma.reshape((sigma.shape[0],) + lead), rgb.reshape((sigma.shape[0],) + lead + (3,))
 
     @staticmethod
     def backward(ctx, g_sigma, g_rgb):
@@ -92,6 +160,9 @@ class NeRFLE(nn.Module):
         # optional device tensor in [0,1): when set, replaces random.random() of the far-plane jitter (nerf.py:178) so
         # that a CUDA-graph-captured step (neural_raytracing_b200.training.GraphedStep) still jitters per replay
         self.far_jitter = None
+        # optional HierarchicalSampling (not a constructor argument: the constructor keeps the reference's signature;
+        # not in state_dict).  None: the reference's 64 shared uniform distances.
+        self.sampling = None
 
     def _sample_ts(self, device):
         if getattr(self, "far_jitter", None) is not None:
@@ -129,19 +200,36 @@ class NeRFLE(nn.Module):
     def _needs_grad(self, rays):
         return torch.is_grad_enabled() and (rays.requires_grad or any(p.requires_grad for p in self.parameters()))
 
+    def _render_sampling(self):
+        """nerfle_render keyword arguments of `sampling` for a gradient-free render."""
+        s = self.sampling
+        return dict(n_coarse=s.n_coarse, n_fine=s.n_fine, t_near=s.t_near, t_far=s.t_far, jitter_seed=s.render_seed)
+
     def render_camera(self, cam, lights):
         """The frame of `cam` (ops.CameraDesc) in one library call, rays generated on the device inside it (f4):
         what pathtrace's tile loop + sample_positions + forward compute for an inference render (main.py:57-88,
-        nerf.py:175-214), with ONE far-plane draw (nerf.py:178) per frame instead of one per tile.
+        nerf.py:175-214), with ONE far-plane draw (nerf.py:178) per frame instead of one per tile (with `sampling` set:
+        its hierarchical samples, seeded by sampling.render_seed).
         -> rgb [n_views, nx, ny, bundle, 3]."""
         device = cam.device
-        ts = self._sample_ts(device)
         code = self._code_rows(self._light_code(lights, device), cam.n_views)
         prec = config.precision if self.first.precision() != "f32" and self.second.precision() != "f32" else "f32"
+        if getattr(self, "sampling", None) is not None:
+            return ops.nerfle_render_camera(self.first.packed(), self.second.packed(), cam, None, code.detach().float(),
+                                            prec=prec, **self._render_sampling())
+        ts = self._sample_ts(device)
         return ops.nerfle_render_camera(self.first.packed(), self.second.packed(), cam, ts, code.detach().float(),
                                         prec=prec)
 
     def forward(self, rays, lights):
+        """nerf.py:175-214.  With `sampling` (a HierarchicalSampling) set, the samples are its stratified coarse +
+        importance-resampled fine distances instead of the reference's 64 shared ones, and neither `far_jitter` nor
+        random.random() is used: a gradient-free forward renders with sampling.render_seed; a differentiable one takes
+        the merged distances from a no-grad coarse pass (at the train precision) seeded by the device tensor
+        sampling.train_seed(), advances that seed by one, and trains both MLPs on all n_coarse + n_fine samples (the
+        light code is a constant there, as on the fused path)."""
+        if getattr(self, "sampling", None) is not None:
+            return self._forward_hierarchical(rays, lights)
         r_o, r_d = rays.split([3, 3], dim=-1)
         device = r_o.device
         ts = self._sample_ts(device)
@@ -169,6 +257,43 @@ class NeRFLE(nn.Module):
         light = code.reshape((1, code.shape[0]) + (1,) * (len(lead) - 2) + (-1,)).expand(lead + (-1,))
         rgb = self.second(torch.cat([latent, r_d[None, ...].expand(lead + (3,)), light], dim=-1), out_act=ops.OUT_SIGMOID)
         return composite(alpha, rgb, ts)
+
+    def _forward_hierarchical(self, rays, lights):
+        s = self.sampling
+        if not rays.is_cuda:
+            raise ops.NrtError("NeRFLE.sampling (%r) runs on the CUDA kernels only; the rays are on %s -- set "
+                               "sampling = None for the reference's sampling on the CPU" % (s, rays.device))
+        r_o, r_d = rays.split([3, 3], dim=-1)
+        # the light code is a constant here, as on the fused path (nerfle.py optimises model.parameters() only)
+        code = self._code_rows(self._light_code(lights, rays.device), rays.shape[0]).detach().float()
+        view = self._view_index(rays)
+        if not self._needs_grad(rays):
+            prec = config.precision if self.first.precision() != "f32" and self.second.precision() != "f32" else "f32"
+            return ops.nerfle_render(self.first.packed(), self.second.packed(), rays.detach().float(), None, code, view,
+                                     prec=prec, **self._render_sampling())
+        tprec = self.first.train_precision()
+        fused = tprec != "f32" and self.second.train_precision() == tprec and not rays.requires_grad
+        seed = s.train_seed(rays.device)
+        with torch.no_grad():
+            ts = ops.nerfle_sample_hierarchical(self.first.packed(), self.second.packed(), rays.detach().float(), code,
+                                                view, prec=tprec if fused else "f32",
+                                                n_coarse=s.n_coarse, n_fine=s.n_fine, t_near=s.t_near, t_far=s.t_far,
+                                                seed=seed)
+            if seed is not None:
+                seed.add_(1)
+        lead = tuple(rays.shape[:-1])
+        if fused:
+            alpha, rgb = _NerfleFused.apply(self, rays, ts, code, view, tprec, *self.first._flat_params(),
+                                            *self.second._flat_params())
+            return _CompositeTs.apply(alpha, rgb, ts.reshape(alpha.shape))
+        ts = ts.reshape((s.n_samples,) + lead)
+        pts = r_o.unsqueeze(0) + ts[..., None] * r_d.unsqueeze(0)
+        first_out = self.first(pts)
+        latent, alpha = first_out[..., 1:], first_out[..., 0]
+        light = code.reshape((1, code.shape[0]) + (1,) * (len(lead) - 1) + (-1,)).expand(latent.shape[:-1] + (-1,))
+        rgb = self.second(torch.cat([latent, r_d[None, ...].expand(latent.shape[:-1] + (3,)), light], dim=-1),
+                          out_act=ops.OUT_SIGMOID)
+        return _CompositeTs.apply(alpha, rgb, ts)
 
 
 class PlainNeRF(nn.Module):

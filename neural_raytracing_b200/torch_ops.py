@@ -195,6 +195,37 @@ def _comp_bwd(ctx, g):
 composite.register_autograd(_comp_bwd, setup_context=_comp_setup)
 
 
+@torch.library.custom_op(NS + "::composite_ts", mutates_args=())
+def composite_ts(sigma_raw: Tensor, rgb: Tensor, ts: Tensor) -> Tensor:
+    """composite with per-sample distances ts [S,R] (hierarchical sampling; the reference's quirks kept) -> [R,3]."""
+    return ops.composite_forward_ts(sigma_raw, rgb, ts).reshape(-1, 3)
+
+
+@composite_ts.register_fake
+def _(sigma_raw, rgb, ts):
+    return sigma_raw.new_empty((sigma_raw[0].numel(), 3))
+
+
+@torch.library.custom_op(NS + "::composite_ts_backward", mutates_args=())
+def composite_ts_backward(sigma_raw: Tensor, rgb: Tensor, ts: Tensor, g_out: Tensor) -> Tuple[Tensor, Tensor]:
+    g_s, g_c = ops.composite_backward_ts(sigma_raw, rgb, ts, g_out.contiguous())
+    return g_s.reshape(sigma_raw.shape), g_c.reshape(rgb.shape)
+
+
+@composite_ts_backward.register_fake
+def _(sigma_raw, rgb, ts, g_out):
+    return sigma_raw.new_empty(sigma_raw.shape), rgb.new_empty(rgb.shape)
+
+
+def _comp_ts_bwd(ctx, g):
+    s, c, t = ctx.saved_tensors
+    g_s, g_c = torch.ops.nrt_b200.composite_ts_backward(s, c, t, g)
+    return g_s, g_c, None
+
+
+composite_ts.register_autograd(_comp_ts_bwd, setup_context=_comp_setup)
+
+
 # ---- a6 / a22: value and Jacobian of an in_size-3 SkipConnMLP (SphereSDF.shift) -----------------------------------
 @torch.library.custom_op(NS + "::mlp_value_jac", mutates_args=())
 def mlp_value_jac(p: Tensor, params: Tensor, basis: Tensor, arch: List[int]) -> Tuple[Tensor, Tensor, Tensor]:
@@ -302,6 +333,24 @@ def _(rays, ts, light_code, params1, basis1, arch1, params2, basis2, arch2, prec
     return rays.new_empty((rays.reshape(-1, 6).shape[0], 3))
 
 
+@torch.library.custom_op(NS + "::nerfle_sample_hierarchical", mutates_args=())
+def nerfle_sample_hierarchical(rays: Tensor, light_code: Tensor, view_of_ray: Optional[Tensor], params1: Tensor, basis1: Tensor,
+                               arch1: List[int], params2: Tensor, basis2: Tensor, arch2: List[int], prec: int, n_coarse: int,
+                               n_fine: int, t_near: float, t_far: float, jitter_seed: int, seed: Optional[Tensor]) -> Tensor:
+    """The merged coarse + fine distances of nerfle_render's hierarchical mode (stratified coarse pass, inverse-CDF
+    resampling; an extension, nerf.py:178 uses one shared ts) -> ts [n_coarse + n_fine, R], sample-major, ascending per
+    ray (gradient-free).  `seed` (one int64 on the device) replaces jitter_seed when given."""
+    return ops.nerfle_sample_hierarchical(_mlp(params1, basis1, arch1), _mlp(params2, basis2, arch2), rays, light_code,
+                                          view_of_ray, prec=prec, n_coarse=n_coarse, n_fine=n_fine, t_near=t_near,
+                                          t_far=t_far, jitter_seed=jitter_seed, seed=seed)
+
+
+@nerfle_sample_hierarchical.register_fake
+def _(rays, light_code, view_of_ray, params1, basis1, arch1, params2, basis2, arch2, prec, n_coarse, n_fine, t_near, t_far,
+      jitter_seed, seed):
+    return rays.new_empty((n_coarse + n_fine, rays.reshape(-1, 6).shape[0]))
+
+
 # ---- a21 / f4: ray generators and the camera-driven render -------------------------------------------------------
 def _cam(kind: int, a: Tensor, b: Optional[Tensor], focal: float, size: float, x0: int, y0: int, nx: int, ny: int, bundle: int,
          positions: Optional[Tensor], jitter: float, jitter_seed: int) -> "ops.CameraDesc":
@@ -340,4 +389,5 @@ def _(kind, a, b, focal, size, x0, y0, nx, ny, bundle, jitter, jitter_seed, ts, 
 
 
 OPERATORS = ["camera_rays", "nerfle_render_camera", "mlp_forward", "mlp_backward", "mlp_forward_train_tc", "mlp_backward_tc", "composite", "composite_backward", "mlp_value_jac", "mlp_value_jac_backward",
-             "sdf_eval", "sdf_sphere_trace", "sdf_shadow_test", "sdf_min_scan", "nerfle_render"]
+             "sdf_eval", "sdf_sphere_trace", "sdf_shadow_test", "sdf_min_scan", "nerfle_render", "composite_ts",
+             "composite_ts_backward", "nerfle_sample_hierarchical"]
