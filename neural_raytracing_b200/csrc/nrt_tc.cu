@@ -467,7 +467,7 @@ extern "C" int nrt_mlp_pack_tc(const nrt_mlp_t* m, int prec, void* blob_out, voi
   NRT_REQUIRE(blob_out != nullptr && ((uintptr_t)blob_out & 15) == 0, "blob_out must be 16-byte aligned");
   NRT_REQUIRE(d.hidden % 16 == 0, "hidden must be a multiple of 16");
   const Layout y = make_layout(d.in_size, d.latent, d.freqs, d.hidden, d.L, d.skip, d.out);
-  const int total = y.w_elems + y.bias_floats;
+  const int total = pack_tc_items(y);
   const int grid = std::min(nrt_cdiv(total, 256), 1184);
   NrtProfScope _ps(TAG_TC_PACK, (cudaStream_t)stream);
   if (fmt_of(prec) == 0) k_pack_tc<0><<<grid, 256, 0, (cudaStream_t)stream>>>(d, y, (uint8_t*)blob_out);

@@ -27,12 +27,30 @@ struct Layout {
   int bias_floats;        // floats of the fp32 area: biases, then the two optional tables below
   int wout_f32_off;       // [H][4] fp32 output weights (out <= 4: the output layer runs in the last epilogue), or -1
   int basis_f32_off;      // [in][FP] fp32 Fourier basis (split-precision inputs: phases on the CUDA cores), or -1
-  int bytes;
+  int bytes;              // everything above, then the bias K-chunks if there are any (bk_off below)
 };
 
 __host__ __device__ constexpr int c16(int x) { return (x + 15) / 16 * 16; }
 __host__ __device__ constexpr int imax(int a, int b) { return a > b ? a : b; }
 __host__ __device__ constexpr bool is_skip(int i, int skip, int L) { return (i % skip) == 0 && i != L - 1; }
+
+// shared memory that k_mlp_tc may fill with a resident blob (larger blobs are streamed stage by stage)
+constexpr int kSmemBudget = 227 * 1024 - 2048;
+
+// NRT_BIAS_MMA: the biases of the MMA layers (init + hidden) ride the layer's MMA as one more K-chunk instead of being
+// pre-loaded into the accumulator by the previous epilogue (LDS + tcgen05.st + wait::st on every stage's critical chain).
+// The blob then carries, after the fp32 area, one 16-deep B chunk per such layer: row 0 = b_hi, row 1 = b_mid, row 2 = b_lo
+// (b = b_hi + b_mid + b_lo in the 16-bit operand format), rows 3..15 zero; k_mlp_tc multiplies it by a constant A chunk
+// [1, 1, 1, 0, ...] held once per CTA in TMEM.  Nothing before the chunks moves, so every kernel that reads the blob
+// without them (training forward, the SDF / wide kernels) sees the same offsets.  Laid out for nets with hidden width <= 64
+// (a stage's MMAs are ~160 cycles, shorter than the preload chain they replace), a tensor-core phase GEMM (in > 5) and a
+// fused output layer (out <= 4: no bias chunk of width NOP), while the resident blob still fits: among the instantiated
+// nets this is NeRFLE.second (point and environment light).  NeRFLE.first (221 KB of 225) would not fit its 7 chunks.
+// The switch is a bit set: bit 0 the bias K-chunks, bit 1 the skipped zero x_lo chunks of the phase GEMM (k_mlp_tc, ZLO);
+// 0 builds the kernels without either.
+#ifndef NRT_BIAS_MMA
+#define NRT_BIAS_MMA 3
+#endif
 
 __host__ __device__ constexpr Layout make_layout(int in, int lat, int f, int h, int L, int skip, int out) {
   Layout y{};
@@ -69,7 +87,16 @@ __host__ __device__ constexpr Layout make_layout(int in, int lat, int f, int h, 
   if (y.split) { y.basis_f32_off = boff; boff += in * y.FP; }
   y.bias_floats = boff;
   y.bytes = off * 2 + boff * 4;
+  if ((NRT_BIAS_MMA & 1) && h <= 64 && !y.split && out <= 4) {
+    const int bytes = (y.bytes + 127) / 128 * 128 + (y.n_ops - 2) * h * 16 * 2;    // ops 1 .. n_ops-2, each N = h
+    if (bytes <= kSmemBudget) y.bytes = bytes;
+  }
   return y;
+}
+// byte offset of the bias K-chunks (128-byte aligned after the fp32 area), or -1 when the blob has none
+__host__ __device__ constexpr int bk_off(const Layout& y) {
+  const int end = y.w_elems * 2 + y.bias_floats * 4;
+  return y.bytes > end ? (end + 127) / 128 * 128 : -1;
 }
 
 // maps a K index of the tensor-core encoding layout to the reference encoding index (-1: padding)
@@ -103,12 +130,30 @@ template <> struct Elem<1> {
 // pack kernel: packed-f32 parameters -> UMMA canonical (no-swizzle, K-major) 16-bit tiles + biases
 // element (n,k) of an [N x K] operand lives at ((k/8)*N + n)*8 + k%8
 // ---------------------------------------------------------------------------------------------
+// elements k_pack_tc writes: 16-bit weights, fp32 area, 16-bit bias K-chunks
+__host__ __device__ constexpr int pack_tc_items(const Layout& y) {
+  return y.w_elems + y.bias_floats + (bk_off(y) >= 0 ? (y.n_ops - 2) * y.opN[1] * 16 : 0);
+}
 template <int FMT>
 __global__ void k_pack_tc(MlpDev m, Layout y, uint8_t* __restrict__ blob) {
   uint16_t* w = reinterpret_cast<uint16_t*>(blob);
   float* bias = reinterpret_cast<float*>(blob + (size_t)y.w_elems * 2);
-  const int total = y.w_elems + y.bias_floats;
+  const int total = pack_tc_items(y);
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
+    if (idx >= y.w_elems + y.bias_floats) {
+      // bias K-chunk of op o = 1 + e / (N*16), N = hidden: element (n, k) at (k/8)*N*8 + n*8 + k%8; rows k = 0, 1, 2 hold
+      // b_hi, b_mid, b_lo (each the rounding of what the previous terms left over)
+      const int e = idx - y.w_elems - y.bias_floats, N = y.opN[1];
+      const int o = 1 + e / (N * 16), r = e - (o - 1) * (N * 16);
+      const int kg = r / (N * 8), rem = r - kg * (N * 8), n = rem / 8, k = kg * 8 + (rem & 7);
+      float v = 0.0f;
+      if (k < 3 && n < m.N[o - 1]) {
+        float res = m.params[m.b_off[o - 1] + n];
+        for (int t = 0; t <= k; ++t) { v = Elem<FMT>::back(Elem<FMT>::cvt(res)); res -= v; }
+      }
+      reinterpret_cast<uint16_t*>(blob + bk_off(y))[e] = Elem<FMT>::cvt(v);
+      continue;
+    }
     if (idx >= y.w_elems) {
       int b = idx - y.w_elems;
       if (y.basis_f32_off >= 0 && b >= y.basis_f32_off) {
@@ -897,8 +942,12 @@ struct Net {
   static_assert(H % 16 == 0 && H <= 256, "hidden must be a multiple of 16");
   // Weights that do not fit in shared memory are STREAMED: each tile slot owns two stage buffers and the MMA warp
   // prefetches the next stage's operand (cp.async.bulk from L2) while the current stage computes.
-  static constexpr int kSmemBudget = 227 * 1024 - 2048;
   static constexpr bool STREAM = Y.bytes > kSmemBudget;
+  // Bias K-chunks (NRT_BIAS_MMA, see make_layout): the constant A chunk [1, 1, 1, 0, ...] takes 8 TMEM columns after the
+  // slots (NeRFLE.second: 3 x 160 + 8 = 488 of 512 point light, 2 x 208 + 8 = 424 environment light)
+  static constexpr int ONES_COL = NSLOT * COLS;
+  static constexpr int BK_OFF = bk_off(Y);
+  static constexpr bool BIAS_MMA = BK_OFF >= 0 && !STREAM && FUSE_OUT && ONES_COL + 8 <= 512;
   // One MMA-issuing warp per tile slot for the networks with resident weights (NRT_MMA_WARP_PER_SLOT=0: always a
   // single warp that serves the slots in ready order).  Measured on B200: NeRFLE.first 32.3 -> 30.7 ms, .second
   // 32.2 -> 24.3 ms per 800x800x192 frame; the weight-streaming softplus SDF net is SFU-bound in its epilogue and
@@ -938,7 +987,10 @@ constexpr int kEpiThreads = 128;
 // ELECT / R2UR / BRA.U.ANY serialisation loop: ~135 cycles per MMA instead of ~72, see profiles/.)
 // PART 0: the whole stage; 1: first half of the hidden K-chunks + the encoding chunks, no commit (K-split, on
 // `ready_a`); 2: second half of the hidden K-chunks + commit (on `ready`).
-template <class NET, int FMT, int ST, int PART = 0>
+// BMMA: stages >= 1 start with the layer's bias K-chunk (NET::BIAS_MMA), which overwrites the accumulator.
+// ZLO: leading 16-column chunks of the x_lo segment of the phase GEMM that are identically zero (a latent handed over
+// already in the operand format has x_lo = 0); they are not issued.
+template <class NET, int FMT, int ST, int PART = 0, bool BMMA = false, int ZLO = 0>
 __device__ __forceinline__ void issue_stage(uint32_t b_addr, uint32_t dD, uint32_t aU, uint32_t aE, uint64_t* done_bar) {
   constexpr Layout Y = NET::Y;
   constexpr uint32_t N = (uint32_t)Y.opN[ST];
@@ -953,6 +1005,11 @@ __device__ __forceinline__ void issue_stage(uint32_t b_addr, uint32_t dD, uint32
     // resident weights: b_addr is the base of the weight area and the operand offset is a compile-time constant;
     // streamed weights: b_addr is the stage buffer
     const uint64_t bd0 = make_desc(NET::STREAM ? b_addr : b_addr + (uint32_t)Y.op_off[ST] * 2u, lbo, sbo);
+    constexpr bool kBiasChunk = BMMA && ST > 0 && ST < NET::END_STAGE;
+    if constexpr (kBiasChunk) {
+      static_assert(NET::BIAS_MMA && N == (uint32_t)NET::H, "bias K-chunks: hidden-width MMA layers of a resident blob");
+      mma_ts(dD, (uint32_t)NET::ONES_COL, make_desc(b_addr + (uint32_t)NET::BK_OFF + (uint32_t)(ST - 1) * N * 32u, lbo, sbo), idesc, 0u);
+    }
 #pragma unroll
     for (int kc = 0; kc < kch; ++kc) {
       if (PART == 1 && kc >= k_u / 2 && kc < k_u) continue;
@@ -963,13 +1020,15 @@ __device__ __forceinline__ void issue_stage(uint32_t b_addr, uint32_t dD, uint32
         // raw encoding keeps it (in-place plan: the encoding region, else the union region), x_lo in the other one
         // (free until the epilogue of this stage has run).
         constexpr int xch = NET::XR / 16;
+        static_assert(ZLO < xch, "the chunk with the non-latent x_lo columns stays");
+        if (kc >= xch && kc < xch + ZLO) continue;
         const uint32_t hi = NET::INPLACE ? aE : aU, lo = NET::INPLACE ? aU : aE;
         a = (kc >= xch && kc < 2 * xch) ? (lo + (kc - xch) * 8) : (hi + (kc % xch) * 8);
       } else {
         a = (kc < k_u) ? (aU + kc * 8) : (aE + (kc - k_u) * 8);
       }
-      // every layer's accumulator was pre-loaded with its bias by the previous epilogue; only the
-      // phase GEMM (stage 0) starts from zero
+      // the phase GEMM (stage 0) starts from zero; every other layer's accumulator holds its bias already: pre-loaded
+      // by the previous epilogue, or written by the bias chunk above
       mma_ts(dD, a, bd0 + (uint64_t)((kc * 2 * lbo) >> 4), idesc, (ST > 0 || kc > 0) ? 1u : 0u);
     }
     if (PART != 1) tc_commit(done_bar);
@@ -978,10 +1037,10 @@ __device__ __forceinline__ void issue_stage(uint32_t b_addr, uint32_t dD, uint32
 }
 // runtime stage -> compile-time stage through a jump table (a linear if-chain cost up to ~150 cycles of taken
 // branches per stage on the single issuing warp, which serves every tile slot)
-template <class NET, int FMT, int PART = 0>
+template <class NET, int FMT, int PART = 0, bool BMMA = false, int ZLO = 0>
 __device__ __forceinline__ void issue_stage_dyn(int st, uint32_t b_addr, uint32_t dD, uint32_t aU, uint32_t aE,
                                                 uint64_t* done_bar) {
-#define NRT_STAGE_CASE(S) case S: if constexpr (S < NET::STAGES && (PART == 0 || S >= 2)) issue_stage<NET, FMT, S, PART>(b_addr, dD, aU, aE, done_bar); break;
+#define NRT_STAGE_CASE(S) case S: if constexpr (S < NET::STAGES && (PART == 0 || S >= 2)) issue_stage<NET, FMT, S, PART, BMMA, ZLO>(b_addr, dD, aU, aE, done_bar); break;
   switch (st) {
     NRT_STAGE_CASE(0) NRT_STAGE_CASE(1) NRT_STAGE_CASE(2) NRT_STAGE_CASE(3) NRT_STAGE_CASE(4) NRT_STAGE_CASE(5)
     NRT_STAGE_CASE(6) NRT_STAGE_CASE(7) NRT_STAGE_CASE(8) NRT_STAGE_CASE(9) NRT_STAGE_CASE(10) NRT_STAGE_CASE(11)
@@ -1069,6 +1128,12 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
   __shared__ uint32_t tmem_base_s;
   __shared__ uint32_t s_bias[NET::STAGES];
   constexpr bool ITER = IsIterative<IO>::value;
+  // bias K-chunks instead of the epilogue's bias preload (not in the training forward, which keeps the preload)
+  constexpr bool BMMA = NET::BIAS_MMA && !KSPLIT && WPS == 4 && !SV::kOn && !SV::kF32;
+  // leading input pairs that the IO policy can hand over already packed in the operand format (IoNerfSecond); their x_lo
+  // is zero, so the phase GEMM skips the ZLO x_lo chunks that hold nothing else
+  constexpr int kPP = (!ITER && !NET::SPLIT && !SV::kOn && !SV::kF32 && LAT == 0 && NET::ACT == NRT_ACT_LEAKY_RELU) ? PackedPairsOf<IO>::value : 0;
+  constexpr int ZLO = (NRT_BIAS_MMA & 2) ? 2 * kPP / 16 : 0;
   __shared__ volatile uint32_t s_slot_live[3];   // iterative policies: 0 once the slot's queue has run dry
   __shared__ uint32_t s_warp_live[3][4];
 
@@ -1126,6 +1191,19 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
   // base comes out of shared memory into a vector register and costs ~7 R2UR moves in front of every stage.
   if (tmem_base_s != 0u) __trap();
   constexpr uint32_t tmem = 0u;
+  if constexpr (BMMA) {
+    // the constant A chunk of the bias K-chunks, K elements [1, 1, 1, 0, ...] in every lane, shared read-only by all
+    // slots: warp w writes lane quarter w, before any MMA can read it
+    if (warp < 4) {
+      const uint32_t one = (uint32_t)one16<FMT>();
+      const uint32_t r[8] = {one | (one << 16), one, 0u, 0u, 0u, 0u, 0u, 0u};
+      TmemIO<8>::st(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)NET::ONES_COL, r);
+      tc_wait_st();
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+  }
   mbar_wait(&bar_w, 0);
 
   if (mma_id >= 0) {
@@ -1229,7 +1307,7 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           half_issued[slot] = false;
           issue_stage_dyn<NET, FMT, 2>(st[slot], b_addr, base, base + NET::DC, base + NET::DC + NET::UC, &bar_done[slot]);
         } else {
-          issue_stage_dyn<NET, FMT>(st[slot], b_addr, base, base + NET::DC, base + NET::DC + NET::UC, &bar_done[slot]);
+          issue_stage_dyn<NET, FMT, 0, BMMA, ZLO>(st[slot], b_addr, base, base + NET::DC, base + NET::DC + NET::UC, &bar_done[slot]);
         }
         if ((tid & 31) == 0) stamp(it_dbg[slot], st[slot], slot, 2);
         if (++st[slot] == NET::END_STAGE) {
@@ -1345,8 +1423,6 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
         int64_t m = 0;
         bool valid;
         float x[IN + LAT];
-        // leading input pairs that the IO policy can hand over already packed in the operand format (IoNerfSecond)
-        constexpr int kPP = (!ITER && !NET::SPLIT && !SV::kOn && !SV::kF32 && LAT == 0 && NET::ACT == NRT_ACT_LEAKY_RELU) ? PackedPairsOf<IO>::value : 0;
         uint32_t pw[kPP > 0 ? kPP : 1];
         if constexpr (ITER) {
           valid = primary ? io.next(state, x) : false;
@@ -1487,7 +1563,7 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
             // the phase GEMM has read x_lo: act(x) takes its place in the encoding region
             if constexpr (!NET::INPLACE) tmem_store<NET::XR / 2>(aE, ex);
           }
-          preload_bias<H>(dD, sBias + s_bias[1]);
+          if constexpr (!BMMA) preload_bias<H>(dD, sBias + s_bias[1]);
           uint32_t sr[F / 2], cr[F / 2], sa[F / 2], ca[F / 2];
 #pragma unroll
           for (int j = 0; j < F / 2; ++j) {
@@ -1556,7 +1632,9 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
                 }
               }
             }
-            if (st < L) preload_bias<HW>(dD + coff, sBias + s_bias[2 + st] + coff);
+            if constexpr (BMMA) {
+              // the next stage's bias K-chunk overwrites the accumulator
+            } else if (st < L) preload_bias<HW>(dD + coff, sBias + s_bias[2 + st] + coff);
             else {
               // output-layer bias: every half writes only the accumulator columns it has just read
               // (one warp per lane quarter: the primary writes all of them, also those beyond the hidden width -- an
