@@ -369,6 +369,44 @@ int nrt_nerfle_render_camera_host(const nrt_mlp_t* first, const nrt_mlp_t* secon
                                   const nrt_nerf_sampling_t* sampling, const float* light_code, int light_dim,
                                   float* out_rgb_host, void* stream);
 
+/* ---- meshes: a SphereSDF on a lattice, and the isosurface of a lattice (extension; the reference has no mesh output) ----
+ * Lattice: values[i][j][k] fp32 in C order (z fastest, torch's [nx, ny, nz]); point (i,j,k) is at origin + (i,j,k) * spacing,
+ * per axis one rounded product and one rounded sum (no FMA contraction).  Dimensions are in [2, NRT_MAX_LATTICE_DIM]; origin
+ * and spacing are finite, spacing > 0.  A caller with a box [bbox_min, bbox_max] uses spacing = (bbox_max - bbox_min) / (n - 1)
+ * computed in double and rounded to float once.
+ *
+ * Isosurface: marching tetrahedra on the Freudenthal (Kuhn) triangulation, 6 tetrahedra per cell, 0 -> e_a -> e_a + e_b ->
+ * (1,1,1) for the permutations (a,b,c) of the axes in lexicographic order.  A point is inside iff value < level (NaN is
+ * outside).  An edge from a (its lower end) to b carries a vertex iff the two ends differ in that test; the vertex is
+ * p_a + t (p_b - p_a) with t = (level - a) / (b - a), every operation rounded in fp32.  Outputs are deterministic:
+ *   verts [V,3] fp32, ascending by (lattice index of the lower end, direction d = 1..7, bit 0 = +i, bit 1 = +j, bit 2 = +k);
+ *   faces [F,3] int64 vertex indices, ascending by (cell = lattice index of its lowest corner, tetrahedron, triangle);
+ *   (v1 - v0) x (v2 - v0) points toward value >= level (outward for an SDF).
+ * The mesh is indexed and closed wherever the surface stays inside the lattice; where it leaves, its boundary lies on the
+ * lattice's faces.  Non-finite values never make a kernel read or write out of bounds, but a crossing next to a NaN or an
+ * infinity can give a non-finite vertex.
+ * Workspace of nrt_isosurface_*: 19 bytes per lattice point (a crossing mask, a vertex count and a triangle count of one byte,
+ * two int64 exclusive scans) plus CUB's scan storage; nrt_isosurface_workspace gives the exact size (256-byte aligned). */
+#define NRT_MAX_LATTICE_DIM 1024
+typedef struct nrt_lattice {
+  int64_t nx, ny, nz;
+  float origin[3];
+  float spacing[3];
+} nrt_lattice_t;
+/* values [nx,ny,nz] = SphereSDF.forward at the lattice points (nrt_sdf_eval at `prec`, bit-identical to it on the same points),
+ * 4,194,304 points per chunk.  workspace: nrt_sdf_lattice_eval_workspace bytes (12 per point of one chunk). */
+int64_t nrt_sdf_lattice_eval_workspace(const nrt_lattice_t* g);
+int nrt_sdf_lattice_eval(const nrt_sphere_sdf_t* s, int prec, const nrt_lattice_t* g, float* values, void* workspace,
+                         size_t workspace_bytes, void* stream);
+int64_t nrt_isosurface_workspace(const nrt_lattice_t* g);
+/* Count pass + scans: counts_dev (device int64[2]) receives V and F; the masks and offsets stay in the workspace for
+ * nrt_isosurface_emit, which must get the same lattice, values and level.  Does not synchronise. */
+int nrt_isosurface_count(const nrt_lattice_t* g, const float* values, float level, void* workspace, size_t workspace_bytes,
+                         int64_t* counts_dev, void* stream);
+/* Writes the first min(V, max_vertices) vertices and min(F, max_faces) faces, nothing past either. */
+int nrt_isosurface_emit(const nrt_lattice_t* g, const float* values, float level, void* workspace, size_t workspace_bytes,
+                        int64_t max_vertices, int64_t max_faces, float* verts, int64_t* faces, void* stream);
+
 /* ---- a8/a9/a12/a14/a15/a16: shading glue as fused elementwise kernels ---------------- */
 /* coordinate_system + to_local(-r_d) (interaction.py:9-27,38-41; sdfs.py:158-159).
  * normals [R,3] -> frame [R,3,3] (columns s,t,n as torch.stack(dim=-1)), wi [R,3]. */

@@ -46,6 +46,11 @@ class NrtCamera(ctypes.Structure):
 
 
 MAX_BSDFS = 16
+MAX_LATTICE_DIM = 1024     # NRT_MAX_LATTICE_DIM
+
+
+class NrtLattice(ctypes.Structure):
+    _fields_ = [("nx", c_i64), ("ny", c_i64), ("nz", c_i64), ("origin", c_f32 * 3), ("spacing", c_f32 * 3)]
 
 
 class NrtLight(ctypes.Structure):
@@ -65,6 +70,7 @@ class NrtError(RuntimeError):
 _PM, _PS, _PN = ctypes.POINTER(NrtMlp), ctypes.POINTER(NrtSphereSdf), ctypes.POINTER(NrtNerfSampling)
 _PL, _PB = ctypes.POINTER(NrtLight), ctypes.POINTER(NrtBlend)
 _PC = ctypes.POINTER(NrtCamera)
+_PG = ctypes.POINTER(NrtLattice)
 
 # every symbol declared in include/nrt_b200.h: name -> (restype, argtypes)
 SIGNATURES = {
@@ -118,6 +124,11 @@ SIGNATURES = {
     "nrt_nerfle_render_camera_workspace": (c_sz, [_PM, _PM, c_int, _PC, _PN]),
     "nrt_nerfle_render_camera": (c_int, [_PM, _PM, c_int, _PC, c_vp, _PN, c_vp, c_int, c_vp, c_vp, c_sz, c_vp]),
     "nrt_nerfle_render_camera_host": (c_int, [_PM, _PM, c_int, _PC, c_vp, c_int, _PN, c_vp, c_int, c_vp, c_vp]),
+    "nrt_sdf_lattice_eval_workspace": (c_i64, [_PG]),
+    "nrt_sdf_lattice_eval": (c_int, [_PS, c_int, _PG, c_vp, c_vp, c_sz, c_vp]),
+    "nrt_isosurface_workspace": (c_i64, [_PG]),
+    "nrt_isosurface_count": (c_int, [_PG, c_vp, c_f32, c_vp, c_sz, c_vp, c_vp]),
+    "nrt_isosurface_emit": (c_int, [_PG, c_vp, c_f32, c_vp, c_sz, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "nrt_shading_frame": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp]),
     "nrt_to_local": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp]),
     "nrt_param_rusin2": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp]),

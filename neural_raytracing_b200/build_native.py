@@ -29,6 +29,7 @@ EXTRA = {
     "nrt_shade.cu": ["-fmad=false"],
     "nrt_shade_direct.cu": ["-fmad=false"],
     "nrt_camera.cu": ["-fmad=false"],
+    "nrt_mesh.cu": ["-fmad=false"],
 }
 
 

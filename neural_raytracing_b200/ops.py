@@ -862,6 +862,66 @@ def nerfle_render_camera_host(first: PackedMLP, second: PackedMLP, cam: CameraDe
     return out_host
 
 
+# ---- meshes: a SphereSDF on a lattice, isosurface extraction (nrt_sdf_lattice_eval, nrt_isosurface_*) --------------
+def lattice(shape, origin, spacing) -> N.NrtLattice:
+    """nrt_lattice_t of a [nx, ny, nz] lattice with fp32 origin and spacing (validated by the library)."""
+    nx, ny, nz = (int(n) for n in shape)
+    return N.NrtLattice(nx, ny, nz, (ctypes.c_float * 3)(*[float(x) for x in origin]),
+                        (ctypes.c_float * 3)(*[float(x) for x in spacing]))
+
+
+def _cached_ws(cache, dev, nbytes):
+    if nbytes < 0:
+        N.check(int(nbytes))
+    key = (dev.index, torch.cuda.current_stream().cuda_stream)
+    ws = cache.get(key)
+    if ws is None or ws.numel() < nbytes:
+        cache.pop(key, None)
+        ws = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
+        cache[key] = ws
+    return ws
+
+
+_lattice_ws_cache = {}
+_iso_ws_cache = {}
+
+
+def sdf_lattice(s: PackedSDF, g: N.NrtLattice, prec=PREC_F32) -> torch.Tensor:
+    """SphereSDF.forward at every point of lattice g: values [nx, ny, nz] (nrt_sdf_lattice_eval, nrt_sdf_eval at `prec`)."""
+    prec = prec_id(prec)
+    dev = s.centers.device
+    values = torch.empty((g.nx, g.ny, g.nz), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        c = s.c_struct(prec)
+        ws = _cached_ws(_lattice_ws_cache, dev, N.lib().nrt_sdf_lattice_eval_workspace(ctypes.byref(g)))
+        N.check(N.lib().nrt_sdf_lattice_eval(ctypes.byref(c), prec, ctypes.byref(g), _ptr(values), _ptr(ws), ws.numel(),
+                                             _stream()))
+    return values
+
+
+def isosurface(values: torch.Tensor, origin, spacing, level=0.0):
+    """Marching tetrahedra on the lattice values [nx, ny, nz] (point (i,j,k) at origin + (i,j,k) * spacing) ->
+    verts [V,3] float32, faces [F,3] int64; conventions in include/nrt_b200.h.  Count pass, ONE device-to-host read of
+    (V, F) (the only host synchronisation), allocation, emit pass.  The workspace (19 bytes per lattice point) is kept
+    per device and stream."""
+    v = _chk(values, "values")
+    if v.dim() != 3:
+        raise NrtError("values must be a 3-D [nx, ny, nz] lattice, got %s" % (tuple(values.shape),))
+    g = lattice(v.shape, origin, spacing)
+    dev = v.device
+    with torch.cuda.device(dev):
+        ws = _cached_ws(_iso_ws_cache, dev, N.lib().nrt_isosurface_workspace(ctypes.byref(g)))
+        counts = torch.empty(2, dtype=torch.int64, device=dev)
+        N.check(N.lib().nrt_isosurface_count(ctypes.byref(g), _ptr(v), float(level), _ptr(ws), ws.numel(), _ptr(counts),
+                                             _stream()))
+        nv, nf = counts.tolist()
+        verts = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+        faces = torch.empty((nf, 3), dtype=torch.int64, device=dev)
+        N.check(N.lib().nrt_isosurface_emit(ctypes.byref(g), _ptr(v), float(level), _ptr(ws), ws.numel(), nv, nf,
+                                            _ptr(verts), _ptr(faces), _stream()))
+    return verts, faces
+
+
 # ---- launch accounting / per-kernel timing ----------------------------------------------------
 def profile_enable(on: bool):
     N.check(N.lib().nrt_profile_enable(1 if on else 0))

@@ -7,6 +7,6 @@ from .samplers import Sampler
 from .main import pathtrace, pathtrace_sample
 from .utils import LossSampler
 from .neural_blocks import SkipConnMLP
-from . import bsdf, cameras, checkpoint, integrators, lights, shapes, training_utils, utils, warps  # noqa: F401
+from . import bsdf, cameras, checkpoint, integrators, lights, mesh, shapes, training_utils, utils, warps  # noqa: F401
 
 __all__ = [k for k in globals().keys() if not k.startswith("_")]

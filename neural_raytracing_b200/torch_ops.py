@@ -388,6 +388,21 @@ def _(kind, a, b, focal, size, x0, y0, nx, ny, bundle, jitter, jitter_seed, ts, 
     return a.new_empty((a.shape[0], nx, ny, bundle, 3))
 
 
+# ---- meshes: isosurface of a lattice (extension; the reference has no mesh output) ----------------------------------
+@torch.library.custom_op(NS + "::isosurface", mutates_args=())
+def isosurface(values: Tensor, origin: List[float], spacing: List[float], level: float) -> Tuple[Tensor, Tensor]:
+    """Marching tetrahedra on the lattice values [nx, ny, nz] (point (i,j,k) at origin + (i,j,k) * spacing) ->
+    (verts [V,3] float32, faces [F,3] int64), V and F data-dependent (gradient-free)."""
+    return ops.isosurface(values, origin, spacing, level)
+
+
+@isosurface.register_fake
+def _(values, origin, spacing, level):
+    ctx = torch.library.get_ctx()
+    nv, nf = ctx.new_dynamic_size(), ctx.new_dynamic_size()
+    return values.new_empty((nv, 3)), values.new_empty((nf, 3), dtype=torch.int64)
+
+
 OPERATORS = ["camera_rays", "nerfle_render_camera", "mlp_forward", "mlp_backward", "mlp_forward_train_tc", "mlp_backward_tc", "composite", "composite_backward", "mlp_value_jac", "mlp_value_jac_backward",
              "sdf_eval", "sdf_sphere_trace", "sdf_shadow_test", "sdf_min_scan", "nerfle_render", "composite_ts",
-             "composite_ts_backward", "nerfle_sample_hierarchical"]
+             "composite_ts_backward", "nerfle_sample_hierarchical", "isosurface"]
