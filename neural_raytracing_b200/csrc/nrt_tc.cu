@@ -424,13 +424,16 @@ static int launch(const void* blob, const IO& io, int64_t M, cudaStream_t st, in
   const int64_t ntiles = (M + 127) / 128;
   const int grid = (int)std::min<int64_t>((ntiles + NET::NSLOT - 1) / NET::NSLOT, (int64_t)nrt_sm_count());
   NrtProfScope _ps(tag, st);
-  kern<<<grid, NET::threads(NET::WPS), bytes, st>>>(reinterpret_cast<const uint8_t*>(blob), io, M, g_dbg_timeline, sv);
+  kern<<<grid, NET::threads(NET::WPS), bytes, st>>>(reinterpret_cast<const uint8_t*>(blob) + NET::BLOB_OFF, io, M, g_dbg_timeline, sv);
   NRT_CUDA(cudaGetLastError());
   return NRT_OK;
 }
 
 // the networks instantiated on the tensor-core path (all weights must fit in 227 KB of smem)
 using NetNerfFirst = Net<3, 0, 16, 128, 5, 3, 65, NRT_ACT_LEAKY_RELU>;      // NeRFLE.first   nerf.py:162-167
+// NeRFLE.first's inference kernels (render pass, plain forward): with NRT_BIAS_MMA bit 2 they read the render layout, which
+// nrt_mlp_pack_tc appends to the training layout (tc_core.cuh, make_render_layout); otherwise the same net as above
+using NetNerfFirstR = Net<3, 0, 16, 128, 5, 3, 65, NRT_ACT_LEAKY_RELU, (NRT_BIAS_MMA & 4) != 0>;
 using NetNerfSecondPT = Net<70, 0, 16, 64, 8, 3, 3, NRT_ACT_LEAKY_RELU>;    // NeRFLE.second  nerf.py:169-172
 using NetNerfSecondLE = Net<115, 0, 16, 64, 8, 3, 3, NRT_ACT_LEAKY_RELU>;   // NeRFLE.second, envmap code (64+3+48)
 using NetNeuralBsdf = Net<3, 0, 64, 96, 6, 3, 3, NRT_ACT_LEAKY_RELU>;       // NeuralBSDF.mlp bsdfs.py:616-621
@@ -444,6 +447,11 @@ static bool matches(const MlpDev& d) {
   return d.in_size == NET::IN && d.latent == NET::LAT && d.freqs == NET::F && d.hidden == NET::H && d.L == NET::L &&
          d.skip == NET::SKIP && d.out == NET::OUT && d.act == NET::ACT;
 }
+template <class NET>
+static bool matches(const nrt_mlp_t& m) {
+  return m.in_size == NET::IN && m.latent_size == NET::LAT && m.freqs == NET::F && m.hidden == NET::H && m.num_layers == NET::L &&
+         m.skip == NET::SKIP && m.out_size == NET::OUT && m.act == NET::ACT;
+}
 
 }  // namespace tc
 
@@ -455,6 +463,7 @@ extern "C" int64_t nrt_mlp_tc_blob_bytes(const nrt_mlp_t* m, int prec) {
   NRT_REQUIRE(m != nullptr, "mlp descriptor is NULL");
   NRT_REQUIRE(prec == NRT_PREC_F16 || prec == NRT_PREC_BF16, "nrt_mlp_tc_blob_bytes: prec must be F16 or BF16");
   NRT_REQUIRE(m->num_layers >= 1 && m->num_layers <= NRT_MAX_LAYERS && m->hidden % 16 == 0, "unsupported MLP shape");
+  if (matches<NetNerfFirst>(*m)) return (int64_t)NetNerfFirstR::BLOB_OFF + NetNerfFirstR::Y.bytes;   // + the render layout
   const Layout y = make_layout(m->in_size, m->latent_size, m->freqs, m->hidden, m->num_layers, m->skip, m->out_size);
   return (int64_t)y.bytes;
 }
@@ -466,12 +475,15 @@ extern "C" int nrt_mlp_pack_tc(const nrt_mlp_t* m, int prec, void* blob_out, voi
   NRT_REQUIRE(prec == NRT_PREC_F16 || prec == NRT_PREC_BF16, "nrt_mlp_pack_tc: prec must be F16 or BF16");
   NRT_REQUIRE(blob_out != nullptr && ((uintptr_t)blob_out & 15) == 0, "blob_out must be 16-byte aligned");
   NRT_REQUIRE(d.hidden % 16 == 0, "hidden must be a multiple of 16");
-  const Layout y = make_layout(d.in_size, d.latent, d.freqs, d.hidden, d.L, d.skip, d.out);
-  const int total = pack_tc_items(y);
-  const int grid = std::min(nrt_cdiv(total, 256), 1184);
   NrtProfScope _ps(TAG_TC_PACK, (cudaStream_t)stream);
-  if (fmt_of(prec) == 0) k_pack_tc<0><<<grid, 256, 0, (cudaStream_t)stream>>>(d, y, (uint8_t*)blob_out);
-  else k_pack_tc<1><<<grid, 256, 0, (cudaStream_t)stream>>>(d, y, (uint8_t*)blob_out);
+  auto pack = [&](const Layout& y, const BiasRows& br, uint8_t* dst) {
+    const int grid = std::min(nrt_cdiv(pack_tc_items(y), 256), 1184);
+    if (fmt_of(prec) == 0) k_pack_tc<0><<<grid, 256, 0, (cudaStream_t)stream>>>(d, y, br, dst);
+    else k_pack_tc<1><<<grid, 256, 0, (cudaStream_t)stream>>>(d, y, br, dst);
+  };
+  pack(make_layout(d.in_size, d.latent, d.freqs, d.hidden, d.L, d.skip, d.out), no_bias_rows(), (uint8_t*)blob_out);
+  if (NetNerfFirstR::BLOB_OFF > 0 && matches<NetNerfFirst>(d))
+    pack(NetNerfFirstR::Y, NetNerfFirstR::BR, (uint8_t*)blob_out + NetNerfFirstR::BLOB_OFF);
   NRT_CUDA(cudaGetLastError());
   return NRT_OK;
 }
@@ -514,7 +526,7 @@ int nrt_mlp_forward_tc(const nrt_mlp_t* m, int prec, int out_act, const float* x
                   "NeuralBSDF.mlp and the occlusion MLP only");
     return NRT_E_UNSUPPORTED;
   }
-  if (matches<NetNerfFirst>(d)) return forward_plain<NetNerfFirst>(m, prec, out_act, x, latent, M, out, st);
+  if (matches<NetNerfFirst>(d)) return forward_plain<NetNerfFirstR>(m, prec, out_act, x, latent, M, out, st);
   if (matches<NetNerfSecondPT>(d)) return forward_plain<NetNerfSecondPT>(m, prec, out_act, x, latent, M, out, st);
   if (matches<NetNerfSecondLE>(d)) return forward_plain<NetNerfSecondLE>(m, prec, out_act, x, latent, M, out, st);
   if (matches<NetNeuralBsdf>(d)) return forward_plain<NetNeuralBsdf>(m, prec, out_act, x, latent, M, out, st);
@@ -669,16 +681,16 @@ int nrt_nerfle_pass_tc(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
     NRT_REQUIRE(pt && !lat32, "camera-fed tensor-core NeRF pass: point-light net with the 16-bit latent only");
     const WithCam wc{nrtcam::make_cam_dev(cam), cam_r0};
     IoNerfFirst<64, true> io1{nullptr, ts, ts_per_ray, S, out_sigma, lat, fmt, lat32, s_shift, wc};
-    rc = fmt == 0 ? launch<NetNerfFirst, decltype(io1), 0>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST)
-                  : launch<NetNerfFirst, decltype(io1), 1>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST);
+    rc = fmt == 0 ? launch<NetNerfFirstR, decltype(io1), 0>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST)
+                  : launch<NetNerfFirstR, decltype(io1), 1>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST);
     if (rc != NRT_OK) return rc;
     IoNerfSecond<64, 3, true, true> io2{nullptr, lat, light_code, nullptr, S, out_srgb, fmt, second_out_act, lat32, s_shift, wc};
     return fmt == 0 ? launch<NetNerfSecondPT, decltype(io2), 0>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND)
                     : launch<NetNerfSecondPT, decltype(io2), 1>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND);
   }
   IoNerfFirst<64> io1{rays, ts, ts_per_ray, S, out_sigma, lat, fmt, lat32, s_shift};
-  rc = fmt == 0 ? launch<NetNerfFirst, decltype(io1), 0>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST)
-                : launch<NetNerfFirst, decltype(io1), 1>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST);
+  rc = fmt == 0 ? launch<NetNerfFirstR, decltype(io1), 0>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST)
+                : launch<NetNerfFirstR, decltype(io1), 1>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST);
   if (rc != NRT_OK) return rc;
   if (pt && !lat32) {
     IoNerfSecond<64, 3, true> io2{rays, lat, light_code, view_of_ray, S, out_srgb, fmt, second_out_act, lat32, s_shift};

@@ -29,6 +29,12 @@ struct Layout {
   int basis_f32_off;      // [in][FP] fp32 Fourier basis (split-precision inputs: phases on the CUDA cores), or -1
   int bytes;              // everything above, then the bias K-chunks if there are any (bk_off below)
 };
+// where the biases of a render layout (make_render_layout) are; -1 = none (every other layout).  Kept out of Layout, whose
+// size shapes the stack frame of every k_mlp_tc instance.
+struct BiasRows {
+  int row;                // K index in the x segment of the encoding of the three rows b_hi, b_mid, b_lo (init / skip layers)
+  int bk8_off[kMaxOps];   // 16-bit element offset of the op's 8-deep bias chunk (before the weights)
+};
 
 __host__ __device__ constexpr int c16(int x) { return (x + 15) / 16 * 16; }
 __host__ __device__ constexpr int imax(int a, int b) { return a > b ? a : b; }
@@ -45,11 +51,12 @@ constexpr int kSmemBudget = 227 * 1024 - 2048;
 // without them (training forward, the SDF / wide kernels) sees the same offsets.  Laid out for nets with hidden width <= 64
 // (a stage's MMAs are ~160 cycles, shorter than the preload chain they replace), a tensor-core phase GEMM (in > 5) and a
 // fused output layer (out <= 4: no bias chunk of width NOP), while the resident blob still fits: among the instantiated
-// nets this is NeRFLE.second (point and environment light).  NeRFLE.first (221 KB of 225) would not fit its 7 chunks.
-// The switch is a bit set: bit 0 the bias K-chunks, bit 1 the skipped zero x_lo chunks of the phase GEMM (k_mlp_tc, ZLO);
-// 0 builds the kernels without either.
+// nets this is NeRFLE.second (point and environment light).  NeRFLE.first (221 KB of 225) would not fit its 7 chunks;
+// its inference kernels read a layout of their own instead (make_render_layout).
+// The switch is a bit set: bit 0 the bias K-chunks, bit 1 the skipped zero x_lo chunks of the phase GEMM (k_mlp_tc, ZLO),
+// bit 2 the render layout of NeRFLE.first (nrt_tc.cu); 0 builds the kernels without any of them.
 #ifndef NRT_BIAS_MMA
-#define NRT_BIAS_MMA 3
+#define NRT_BIAS_MMA 7
 #endif
 
 __host__ __device__ constexpr Layout make_layout(int in, int lat, int f, int h, int L, int skip, int out) {
@@ -98,6 +105,53 @@ __host__ __device__ constexpr int bk_off(const Layout& y) {
   const int end = y.w_elems * 2 + y.bias_floats * 4;
   return y.bytes > end ? (end + 127) / 128 * 128 : -1;
 }
+// Render layout (NRT_BIAS_MMA bit 2; NeRFLE.first, whose training layout leaves 5 KB of shared memory free): every bias
+// rides an MMA that k_mlp_tc issues, so the layout has no fp32 biases, only the Fourier basis.
+//  * init and skip layers: the x segment of the encoding is [x_hi | x_lo | x_hi | 0 ...] (raw) and [act_hi | act_lo | 0 ...]
+//    (activated); the kernel writes the constant 1 into its columns bias_row .. bias_row+2 = 3*in .. 3*in+2 in both, and
+//    the three weight rows there hold b_hi, b_mid, b_lo.  The bias enters through MMAs that are issued anyway.
+//  * the other layers: an 8-deep B chunk, rows b_hi, b_mid, b_lo, 0 ..., times the constant A chunk [1, 1, 1, 0, ...].
+//    Only the k = 0..7 core-matrix group is stored; the MMA still reads a k = 8..15 group at +LBO = 16*N bytes, which
+//    meets zeros of the A chunk and may be any finite 16-bit data.  The chunks sit in front of the weights, the output
+//    layer's (the narrowest) first, so each of those windows lies on the next chunk or on the weights.
+// The weights follow unchanged (op_off shifted by the chunks).
+__host__ __device__ constexpr BiasRows no_bias_rows() {
+  BiasRows b{};
+  b.row = -1;
+  for (int o = 0; o < kMaxOps; ++o) b.bk8_off[o] = -1;
+  return b;
+}
+__host__ __device__ constexpr BiasRows render_bias_rows(int in, int lat, int f, int h, int L, int skip, int out) {
+  const Layout y = make_layout(in, lat, f, h, L, skip, out);
+  BiasRows b = no_bias_rows();
+  b.row = 3 * in;
+  int c = 0;
+  b.bk8_off[y.n_ops - 1] = c; c += 8 * y.opN[y.n_ops - 1];
+  for (int o = 2; o < y.n_ops - 1; ++o)
+    if (!is_skip(o - 2, skip, L)) { b.bk8_off[o] = c; c += 8 * y.opN[o]; }
+  return b;
+}
+__host__ __device__ constexpr Layout make_render_layout(int in, int lat, int f, int h, int L, int skip, int out) {
+  Layout y = make_layout(in, lat, f, h, L, skip, out);
+  const BiasRows b = render_bias_rows(in, lat, f, h, L, skip, out);
+  int c = 0;   // 16-bit elements of the chunks
+  for (int o = 0; o < y.n_ops; ++o) c += b.bk8_off[o] >= 0 ? 8 * y.opN[o] : 0;
+  for (int o = 0; o < y.n_ops; ++o) { y.op_off[o] += c; y.bias_off[o] = -1; }
+  y.w_elems += c;
+  y.wout_f32_off = -1;
+  y.basis_f32_off = 0;
+  y.bias_floats = in * y.FP;
+  y.bytes = y.w_elems * 2 + y.bias_floats * 4;
+  return y;
+}
+// what k_mlp_tc relies on in a render layout: split inputs with room for the three bias rows in the x segment, an output
+// layer on the tensor cores, and every 8-deep chunk's k = 8..15 window inside 16-bit chunk or weight data
+__host__ __device__ constexpr bool render_layout_ok(const Layout& y, const BiasRows& b) {
+  if (!y.split || b.row + 3 > y.XR || y.wout_f32_off >= 0) return false;
+  for (int o = 0; o < y.n_ops; ++o)
+    if (b.bk8_off[o] >= 0 && (b.bk8_off[o] + 16 * y.opN[o] > y.w_elems || b.bk8_off[o] + 8 * y.opN[o] > y.op_off[0])) return false;
+  return true;
+}
 
 // maps a K index of the tensor-core encoding layout to the reference encoding index (-1: padding)
 __host__ __device__ inline int enc_ref_index(const Layout& y, int in, int k) {
@@ -134,24 +188,36 @@ template <> struct Elem<1> {
 __host__ __device__ constexpr int pack_tc_items(const Layout& y) {
   return y.w_elems + y.bias_floats + (bk_off(y) >= 0 ? (y.n_ops - 2) * y.opN[1] * 16 : 0);
 }
+// term t (0: b_hi, 1: b_mid, 2: b_lo) of a bias b = b_hi + b_mid + b_lo in the 16-bit operand format: each term is the
+// rounding of what the previous ones left over
 template <int FMT>
-__global__ void k_pack_tc(MlpDev m, Layout y, uint8_t* __restrict__ blob) {
+__device__ __forceinline__ float bias_term(float b, int t) {
+  float v = 0.0f;
+  for (int i = 0; i <= t; ++i) { v = Elem<FMT>::back(Elem<FMT>::cvt(b)); b -= v; }
+  return v;
+}
+template <int FMT>
+__global__ void k_pack_tc(MlpDev m, Layout y, BiasRows br, uint8_t* __restrict__ blob) {
   uint16_t* w = reinterpret_cast<uint16_t*>(blob);
   float* bias = reinterpret_cast<float*>(blob + (size_t)y.w_elems * 2);
   const int total = pack_tc_items(y);
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
     if (idx >= y.w_elems + y.bias_floats) {
       // bias K-chunk of op o = 1 + e / (N*16), N = hidden: element (n, k) at (k/8)*N*8 + n*8 + k%8; rows k = 0, 1, 2 hold
-      // b_hi, b_mid, b_lo (each the rounding of what the previous terms left over)
+      // b_hi, b_mid, b_lo
       const int e = idx - y.w_elems - y.bias_floats, N = y.opN[1];
       const int o = 1 + e / (N * 16), r = e - (o - 1) * (N * 16);
       const int kg = r / (N * 8), rem = r - kg * (N * 8), n = rem / 8, k = kg * 8 + (rem & 7);
-      float v = 0.0f;
-      if (k < 3 && n < m.N[o - 1]) {
-        float res = m.params[m.b_off[o - 1] + n];
-        for (int t = 0; t <= k; ++t) { v = Elem<FMT>::back(Elem<FMT>::cvt(res)); res -= v; }
-      }
+      const float v = (k < 3 && n < m.N[o - 1]) ? bias_term<FMT>(m.params[m.b_off[o - 1] + n], k) : 0.0f;
       reinterpret_cast<uint16_t*>(blob + bk_off(y))[e] = Elem<FMT>::cvt(v);
+      continue;
+    }
+    if (idx < y.op_off[0]) {
+      // 8-deep bias chunk of the render layout: element (n, k < 8) at n*8 + k
+      int o = 0;
+      while (br.bk8_off[o] < 0 || idx < br.bk8_off[o] || idx >= br.bk8_off[o] + 8 * y.opN[o]) ++o;
+      const int e = idx - br.bk8_off[o], n = e >> 3, k = e & 7;
+      w[idx] = Elem<FMT>::cvt((k < 3 && n < m.N[o - 1]) ? bias_term<FMT>(m.params[m.b_off[o - 1] + n], k) : 0.0f);
       continue;
     }
     if (idx >= y.w_elems) {
@@ -209,6 +275,9 @@ __global__ void k_pack_tc(MlpDev m, Layout y, uint8_t* __restrict__ blob) {
       else if (k < m.hidden) kref = k;
       else { const int r = enc_ref_index(y, m.in_size, k - m.hidden); kref = r < 0 ? -1 : m.hidden + r; }
       if (kref >= 0) v = m.params[m.w_off[li] + kref * m.hidden + n];
+      // render layout: the bias rows in the padding of the encoding's x segment (init and skip layers)
+      const int ke = o == 1 ? k : k - m.hidden;
+      if (br.row >= 0 && ke >= br.row && ke < br.row + 3) v = bias_term<FMT>(m.params[m.b_off[li] + n], ke - br.row);
     }
     w[idx] = Elem<FMT>::cvt(v);
   }
@@ -885,10 +954,15 @@ __device__ __forceinline__ void sincos_fast(float x, float* s, float* c) {
 // ---------------------------------------------------------------------------------------------
 // compile-time network description
 // ---------------------------------------------------------------------------------------------
-template <int IN_, int LAT_, int F_, int H_, int L_, int SKIP_, int OUT_, int ACT_>
+// RENDER: the net reads the render layout (make_render_layout), which the pack appends to the training layout in the same
+// blob at BLOB_OFF; inference kernels only (k_mlp_tc without saved activations).
+template <int IN_, int LAT_, int F_, int H_, int L_, int SKIP_, int OUT_, int ACT_, bool RENDER = false>
 struct Net {
   static constexpr int IN = IN_, LAT = LAT_, F = F_, H = H_, L = L_, SKIP = SKIP_, OUT = OUT_, ACT = ACT_;
-  static constexpr Layout Y = make_layout(IN, LAT, F, H, L, SKIP, OUT);
+  static constexpr Layout Y = RENDER ? make_render_layout(IN, LAT, F, H, L, SKIP, OUT) : make_layout(IN, LAT, F, H, L, SKIP, OUT);
+  static constexpr int BLOB_OFF = RENDER ? (make_layout(IN, LAT, F, H, L, SKIP, OUT).bytes + 127) / 128 * 128 : 0;
+  static constexpr BiasRows BR = RENDER ? render_bias_rows(IN, LAT, F, H, L, SKIP, OUT) : no_bias_rows();
+  static constexpr bool BIAS_ROWS = RENDER;
   static constexpr bool SPLIT = Y.split != 0;
   static constexpr int XR = Y.XR, KE = Y.KE, KX = Y.KX, KPH = Y.KPH, FP = Y.FP, NOP = Y.NOP, KRAW = Y.KRAW;
   static constexpr int DC = imax(H, imax(NOP, FP));       // fp32 accumulator columns
@@ -943,11 +1017,14 @@ struct Net {
   // Weights that do not fit in shared memory are STREAMED: each tile slot owns two stage buffers and the MMA warp
   // prefetches the next stage's operand (cp.async.bulk from L2) while the current stage computes.
   static constexpr bool STREAM = Y.bytes > kSmemBudget;
-  // Bias K-chunks (NRT_BIAS_MMA, see make_layout): the constant A chunk [1, 1, 1, 0, ...] takes 8 TMEM columns after the
-  // slots (NeRFLE.second: 3 x 160 + 8 = 488 of 512 point light, 2 x 208 + 8 = 424 environment light)
+  // Bias K-chunks (NRT_BIAS_MMA, see make_layout and make_render_layout): the constant A chunk [1, 1, 1, 0, ...] takes 8
+  // TMEM columns after the slots (NeRFLE.second: 3 x 160 + 8 = 488 of 512 point light, 2 x 208 + 8 = 424 environment
+  // light; NeRFLE.first: 2 x 216 + 8 = 440)
   static constexpr int ONES_COL = NSLOT * COLS;
   static constexpr int BK_OFF = bk_off(Y);
-  static constexpr bool BIAS_MMA = BK_OFF >= 0 && !STREAM && FUSE_OUT && ONES_COL + 8 <= 512;
+  static constexpr bool BIAS_MMA = (BK_OFF >= 0 && !STREAM && FUSE_OUT && ONES_COL + 8 <= 512) || RENDER;
+  static_assert(!RENDER || (Y.bytes <= kSmemBudget && ONES_COL + 8 <= 512 && render_layout_ok(Y, BR)),
+                "render layout: resident in shared memory, room for the constant A chunk in TMEM, bias rows and chunks in place");
   // One MMA-issuing warp per tile slot for the networks with resident weights (NRT_MMA_WARP_PER_SLOT=0: always a
   // single warp that serves the slots in ready order).  Measured on B200: NeRFLE.first 32.3 -> 30.7 ms, .second
   // 32.2 -> 24.3 ms per 800x800x192 frame; the weight-streaming softplus SDF net is SFU-bound in its epilogue and
@@ -1005,10 +1082,18 @@ __device__ __forceinline__ void issue_stage(uint32_t b_addr, uint32_t dD, uint32
     // resident weights: b_addr is the base of the weight area and the operand offset is a compile-time constant;
     // streamed weights: b_addr is the stage buffer
     const uint64_t bd0 = make_desc(NET::STREAM ? b_addr : b_addr + (uint32_t)Y.op_off[ST] * 2u, lbo, sbo);
-    constexpr bool kBiasChunk = BMMA && ST > 0 && ST < NET::END_STAGE;
+    // render layout: the init and skip layers take their bias from the encoding's bias rows, so their first MMA starts
+    // from zero; the other layers start with their 8-deep bias chunk
+    constexpr bool kBiasChunk = BMMA && !NET::BIAS_ROWS && ST > 0 && ST < NET::END_STAGE;
+    constexpr bool kBiasChunk8 = BMMA && NET::BIAS_ROWS && NET::BR.bk8_off[ST] >= 0;
+    constexpr bool kFromZero = ST == 0 || (BMMA && NET::BIAS_ROWS && NET::BR.bk8_off[ST] < 0);
     if constexpr (kBiasChunk) {
       static_assert(NET::BIAS_MMA && N == (uint32_t)NET::H, "bias K-chunks: hidden-width MMA layers of a resident blob");
       mma_ts(dD, (uint32_t)NET::ONES_COL, make_desc(b_addr + (uint32_t)NET::BK_OFF + (uint32_t)(ST - 1) * N * 32u, lbo, sbo), idesc, 0u);
+    }
+    if constexpr (kBiasChunk8) {
+      static_assert(!NET::STREAM, "bias chunks of a resident blob");
+      mma_ts(dD, (uint32_t)NET::ONES_COL, make_desc(b_addr + (uint32_t)NET::BR.bk8_off[ST] * 2u, lbo, sbo), idesc, 0u);
     }
 #pragma unroll
     for (int kc = 0; kc < kch; ++kc) {
@@ -1027,9 +1112,9 @@ __device__ __forceinline__ void issue_stage(uint32_t b_addr, uint32_t dD, uint32
       } else {
         a = (kc < k_u) ? (aU + kc * 8) : (aE + (kc - k_u) * 8);
       }
-      // the phase GEMM (stage 0) starts from zero; every other layer's accumulator holds its bias already: pre-loaded
-      // by the previous epilogue, or written by the bias chunk above
-      mma_ts(dD, a, bd0 + (uint64_t)((kc * 2 * lbo) >> 4), idesc, (ST > 0 || kc > 0) ? 1u : 0u);
+      // the phase GEMM (stage 0) starts from zero, and so do the layers with bias rows; every other layer's accumulator
+      // holds its bias already: pre-loaded by the previous epilogue, or written by the bias chunk above
+      mma_ts(dD, a, bd0 + (uint64_t)((kc * 2 * lbo) >> 4), idesc, (!kFromZero || kc > 0) ? 1u : 0u);
     }
     if (PART != 1) tc_commit(done_bar);
   }
@@ -1130,6 +1215,7 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
   constexpr bool ITER = IsIterative<IO>::value;
   // bias K-chunks instead of the epilogue's bias preload (not in the training forward, which keeps the preload)
   constexpr bool BMMA = NET::BIAS_MMA && !KSPLIT && WPS == 4 && !SV::kOn && !SV::kF32;
+  static_assert(BMMA || !NET::BIAS_ROWS, "the render layout has no fp32 biases to pre-load");
   // leading input pairs that the IO policy can hand over already packed in the operand format (IoNerfSecond); their x_lo
   // is zero, so the phase GEMM skips the ZLO x_lo chunks that hold nothing else
   constexpr int kPP = (!ITER && !NET::SPLIT && !SV::kOn && !SV::kF32 && LAT == 0 && NET::ACT == NRT_ACT_LEAKY_RELU) ? PackedPairsOf<IO>::value : 0;
@@ -1480,10 +1566,19 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
               const uint16_t ahi = E::cvt(ax_);
               a[j] = ahi; a[IN + j] = E::cvt(ax_ - E::back(ahi));
             }
+            // render layout: the constant-1 columns that the bias rows of the init and skip layers multiply
+            if constexpr (NET::BIAS_ROWS) {
+#pragma unroll
+              for (int t = 0; t < 3; ++t) v[NET::BR.row + t] = one16<FMT>();
+            }
 #pragma unroll
             for (int j = 0; j < 8; ++j) ax[j] = (uint32_t)v[2 * j] | ((uint32_t)v[2 * j + 1] << 16);
 #pragma unroll
             for (int j = 0; j < IN; ++j) ex[j] = (uint32_t)a[2 * j] | ((uint32_t)a[2 * j + 1] << 16);
+            if constexpr (NET::BIAS_ROWS) {
+#pragma unroll
+              for (int t = 0; t < 3; ++t) ex[(NET::BR.row + t) / 2] |= (uint32_t)one16<FMT>() << (16 * ((NET::BR.row + t) & 1));
+            }
             tmem_store<NET::KX / 2>(aU, ax);
             if constexpr (NET::INPLACE) tmem_store<NET::XR / 2>(aE, ax);   // raw x part; activated in place later
             else tmem_store<NET::XR / 2>(aE, ex);
