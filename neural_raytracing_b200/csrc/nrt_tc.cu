@@ -71,21 +71,29 @@ struct IoNerfFirst {
   const float* rays; const float* ts; const float* ts_per_ray; int S;
   float* sigma; void* latent; int fmt; int lat32; int s_shift;
   std::conditional_t<CAM, WithCam, NoCam> c;
-  __device__ __forceinline__ void load(int64_t m, float* v) const {
+  // load() in two halves (k_mlp_tc, NRT_FIRST_PIPE): fetch() issues the loads of t and of the ray (the camera variant also
+  // computes the ray), point() forms o + t d once they have landed
+  struct Fetch { float t, o[3], d[3]; };
+  __device__ __forceinline__ void fetch(int64_t m, Fetch& f) const {
     const int64_t ray = ray_of(m, S, s_shift);
     const int s = (int)(m - ray * S);
-    const float t = ts_per_ray ? __ldg(ts_per_ray + m) : __ldg(ts + s);
+    f.t = ts_per_ray ? __ldg(ts_per_ray + m) : __ldg(ts + s);
     if constexpr (CAM) {
-      float o[3], d[3];
       int view;
-      nrtcam::cam_ray(c.cam, c.r_off + ray, o, d, &view);
-      v[0] = o[0] + t * d[0]; v[1] = o[1] + t * d[1]; v[2] = o[2] + t * d[2];
+      nrtcam::cam_ray(c.cam, c.r_off + ray, f.o, f.d, &view);
     } else {
       const float* r = rays + ray * 6;
-      v[0] = __ldg(r) + t * __ldg(r + 3);
-      v[1] = __ldg(r + 1) + t * __ldg(r + 4);
-      v[2] = __ldg(r + 2) + t * __ldg(r + 5);
+#pragma unroll
+      for (int j = 0; j < 3; ++j) { f.o[j] = __ldg(r + j); f.d[j] = __ldg(r + 3 + j); }
     }
+  }
+  __device__ __forceinline__ static void point(const Fetch& f, float* v) {
+    v[0] = f.o[0] + f.t * f.d[0]; v[1] = f.o[1] + f.t * f.d[1]; v[2] = f.o[2] + f.t * f.d[2];
+  }
+  __device__ __forceinline__ void load(int64_t m, float* v) const {
+    Fetch f;
+    fetch(m, f);
+    point(f, v);
   }
   __device__ __forceinline__ void store(int64_t m, const float* o) const {
     sigma[m] = o[0];
@@ -188,7 +196,9 @@ struct IoNerfSecond {
 };
 
 static long long* g_dbg_timeline = nullptr;   // development only, see tools/tc_timeline.py
+static int g_dbg_timeline_tag = -1;            // stamp only the launches of this profile tag (-1: every launch)
 extern "C" void nrtdbg_set_timeline(long long* dev_buf) { g_dbg_timeline = dev_buf; }
+extern "C" void nrtdbg_set_timeline_tag(int tag) { g_dbg_timeline_tag = tag; }
 
 // smooth-min of the warped spheres (sdfs.py:37-46, utils.py:385-387), fast-math version for the 16-bit path.
 // The sphere parameters sit in shared memory as rows [A_j0 A_j1 A_j2 c_j] of (I + T_i) and the centre, plus the radii
@@ -424,7 +434,8 @@ static int launch(const void* blob, const IO& io, int64_t M, cudaStream_t st, in
   const int64_t ntiles = (M + 127) / 128;
   const int grid = (int)std::min<int64_t>((ntiles + NET::NSLOT - 1) / NET::NSLOT, (int64_t)nrt_sm_count());
   NrtProfScope _ps(tag, st);
-  kern<<<grid, NET::threads(NET::WPS), bytes, st>>>(reinterpret_cast<const uint8_t*>(blob) + NET::BLOB_OFF, io, M, g_dbg_timeline, sv);
+  long long* dbg = g_dbg_timeline_tag < 0 || g_dbg_timeline_tag == tag ? g_dbg_timeline : nullptr;
+  kern<<<grid, NET::threads(NET::WPS), bytes, st>>>(reinterpret_cast<const uint8_t*>(blob) + NET::BLOB_OFF, io, M, dbg, sv);
   NRT_CUDA(cudaGetLastError());
   return NRT_OK;
 }

@@ -1153,6 +1153,10 @@ __device__ __forceinline__ void stream_op(uint8_t* dst, const uint8_t* src, uint
 //     row is (up to the queue tail) spent on a live ray: this is the compaction of the sphere-trace march.
 template <class T, class = void> struct PackedPairsOf { static constexpr int value = 0; };
 template <class T> struct PackedPairsOf<T, std::void_t<decltype(T::kPackedPairs)>> { static constexpr int value = T::kPackedPairs; };
+// tile policies whose load() is a dependent global load followed by arithmetic can split it into fetch() (issue the loads
+// into a `Fetch` record) and point() (the arithmetic); k_mlp_tc with NRT_FIRST_PIPE fetches one tile ahead
+template <class T, class D, class = void> struct FetchOf { using type = D; };
+template <class T, class D> struct FetchOf<T, D, std::void_t<typename T::Fetch>> { using type = typename T::Fetch; };
 template <class T, class = void> struct HasCtaInit : std::false_type {};
 template <class T> struct HasCtaInit<T, std::void_t<decltype(&T::cta_init)>> : std::true_type {};
 template <class T, class = void> struct IsIterative : std::false_type {};
@@ -1220,6 +1224,16 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
   // is zero, so the phase GEMM skips the ZLO x_lo chunks that hold nothing else
   constexpr int kPP = (!ITER && !NET::SPLIT && !SV::kOn && !SV::kF32 && LAT == 0 && NET::ACT == NRT_ACT_LEAKY_RELU) ? PackedPairsOf<IO>::value : 0;
   constexpr int ZLO = (NRT_BIAS_MMA & 2) ? 2 * kPP / 16 : 0;
+  // NRT_FIRST_PIPE (NeRFLE.first's inference kernels, i.e. the render layout): the tile boundary leaves the per-slot chain.
+  // The next tile's inputs are fetched right after this tile's encoding was handed to the MMA warp, its encoding is
+  // computed while the output layer runs, and on the output `done` the epilogue reads the accumulator, stores that
+  // encoding and arrives on `ready` before it writes this tile's outputs: the next tile's init layer runs under the stores.
+#ifndef NRT_FIRST_PIPE
+#define NRT_FIRST_PIPE 1
+#endif
+  constexpr bool PIPE = NRT_FIRST_PIPE != 0 && NET::BIAS_ROWS && !ITER;
+  static_assert(!PIPE || (BMMA && NET::SPLIT && NET::ENC_CUDA && !NET::FUSE_OUT && !NET::INPLACE && LAT == 0 && WPS == 4),
+                "NRT_FIRST_PIPE: NeRFLE.first's render layout (split fp32 encoding, bias rows, an MMA output layer)");
   __shared__ volatile uint32_t s_slot_live[3];   // iterative policies: 0 once the slot's queue has run dry
   __shared__ uint32_t s_warp_live[3][4];
 
@@ -1505,6 +1519,113 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
         const long long t_start = clock64();
         while (clock64() - t_start < (long long)slot * NRT_SLOT_STAGGER) {}
       }
+      // development (NRT_DBG_BOUNDARY, tools/tc_timeline_nerf.py --first): the tile boundary in row 0 of the stamps --
+      // 3 output `done` seen, 4 outputs stored, 5 inputs in registers, 6 encoding stored, 7 `ready` arrived for the init layer
+#ifdef NRT_DBG_BOUNDARY
+      auto bstamp = [&](int it, int k) { if (lane_row == NRT_DBG_LANE) stamp(it, 0, slot, k); };
+      auto bstamp_dep = [&](int it, int k, float v) { if (lane_row == NRT_DBG_LANE && __float_as_uint(v) != 0xffffffffu) stamp(it, 0, slot, k); };
+#else
+      auto bstamp = [&](int, int) {};
+      auto bstamp_dep = [&](int, int, float) {};
+#endif
+      // ---- NRT_FIRST_PIPE: a tile's inputs fetched one tile ahead, its encoding computed in registers ----
+      struct Inputs { float v[IN + LAT]; };
+      using Pre = typename FetchOf<IO, Inputs>::type;
+      struct Enc { uint32_t ax[NET::KX / 2], ex[NET::XR / 2], sr[F / 2], cr[F / 2], sa[F / 2], ca[F / 2]; };
+      const int64_t tstride = (int64_t)gridDim.x * NSLOT;
+      Pre pre;                 // inputs of the slot's next tile (rows m >= M: not fetched, pre_ok false)
+      bool pre_ok = false;
+      auto fetch = [&](int64_t mm) {
+        if constexpr (PIPE) {
+          pre_ok = mm < M;    // (also false past the last tile: mm >= ntiles * 128 >= M)
+          if (pre_ok) {
+            if constexpr (std::is_same_v<Pre, Inputs>) io.load(mm, pre.v);
+            else io.fetch(mm, pre);
+          }
+        }
+      };
+      auto inputs = [&](float* xi) {
+        if (PIPE && pre_ok) {
+          if constexpr (std::is_same_v<Pre, Inputs>) {
+#pragma unroll
+            for (int j = 0; j < IN; ++j) xi[j] = pre.v[j];
+          } else io.point(pre, xi);
+        } else {
+#pragma unroll
+          for (int j = 0; j < IN; ++j) xi[j] = 0.0f;
+        }
+      };
+      // stages 0 and 1 of the loop below (the SPLIT, BIAS_ROWS and ENC_CUDA branches), the same operations in the same order
+      auto encode = [&](const float* xi, Enc& e) {
+        if constexpr (PIPE) {
+        uint16_t v[16];
+#pragma unroll
+        for (int j = 0; j < 16; ++j) v[j] = 0;
+        uint16_t a[2 * IN];
+#pragma unroll
+        for (int j = 0; j < IN; ++j) {
+          const uint16_t hi = E::cvt(xi[j]);
+          const uint16_t lo = E::cvt(xi[j] - E::back(hi));
+          v[j] = hi; v[IN + j] = lo; v[2 * IN + j] = hi;
+          const float ax_ = act_fast<NET::ACT>(xi[j]);
+          const uint16_t ahi = E::cvt(ax_);
+          a[j] = ahi; a[IN + j] = E::cvt(ax_ - E::back(ahi));
+        }
+#pragma unroll
+        for (int t = 0; t < 3; ++t) v[NET::BR.row + t] = one16<FMT>();
+#pragma unroll
+        for (int j = 0; j < NET::XR / 2; ++j) e.ex[j] = 0;
+#pragma unroll
+        for (int j = 0; j < NET::KX / 2; ++j) e.ax[j] = (uint32_t)v[2 * j] | ((uint32_t)v[2 * j + 1] << 16);
+#pragma unroll
+        for (int j = 0; j < IN; ++j) e.ex[j] = (uint32_t)a[2 * j] | ((uint32_t)a[2 * j + 1] << 16);
+#pragma unroll
+        for (int t = 0; t < 3; ++t) e.ex[(NET::BR.row + t) / 2] |= (uint32_t)one16<FMT>() << (16 * ((NET::BR.row + t) & 1));
+        const float* sB = sBias + Y.basis_f32_off;
+        uint32_t ph[F];
+#pragma unroll
+        for (int f = 0; f < F; ++f) {
+          float p = xi[0] * sB[f];
+#pragma unroll
+          for (int j = 1; j < IN; ++j) p = fmaf(xi[j], sB[j * NET::FP + f], p);
+          ph[f] = __float_as_uint(p);
+        }
+#pragma unroll
+        for (int j = 0; j < F / 2; ++j) {
+          float s0, c0, s1, c1;
+          sincos_fast(__uint_as_float(ph[2 * j]), &s0, &c0);
+          sincos_fast(__uint_as_float(ph[2 * j + 1]), &s1, &c1);
+          e.sr[j] = E::pack(s0, s1); e.cr[j] = E::pack(c0, c1);
+          e.sa[j] = E::pack(act_fast<NET::ACT>(s0), act_fast<NET::ACT>(s1));
+          e.ca[j] = E::pack(act_fast<NET::ACT>(c0), act_fast<NET::ACT>(c1));
+        }
+        }
+      };
+      auto enc_store = [&](const Enc& e) {
+        tmem_store<NET::KX / 2>(aU, e.ax);
+        tmem_store<NET::XR / 2>(aE, e.ex);
+        tmem_store<F / 2>(aU + NET::XR / 2, e.sr);
+        tmem_store<F / 2>(aU + NET::XR / 2 + F / 2, e.cr);
+        tmem_store<F / 2>(aE + NET::XR / 2, e.sa);
+        tmem_store<F / 2>(aE + NET::XR / 2 + F / 2, e.ca);
+      };
+      if constexpr (PIPE) {
+        // the slot's first tile: fetched, encoded and handed to the MMA warp here; later tiles in the previous tile's
+        // output stage
+        const int64_t tile = (int64_t)blockIdx.x * NSLOT + slot;
+        if (tile < ntiles) {
+          fetch(tile * 128 + lane_row);
+          float xi[IN];
+          inputs(xi);
+          Enc e;
+          encode(xi, e);
+          enc_store(e);
+          tc_wait_st();
+          tc_fence_before();
+          mbar_arrive(&bar_ready[slot]);
+          fetch((tile + tstride) * 128 + lane_row);
+        }
+      }
       for (int64_t t0 = (int64_t)blockIdx.x * NSLOT;; t0 += (int64_t)gridDim.x * NSLOT, ++it_dbg) {
         int64_t m = 0;
         bool valid;
@@ -1527,13 +1648,17 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           if (tile >= ntiles) { self_drain(); break; }
           m = tile * 128 + lane_row;
           valid = m < M;
-          if constexpr (kPP > 0) {
+          if constexpr (PIPE) {
+            // the tile's encoding is in TMEM already
+          } else if constexpr (kPP > 0) {
             if (valid && primary) io.load_packed(m, pw, x);
           } else {
             if (valid && primary) io.load(m, x);
+            if (valid) bstamp_dep(it_dbg, 5, x[0]);
           }
         }
-        if (!primary) {
+        if constexpr (PIPE) {
+        } else if (!primary) {
           // the helper half has no work before the first hidden layer: keep in phase with the barriers only
           if constexpr (!NET::ENC_CUDA) {
             mbar_arrive(&bar_ready[slot]);
@@ -1691,8 +1816,10 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           // (the raw-x segment keeps the phase-GEMM tile [x_hi | x_lo | x_hi | 0]; the init / skip weights
           //  of the third copy and of the padding are zero, see enc_ref_index)
           tc_wait_st();
+          bstamp(it_dbg, 6);
           tc_fence_before();
           mbar_arrive(&bar_ready[slot]);
+          bstamp(it_dbg, 7);
           self_issue();
         }
         }   // primary
@@ -1778,6 +1905,17 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           self_issue();
           }
         }
+        // ---- NRT_FIRST_PIPE: the next tile's encoding, under the output layer's MMAs ----
+        const bool has_next = PIPE && t0 + slot + tstride < ntiles;
+        Enc en;
+        if constexpr (PIPE) {
+          if (has_next) {
+            float xi[IN];
+            inputs(xi);
+            bstamp_dep(it_dbg + 1, 5, xi[0]);
+            encode(xi, en);
+          }
+        }
         // ---- output layer ----
         if (!primary) {
           mbar_wait(&bar_done[slot], n_done & 1); n_done++;
@@ -1807,13 +1945,30 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           tc_fence_after();
           constexpr int OC = (NET::OUT + 7) / 8 * 8;
           uint32_t acc[OC];
+          bstamp(it_dbg, 3);
           tmem_load<OC>(dD, acc);
-          tc_wait_ld();
+          if constexpr (PIPE) {
+            // the output MMAs have read the last hidden activations: the next tile's encoding goes into the union and
+            // encoding regions, and once the accumulator is in registers its init layer may overwrite it
+            if (has_next) enc_store(en);
+            tc_wait_ld();
+            if (has_next) {
+              tc_wait_st();
+              bstamp(it_dbg + 1, 6);
+              tc_fence_before();
+              mbar_arrive(&bar_ready[slot]);
+              bstamp(it_dbg + 1, 7);
+              fetch((t0 + slot + 2 * tstride) * 128 + lane_row);
+            }
+          } else {
+            tc_wait_ld();
+          }
           float o[NET::OUT];   // bias already accumulated (pre-loaded into the accumulator)
 #pragma unroll
           for (int j = 0; j < NET::OUT; ++j) o[j] = __uint_as_float(acc[j]);
           if constexpr (ITER) { if (valid) io.consume(state, o); }
           else { if (valid) io.store(m, o); }
+          bstamp(it_dbg, 4);
           // the accumulator / operand regions of this slot may now be reused by the next tile
           tc_fence_before();
         }
