@@ -363,6 +363,18 @@ int nrt_nerfle_render_camera(const nrt_mlp_t* first, const nrt_mlp_t* second, in
  * chunk's rays into the workspace before the chunk's first pass; 1 = the MLP kernels compute every sample's ray from the camera
  * in their prologues (no ray array; bit-identical image; measured 2.5-3 % slower on B200, see DESIGN.md section 8).  Process-wide. */
 int nrt_set_camera_rays_mode(int fused);
+/* The render's pass without its compositing: the per-sample values nrt_nerfle_render / nrt_nerfle_render_camera
+ * composite, from the same code (the same chunks of 262,144 rays, the same kernels, the same camera-fed selection), for
+ * tests and for callers that composite themselves.  Exactly one of rays [R,6] / cam (R = the camera's ray count; the view
+ * of a ray is its camera view, view_of_ray must be NULL); exactly one of ts [S] (shared) / ts_per_ray [R,S].
+ * Out: out_sigma [R,S] (pre-relu density), out_rgb [R,S,3] (sigmoid), RAY-major (m = ray * S + s).
+ * workspace: nrt_nerfle_render_samples_workspace bytes (cam: the same descriptor, or NULL for rays). */
+size_t nrt_nerfle_render_samples_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, int64_t R, int S,
+                                           const nrt_camera_t* cam);
+int nrt_nerfle_render_samples(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                              const nrt_camera_t* cam, int64_t R, const float* ts, const float* ts_per_ray, int S,
+                              const float* light_code, int light_dim, const int32_t* view_of_ray, float* out_sigma,
+                              float* out_rgb, void* workspace, size_t workspace_bytes, void* stream);
 /* Host-image variant: nothing but the camera goes in, the image comes back to (pinned) host memory; synchronises. */
 int nrt_nerfle_render_camera_host(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
                                   const nrt_camera_t* cam, const float* ts_host, int S,

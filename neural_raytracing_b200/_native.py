@@ -123,7 +123,10 @@ SIGNATURES = {
     "nrt_set_camera_rays_mode": (c_int, [c_int]),
     "nrt_nerfle_render_camera_workspace": (c_sz, [_PM, _PM, c_int, _PC, _PN]),
     "nrt_nerfle_render_camera": (c_int, [_PM, _PM, c_int, _PC, c_vp, _PN, c_vp, c_int, c_vp, c_vp, c_sz, c_vp]),
-    "nrt_nerfle_render_camera_host": (c_int, [_PM, _PM, c_int, _PC, c_vp, c_int, _PN, c_vp, c_int, c_vp, c_vp]),
+    "nrt_nerfle_render_samples_workspace": (c_sz, [_PM, _PM, c_int, c_i64, c_int, _PC]),
+    "nrt_nerfle_render_samples": (c_int, [_PM, _PM, c_int, c_vp, _PC, c_i64, c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp,
+                                          c_vp, c_sz, c_vp]),
+    "nrt_nerfle_render_camera_host":(c_int, [_PM, _PM, c_int, _PC, c_vp, c_int, _PN, c_vp, c_int, c_vp, c_vp]),
     "nrt_sdf_lattice_eval_workspace": (c_i64, [_PG]),
     "nrt_sdf_lattice_eval": (c_int, [_PS, c_int, _PG, c_vp, c_vp, c_sz, c_vp]),
     "nrt_isosurface_workspace": (c_i64, [_PG]),

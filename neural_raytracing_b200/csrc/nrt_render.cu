@@ -390,19 +390,27 @@ int nrt_camera_rays_dev(const nrt_camera_t* cam, int64_t r0, int64_t n, float* o
                         cudaStream_t st);
 
 // the render of R rays given either as an array (rays) or as a camera (cam: every chunk's rays are generated into the
-// tail of the workspace right before its first pass; SURVEY f4)
+// tail of the workspace right before its first pass; SURVEY f4).
+// Per-sample mode (nrt_nerfle_render_samples): smp_sigma [R,Sc] / smp_rgb [R,Sc,3] not NULL, n_fine = 0 -- every chunk's
+// pass stores its per-sample values there instead of the workspace and nothing is composited; ts_per_ray [R,Sc], when not
+// NULL, gives every ray its own distances in place of ts / the stratified ones.
 static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
                        const nrt_camera_t* cam, int64_t R, const float* ts, const nrt_nerf_sampling_t* sampling,
                        const float* light_code, int light_dim, const int32_t* view_of_ray,
-                       float* out_rgb, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+                       float* out_rgb, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                       const float* ts_per_ray = nullptr, float* smp_sigma = nullptr, float* smp_rgb = nullptr) {
   NRT_REQUIRE(R >= 0, "nrt_nerfle_render: negative R");
   if (R == 0) return NRT_OK;
-  NRT_REQUIRE((rays != nullptr || cam != nullptr) && out_rgb != nullptr, "nrt_nerfle_render: null rays/out");
+  const bool samples = smp_sigma != nullptr;
+  NRT_REQUIRE((rays != nullptr || cam != nullptr) && (out_rgb != nullptr || (samples && smp_rgb != nullptr)),
+              "nrt_nerfle_render: null rays/out");
   NRT_REQUIRE(sampling != nullptr, "nrt_nerfle_render: sampling descriptor is NULL");
   const int Sc = sampling->n_coarse, Sf = sampling->n_fine;
   const bool jitter = sampling->jitter_seed != 0;
   NRT_REQUIRE(Sc >= 1 && Sf >= 0, "nrt_nerfle_render: bad sample counts %d/%d", Sc, Sf);
-  NRT_REQUIRE(ts != nullptr || sampling->t_far > sampling->t_near, "nrt_nerfle_render: need ts or t_near<t_far");
+  NRT_REQUIRE(ts != nullptr || ts_per_ray != nullptr || sampling->t_far > sampling->t_near,
+              "nrt_nerfle_render: need ts or t_near<t_far");
+  NRT_REQUIRE(!samples || Sf == 0, "nrt_nerfle_render: per-sample outputs of a single pass only");
   NRT_REQUIRE(Sf == 0 || Sc >= 3, "hierarchical sampling needs n_coarse >= 3");
   const int64_t C = std::min<int64_t>(R, kRayChunk);
   const size_t need = nrt_nerfle_render_workspace(first, second, prec, R, sampling) + (cam ? cam_scratch_bytes(C) : 0);
@@ -445,16 +453,24 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
       const int rcc = nrt_camera_rays_dev(cam, r0, n, cam_rays, cam_view, st);
       if (rcc != NRT_OK) return rcc;
     }
-    float* c_out = out_rgb + r0 * 3;
+    float* c_out = samples ? nullptr : out_rgb + r0 * 3;
     const float* ts_shared = ts;
     const float* ts_pr = nullptr;
-    if (jitter || ts == nullptr) {
+    if (ts_per_ray) {
+      ts_shared = nullptr; ts_pr = ts_per_ray + r0 * Sc;
+    } else if (jitter || ts == nullptr) {
       // per-ray (stratified) distances; without jitter this is the bin-centre grid
       const int rs = launch_stratified(n, r0, Sc, sampling, nullptr, ts_c, st);
       if (rs != NRT_OK) return rs;
       ts_shared = nullptr; ts_pr = ts_c;
     }
     int rc;
+    if (samples) {
+      rc = nerf_pass(first, second, prec, c_rays, n, ts_shared, ts_pr, Sc, light_code, light_dim, c_view, nullptr,
+                     smp_sigma + r0 * Sc, smp_rgb + r0 * Sc * 3, tcws, tcws_bytes, st, kcam, r0);
+      if (rc != NRT_OK) return rc;
+      continue;
+    }
     if (!store_c) {
       rc = nerf_pass(first, second, prec, c_rays, n, ts_shared, ts_pr, Sc, light_code, light_dim, c_view, c_out,
                      nullptr, nullptr, tcws, tcws_bytes, st, kcam, r0);
@@ -581,6 +597,38 @@ extern "C" int nrt_nerfle_render_camera(const nrt_mlp_t* first, const nrt_mlp_t*
   if (rc != NRT_OK) return rc;
   return render_impl(first, second, prec, nullptr, cam, R, ts, sampling, light_code, light_dim, nullptr, out_rgb,
                      workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- the render's pass with its per-sample values as the output (what k_merge_composite would composite) ----------
+extern "C" size_t nrt_nerfle_render_samples_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
+                                                      int64_t R, int S, const nrt_camera_t* cam) {
+  if (R < 0 || S < 1) return 0;
+  const nrt_nerf_sampling_t samp{S, 0, 0.0f, 0.0f, 0};
+  return nrt_nerfle_render_workspace(first, second, prec, R, &samp) +
+         (cam ? cam_scratch_bytes(std::min<int64_t>(R, kRayChunk)) : 0);
+}
+
+extern "C" int nrt_nerfle_render_samples(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                         const nrt_camera_t* cam, int64_t R, const float* ts, const float* ts_per_ray,
+                                         int S, const float* light_code, int light_dim, const int32_t* view_of_ray,
+                                         float* out_sigma, float* out_rgb, void* workspace, size_t workspace_bytes,
+                                         void* stream) {
+  NRT_REQUIRE(R >= 0, "nrt_nerfle_render_samples: negative R");
+  NRT_REQUIRE((rays != nullptr) != (cam != nullptr), "nrt_nerfle_render_samples: exactly one of rays / cam must be given");
+  if (cam) {
+    int64_t Rc = 0;
+    const int rc = nrt_check_camera(cam, &Rc);
+    if (rc != NRT_OK) return rc;
+    NRT_REQUIRE(R == Rc, "nrt_nerfle_render_samples: R = %lld but the camera has %lld rays", (long long)R, (long long)Rc);
+    NRT_REQUIRE(view_of_ray == nullptr, "nrt_nerfle_render_samples: a camera gives every ray its view; view_of_ray must be NULL");
+  }
+  NRT_REQUIRE(S >= 1, "nrt_nerfle_render_samples: bad sample count %d", S);
+  NRT_REQUIRE((ts != nullptr) != (ts_per_ray != nullptr), "nrt_nerfle_render_samples: exactly one of ts / ts_per_ray must be given");
+  if (R == 0) return NRT_OK;
+  NRT_REQUIRE(out_sigma != nullptr && out_rgb != nullptr, "nrt_nerfle_render_samples: null out_sigma/out_rgb");
+  const nrt_nerf_sampling_t samp{S, 0, 0.0f, 0.0f, 0};
+  return render_impl(first, second, prec, rays, cam, R, ts, &samp, light_code, light_dim, view_of_ray, nullptr, workspace,
+                     workspace_bytes, (cudaStream_t)stream, ts_per_ray, out_sigma, out_rgb);
 }
 
 // The host-buffer entry point keeps grow-only device scratch PER DEVICE (a stream-ordered pool would hand the memory

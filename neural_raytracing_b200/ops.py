@@ -842,6 +842,43 @@ def nerfle_render_camera(first: PackedMLP, second: PackedMLP, cam: CameraDesc, t
     return out
 
 
+def nerfle_render_samples(first: PackedMLP, second: PackedMLP, rays_or_cam, ts: torch.Tensor, light_code: torch.Tensor,
+                          view_of_ray: Optional[torch.Tensor] = None, prec=PREC_F32):
+    """The per-sample values the render composites (nrt_nerfle_render_samples: the render's own chunks and kernels):
+    rays [...,6] or a CameraDesc, ts [S] (shared) or [R,S] (per ray) -> sigma [R,S] (pre-relu), rgb [R,S,3] (sigmoid),
+    ray-major.  A camera picks the light-code row of every ray from its view and takes the camera-fed kernels when
+    set_camera_rays_mode(True) selected them, as nerfle_render_camera does."""
+    prec = prec_id(prec)
+    cam = rays_or_cam if isinstance(rays_or_cam, CameraDesc) else None
+    if cam is not None:
+        r2, R, dev = None, cam.n_rays, cam.device
+        if view_of_ray is not None:
+            raise NrtError("a camera gives every ray its view; view_of_ray must be None")
+    else:
+        r2 = _chk(rays_or_cam, "rays").reshape(-1, 6)
+        R, dev = r2.shape[0], r2.device
+    per_ray = ts.dim() == 2
+    t = _chk(ts, "ts")
+    if per_ray and t.shape[0] != R:
+        raise NrtError("ts [R,S] has %d rows for %d rays" % (t.shape[0], R))
+    S = t.shape[-1] if per_ray else t.numel()
+    lc = _chk(light_code, "light_code")
+    lc = lc.reshape(-1, lc.shape[-1])
+    vor = _chk(view_of_ray.reshape(-1), "view_of_ray", torch.int32) if view_of_ray is not None else None
+    sigma = torch.empty((R, S), dtype=torch.float32, device=dev)
+    rgb = torch.empty((R, S, 3), dtype=torch.float32, device=dev)
+    cs = ctypes.byref(cam.struct) if cam is not None else None
+    with torch.cuda.device(dev):
+        c1, c2 = first.c_struct(prec), second.c_struct(prec)
+        ws = _cached_ws(_ws_cache, dev, N.lib().nrt_nerfle_render_samples_workspace(ctypes.byref(c1), ctypes.byref(c2), prec,
+                                                                                     R, S, cs))
+        N.check(N.lib().nrt_nerfle_render_samples(ctypes.byref(c1), ctypes.byref(c2), prec, _ptr(r2), cs, R,
+                                                  None if per_ray else _ptr(t), _ptr(t) if per_ray else None, S, _ptr(lc),
+                                                  lc.shape[-1], _ptr(vor), _ptr(sigma), _ptr(rgb), _ptr(ws), ws.numel(),
+                                                  _stream()))
+    return sigma, rgb
+
+
 def nerfle_render_camera_host(first: PackedMLP, second: PackedMLP, cam: CameraDesc, ts_host: Optional[torch.Tensor],
                               light_code: torch.Tensor, out_host: torch.Tensor, prec=PREC_F32, n_coarse=None,
                               n_fine=0, t_near=0.0, t_far=0.0, jitter_seed=0):

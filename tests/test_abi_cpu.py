@@ -71,3 +71,32 @@ def test_product_never_imports_oracle():
                 txt = open(os.path.join(dp, fn)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", txt, flags=re.M), fn
                 assert "nrt_oracle" not in txt.replace("oracle/c/nrt_oracle.c", ""), fn
+
+
+def test_render_samples_export_and_argument_checks():
+    """nrt_nerfle_render_samples is exported and rejects malformed calls before touching a device"""
+    import ctypes as C
+    from neural_raytracing_b200 import _native as N
+    L = N.lib()
+    assert "nrt_nerfle_render_samples" in _declared_symbols()
+    assert "nrt_nerfle_render_samples_workspace" in _declared_symbols()
+    m = N.NrtMlp(3, 0, 16, 128, 5, 3, 65, 0, None, None, None)
+    buf = (C.c_float * 64)()
+    p = C.cast(buf, C.c_void_p)
+
+    def call(rays, cam, R, ts, ts_pr, S, sig=p, rgb=p):
+        return L.nrt_nerfle_render_samples(C.byref(m), C.byref(m), N.PREC_F16, rays, cam, R, ts, ts_pr, S, p, 3, None,
+                                           sig, rgb, p, 256, None)
+    cases = [((None, None, 4, p, None, 8), "exactly one of rays / cam"),
+             ((p, None, -1, p, None, 8), "negative R"),
+             ((p, None, 4, p, p, 8), "exactly one of ts / ts_per_ray"),
+             ((p, None, 4, None, None, 8), "exactly one of ts / ts_per_ray"),
+             ((p, None, 4, p, None, 0), "bad sample count")]
+    for args, msg in cases:
+        assert call(*args) == N.E_INVALID
+        assert msg in L.nrt_last_error().decode(), L.nrt_last_error()
+    assert call(p, None, 4, p, None, 8, sig=None) == N.E_INVALID
+    assert "null out_sigma/out_rgb" in L.nrt_last_error().decode()
+    cam = N.NrtCamera()                 # NRT_CAM_NERF with no views: validated as the camera render validates it
+    assert call(None, C.byref(cam), 4, p, None, 8) == N.E_INVALID
+    assert "bad block" in L.nrt_last_error().decode()
