@@ -184,6 +184,16 @@ struct IoNerfSecond {
 #pragma unroll
     for (int j = 0; j < LD; ++j) v[NLAT + 3 + j] = __ldg(light_code + (int64_t)view * LD + j);
   }
+  // load_packed in two pieces (k_mlp_tc, NRT_SECOND_PIPE): the packed latent of a whole tile is one contiguous block of
+  // NLAT / 8 * 128 uint4 (copied to shared memory one tile ahead), and the 3 + LD floats of direction and light code
+  __device__ __forceinline__ const uint4* packed_tile(int64_t tile) const {
+    return reinterpret_cast<const uint4*>(latent) + tile * (int64_t)(NLAT / 8 * 128);
+  }
+  __device__ __forceinline__ void load_dir_code(int64_t m, float* v) const {
+    const int view = dir_and_view(ray_of(m, S, s_shift), v);
+#pragma unroll
+    for (int j = 0; j < LD; ++j) v[3 + j] = __ldg(light_code + (int64_t)view * LD + j);
+  }
   __device__ __forceinline__ void store(int64_t m, const float* o) const {
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
@@ -428,7 +438,7 @@ __global__ void k_scan_argmin(const float* __restrict__ val, const float* __rest
 
 template <class NET, class IO, int FMT, class SV = NoSave>
 static int launch(const void* blob, const IO& io, int64_t M, cudaStream_t st, int tag = TAG_TC_MLP, SV sv = SV{}) {
-  const size_t bytes = (size_t)NET::SMEM_BYTES + 256;
+  const size_t bytes = (size_t)SecondPipe<NET, IO, SV>::SMEM_BYTES + 256;
   auto kern = k_mlp_tc<NET, IO, FMT, SV>;
   NRT_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
   const int64_t ntiles = (M + 127) / 128;

@@ -862,6 +862,21 @@ __device__ __forceinline__ void convert_row_out(uint32_t dD, const float* __rest
   if constexpr (SAVE) save_row[tile_elem(H)] = one16<FMT>();
 }
 
+// convert_row_out's leaky-relu form on an accumulator row already in registers (NRT_SECOND_PIPE), same operation order
+template <int H, int OUT>
+__device__ __forceinline__ void out_from_regs(const uint32_t* acc, const float* __restrict__ wout, float* __restrict__ o) {
+#pragma unroll
+  for (int k = 0; k < H; ++k) {
+    float a = __uint_as_float(acc[k]);
+    a = fmaxf(a, 0.01f * a);
+    const float4 w = *reinterpret_cast<const float4*>(wout + k * 4);
+    o[0] = fmaf(a, w.x, o[0]);
+    if constexpr (OUT > 1) o[1] = fmaf(a, w.y, o[1]);
+    if constexpr (OUT > 2) o[2] = fmaf(a, w.z, o[2]);
+    if constexpr (OUT > 3) o[3] = fmaf(a, w.w, o[3]);
+  }
+}
+
 // Training forward with a tensor-core forward and the fused fp32 backward (256-wide nets, NeuralBSDF, occlusion MLP):
 // the forward kernel also writes the post-activation layer inputs in the layout of
 // the fused fp32 backward (nrt_mlp_backward: acts[(l * H + k) * M + m], fp32) -- the values the next layer's operand
@@ -1165,6 +1180,30 @@ struct NoState {};
 template <class T, class = void> struct StateOf { using type = NoState; };
 template <class T> struct StateOf<T, std::void_t<typename T::State>> { using type = typename T::State; };
 
+// NRT_SECOND_PIPE (NeRFLE.second's point-light inference kernels: IoNerfSecond with the packed 16-bit latent, in-place
+// TMEM plan, fused output layer, three slots): the tile boundary leaves the per-slot chain.  A slot copies its next tile's
+// packed latent (one contiguous block) into a shared-memory buffer of its own one tile ahead; after the last hidden layer's
+// `ready` the epilogue writes the next tile's raw x_hi into the encoding region (dead once the last skip layer has run), on
+// the last layer's `done` it reads the accumulator, writes the next tile's x_lo chunk into the union region and arrives,
+// so the next tile's phase GEMM runs under this tile's fused output layer; then the next tile's sin / cos and its init
+// `ready`, and only then this tile's stores.  Same TMEM words, same MMAs in the same order: bit-identical outputs.
+#ifndef NRT_SECOND_PIPE
+#define NRT_SECOND_PIPE 1
+#endif
+template <class NET, class IO, class SV>
+struct SecondPipe {
+  static constexpr int kPP = (!IsIterative<IO>::value && !NET::SPLIT && !SV::kOn && !SV::kF32 && NET::LAT == 0 &&
+                              NET::ACT == NRT_ACT_LEAKY_RELU) ? PackedPairsOf<IO>::value : 0;
+  static constexpr bool ON = NRT_SECOND_PIPE != 0 && kPP > 0 && (NRT_BIAS_MMA & 2) != 0 && NET::INPLACE && NET::FUSE_OUT &&
+                             !NET::ENC_CUDA && NET::BIAS_MMA && !NET::KSPLIT && NET::WPS == 4 && !NET::STREAM && NET::NSLOT == 3;
+  static constexpr int LAT_BYTES = kPP * 4 * 128;                 // one tile's packed latent
+  static constexpr int LAT_OFF = (NET::SMEM_BYTES + 127) / 128 * 128;   // per-slot buffers after the resident blob
+  static constexpr int BAR_OFF = LAT_OFF + NET::NSLOT * LAT_BYTES;       // then one mbarrier per slot
+  static constexpr int SMEM_BYTES = ON ? BAR_OFF + 8 * NET::NSLOT : NET::SMEM_BYTES;
+  static_assert(!ON || SMEM_BYTES <= kSmemBudget, "NRT_SECOND_PIPE: latent buffers do not fit next to the blob");
+  static_assert(!ON || (NET::XR / 2 >= kPP + 4 && NET::XR / 2 - kPP == 8), "NRT_SECOND_PIPE: one x chunk after the latent");
+};
+
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
@@ -1234,6 +1273,11 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
   constexpr bool PIPE = NRT_FIRST_PIPE != 0 && NET::BIAS_ROWS && !ITER;
   static_assert(!PIPE || (BMMA && NET::SPLIT && NET::ENC_CUDA && !NET::FUSE_OUT && !NET::INPLACE && LAT == 0 && WPS == 4),
                 "NRT_FIRST_PIPE: NeRFLE.first's render layout (split fp32 encoding, bias rows, an MMA output layer)");
+  // NRT_SECOND_PIPE (see SecondPipe): NeRFLE.second's point-light kernels
+  using SP = SecondPipe<NET, IO, SV>;
+  constexpr bool PIPE2 = SP::ON && WPS == 4 && BMMA;
+  static_assert(!PIPE2 || (SP::kPP == kPP && ZLO == 2 * kPP / 16 && !PIPE && NET::H == 64 && NET::OUT <= 4),
+                "NRT_SECOND_PIPE: packed latent, skipped x_lo chunks, fused 64-wide output layer");
   __shared__ volatile uint32_t s_slot_live[3];   // iterative policies: 0 once the slot's queue has run dry
   __shared__ uint32_t s_warp_live[3][4];
 
@@ -1260,6 +1304,9 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
     for (int s = 0; s < 3; ++s) {
       mbar_init(&bar_ready[s], EPI); mbar_init(&bar_done[s], 1); mbar_init(&bar_ready_a[s], EPI);
       mbar_init(&bar_wfull[s][0], 1); mbar_init(&bar_wfull[s][1], 1);
+    }
+    if constexpr (PIPE2) {
+      for (int s = 0; s < NSLOT; ++s) mbar_init(reinterpret_cast<uint64_t*>(smem + SP::BAR_OFF) + s, 1);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -1609,6 +1656,101 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
         tmem_store<F / 2>(aE + NET::XR / 2, e.sa);
         tmem_store<F / 2>(aE + NET::XR / 2 + F / 2, e.ca);
       };
+      // ---- NRT_SECOND_PIPE: a tile's packed latent staged in shared memory one tile ahead, its x_hi / x_lo written ----
+      // ---- under the previous tile's last layers, its phase GEMM issued under that tile's fused output layer     ----
+      constexpr int kDV = IN - 2 * kPP;              // direction + light code floats after the packed latent
+      constexpr int kXLO = NET::XR / 2 - kPP;        // words of the one x_lo chunk the phase GEMM reads
+      uint64_t* const lat_bar = reinterpret_cast<uint64_t*>(smem + SP::BAR_OFF) + slot;
+      uint4* const s_lat = reinterpret_cast<uint4*>(smem + SP::LAT_OFF + (size_t)slot * SP::LAT_BYTES);
+      uint32_t n_lat = 0;
+      // one thread of the slot copies tile tl's packed latent into the slot's buffer.  Every thread of the slot has read
+      // the buffer's previous contents before it arrived on `ready` for the phase GEMM whose `done` this thread has seen.
+      auto lat_prefetch = [&](int64_t tl) {
+        if constexpr (PIPE2) {
+          if (lane_row == 0 && tl < ntiles) {
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            mbar_expect_tx(lat_bar, (uint32_t)SP::LAT_BYTES);
+            bulk_g2s(s_lat, io.packed_tile(tl), (uint32_t)SP::LAT_BYTES, lat_bar);
+          }
+        }
+      };
+      auto dir_code = [&](int64_t mm, float* dv) {
+        if constexpr (PIPE2) {
+          if (mm < M) io.load_dir_code(mm, dv);
+          else {
+#pragma unroll
+            for (int j = 0; j < kDV; ++j) dv[j] = 0.0f;
+          }
+        }
+      };
+      // raw x_hi of row mm into the encoding region (the in-place plan's stage-0 stores: latent words as handed over, the
+      // other inputs packed; rows m >= M zero), and the words of its x_lo chunk into lx
+      auto x_store = [&](int64_t mm, const float* dv, uint32_t* lx) {
+        if constexpr (PIPE2) {
+          mbar_wait(lat_bar, n_lat & 1); n_lat++;
+          const bool ok = mm < M;
+          uint32_t ax[NET::XR / 2];
+#pragma unroll
+          for (int j = 0; j < kPP / 4; ++j) {
+            const uint4 q = s_lat[j * 128 + lane_row];
+            ax[4 * j] = ok ? q.x : 0u; ax[4 * j + 1] = ok ? q.y : 0u; ax[4 * j + 2] = ok ? q.z : 0u; ax[4 * j + 3] = ok ? q.w : 0u;
+          }
+#pragma unroll
+          for (int j = kPP; j < NET::XR / 2; ++j) {
+            ax[j] = 0u; lx[j - kPP] = 0u;
+            if (j < (IN + 1) / 2) {
+              const float xa = dv[2 * j - 2 * kPP], xb = (2 * j + 1 < IN) ? dv[2 * j + 1 < IN ? 2 * j + 1 - 2 * kPP : 0] : 0.0f;
+              ax[j] = E::pack(xa, xb);
+              const float ha = E::back((uint16_t)(ax[j] & 0xffffu)), hb = E::back((uint16_t)(ax[j] >> 16));
+              lx[j - kPP] = E::pack(xa - ha, xb - hb);
+            }
+          }
+          tmem_store<NET::XR / 2>(aE, ax);
+        }
+      };
+      // on the phase GEMM's `done`: sin / cos of the phases into the encoding region, `ready` for the init layer
+      auto enc_phase = [&](int it) {
+        if constexpr (PIPE2) {
+          mbar_wait(&bar_done[slot], n_done & 1); n_done++;
+          tc_fence_after();
+          uint32_t ph[F];
+          tmem_load<F>(dD, ph);
+          tc_wait_ld();
+          uint32_t sr[F / 2], cr[F / 2];
+#pragma unroll
+          for (int j = 0; j < F / 2; ++j) {
+            float s0, c0, s1, c1;
+            sincos_fast(__uint_as_float(ph[2 * j]), &s0, &c0);
+            sincos_fast(__uint_as_float(ph[2 * j + 1]), &s1, &c1);
+            sr[j] = E::pack(s0, s1); cr[j] = E::pack(c0, c1);
+          }
+          tmem_store<F / 2>(aE + NET::XR / 2, sr);
+          tmem_store<F / 2>(aE + NET::XR / 2 + F / 2, cr);
+          tc_wait_st();
+          bstamp(it, 6);
+          tc_fence_before();
+          mbar_arrive(&bar_ready[slot]);
+          bstamp(it, 7);
+        }
+      };
+      if constexpr (PIPE2) {
+        // the slot's first tile: its inputs and encoding here; later tiles in the previous tile's last stages
+        const int64_t tile = (int64_t)blockIdx.x * NSLOT + slot;
+        if (tile < ntiles) {
+          lat_prefetch(tile);
+          const int64_t m0 = tile * 128 + lane_row;
+          float dv[kDV > 0 ? kDV : 1];
+          uint32_t lx[kXLO];
+          dir_code(m0, dv);
+          x_store(m0, dv, lx);
+          tmem_store<kXLO>(aU + kPP, lx);
+          tc_wait_st();
+          tc_fence_before();
+          mbar_arrive(&bar_ready[slot]);
+          enc_phase(0);
+          lat_prefetch(tile + tstride);
+        }
+      }
       if constexpr (PIPE) {
         // the slot's first tile: fetched, encoded and handed to the MMA warp here; later tiles in the previous tile's
         // output stage
@@ -1648,16 +1790,17 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           if (tile >= ntiles) { self_drain(); break; }
           m = tile * 128 + lane_row;
           valid = m < M;
-          if constexpr (PIPE) {
-            // the tile's encoding is in TMEM already
+          if constexpr (PIPE || PIPE2) {
+            // the tile's encoding is in TMEM already (NRT_SECOND_PIPE: its phase GEMM has run, its init layer is issued)
           } else if constexpr (kPP > 0) {
             if (valid && primary) io.load_packed(m, pw, x);
+            if (valid) bstamp_dep(it_dbg, 5, x[IN - 1]);
           } else {
             if (valid && primary) io.load(m, x);
             if (valid) bstamp_dep(it_dbg, 5, x[0]);
           }
         }
-        if constexpr (PIPE) {
+        if constexpr (PIPE || PIPE2) {
         } else if (!primary) {
           // the helper half has no work before the first hidden layer: keep in phase with the barriers only
           if constexpr (!NET::ENC_CUDA) {
@@ -1825,6 +1968,11 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
         }   // primary
         // ---- stages 2 .. L+1: hidden activations ----
         constexpr int NHID = NET::FUSE_OUT ? L : L + 1;   // epilogues that feed another MMA stage
+        // NRT_SECOND_PIPE: the next tile's direction / light code and x_lo words, held from the last hidden stages on
+        const bool has_next2 = PIPE2 && t0 + slot + tstride < ntiles;
+        const int64_t m_next = (t0 + slot + tstride) * 128 + lane_row;
+        float dv_next[kDV > 0 ? kDV : 1];
+        uint32_t lx_next[kXLO > 0 ? kXLO : 1];
 #pragma unroll 1
         for (int st = 0; st < NHID; ++st) {
           estamp(2 + st, 3);
@@ -1903,6 +2051,14 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           mbar_arrive(&bar_ready[slot]);
           estamp(2 + st, 7);
           self_issue();
+          if constexpr (PIPE2) {
+            if (has_next2) {
+              // under stage 8's MMAs: the next tile's direction and light code; after the last skip layer (stage 8) has
+              // been seen done, the encoding region is dead: the next tile's x_hi goes in while stage 9 runs
+              if (st == NHID - 2) { dir_code(m_next, dv_next); bstamp_dep(it_dbg + 1, 5, dv_next[0]); }
+              if (st == NHID - 1) x_store(m_next, dv_next, lx_next);
+            }
+          }
           }
         }
         // ---- NRT_FIRST_PIPE: the next tile's encoding, under the output layer's MMAs ----
@@ -1921,10 +2077,41 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
           mbar_wait(&bar_done[slot], n_done & 1); n_done++;
           tc_fence_after();
           tc_fence_before();
+        } else if constexpr (PIPE2) {
+          // stage 9's `done`: the accumulator into registers and the next tile's x_lo chunk into the union region (both
+          // dead now), then `ready` -- the next tile's phase GEMM runs under this tile's output layer
+          mbar_wait(&bar_done[slot], n_done & 1); n_done++;
+          tc_fence_after();
+          bstamp(it_dbg, 3);
+          // (the phase GEMM writes accumulator columns 0 .. 15 only: the second half is read under it, as convert_row_out
+          //  reads it under the first half's arithmetic; nothing overwrites it before the next tile's init `ready`)
+          static_assert(Y.opN[0] <= H / 2, "phase GEMM within the first half of the accumulator");
+          uint32_t acc[2][H / 2];
+          tmem_load<H / 2>(dD, acc[0]);
+          if (has_next2) tmem_store<kXLO>(aU + kPP, lx_next);
+          tc_wait_ld();
+          if (has_next2) {
+            tc_wait_st();
+            tc_fence_before();
+            mbar_arrive(&bar_ready[slot]);
+          }
+          tmem_load<H / 2>(dD + H / 2, acc[1]);
+          float o[NET::OUT];
+#pragma unroll
+          for (int j = 0; j < NET::OUT; ++j) o[j] = sBias[s_bias[NET::STAGES - 1] + j];
+          out_from_regs<H / 2, NET::OUT>(acc[0], sBias + Y.wout_f32_off, o);
+          tc_wait_ld();
+          out_from_regs<H / 2, NET::OUT>(acc[1], sBias + Y.wout_f32_off + 4 * (H / 2), o);
+          if (has_next2) enc_phase(it_dbg + 1);
+          if (valid) io.store(m, o);
+          bstamp(it_dbg, 4);
+          if (has_next2) lat_prefetch(t0 + slot + 2 * tstride);
+          tc_fence_before();
         } else if constexpr (NET::FUSE_OUT) {
           // last hidden activations and the (tiny) output layer in one pass, fp32 on the CUDA cores
           mbar_wait(&bar_done[slot], n_done & 1); n_done++;
           tc_fence_after();
+          bstamp(it_dbg, 3);
           float o[NET::OUT];
 #pragma unroll
           for (int j = 0; j < NET::OUT; ++j) o[j] = sBias[s_bias[NET::STAGES - 1] + j];
@@ -1939,6 +2126,7 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
             convert_row_out<NET::ACT, FMT, H, NET::OUT, false, kPipeRow || (NRT_SOFTPLUS_POLY != 0)>(dD, sBias + Y.wout_f32_off, o);
           if constexpr (ITER) { if (valid) io.consume(state, o); }
           else { if (valid) io.store(m, o); }
+          bstamp(it_dbg, 4);
           tc_fence_before();
         } else {
           mbar_wait(&bar_done[slot], n_done & 1); n_done++;

@@ -10,7 +10,10 @@ times, reads `ms_per_step` and the per-kernel `kernel_ms` of every JSON line, an
 spread between its own runs ((max - min) / median) and the change of the new build against the base.  Every build,
 including the `--extra` ones, also runs once with `--dump-outputs`, and the frames are compared with the base build's:
 max-abs and RMS difference, and whether they are bit-identical.  The GPU name, its power limit and SM clocks are read
-in the same run.  Writes ab.json and the dumped frames under --out (default: a new temporary directory)."""
+in the same run.  Writes ab.json and the dumped frames under --out (default: a new temporary directory).
+
+The same A/B serves the other compile-time switches of the NeRFLE kernels, with the base build tagged by convention:
+fp0 = NRT_EXTRA_NVCC_FLAGS=-DNRT_FIRST_PIPE=0, sp0 = -DNRT_SECOND_PIPE=0 (e.g. --base sp0 --pairs 4)."""
 import argparse
 import json
 import os
@@ -66,7 +69,7 @@ def main():
     ap.add_argument("--pairs", type=int, default=3)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
-    ap.add_argument("--base", default="bm0", help="library tag of the reference build (NRT_BIAS_MMA=0)")
+    ap.add_argument("--base", default="bm0", help="library tag of the reference build (bm0: NRT_BIAS_MMA=0, fp0: NRT_FIRST_PIPE=0, sp0: NRT_SECOND_PIPE=0)")
     ap.add_argument("--new", default="", help="library tag of the build under test (default: the product build)")
     ap.add_argument("--extra", default="", help="comma-separated further tags whose frames are compared with the base")
     ap.add_argument("--out", default=None)

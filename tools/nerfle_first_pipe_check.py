@@ -1,7 +1,8 @@
-"""Outputs of NeRFLE.first's inference kernels under two library builds, compared bit for bit (NRT_FIRST_PIPE,
-csrc/tc_core.cuh: the change moves work across the tile boundary and must not change a single bit).
+"""Outputs of the NeRFLE inference kernels under two library builds, compared bit for bit (NRT_FIRST_PIPE and
+NRT_SECOND_PIPE, csrc/tc_core.cuh: each moves work across a kernel's tile boundary and must not change a single bit).
 
-    python tools/nerfle_first_pipe_check.py --base fp0 [--new ""] [--out FILE]
+    python tools/nerfle_first_pipe_check.py --base fp0 [--new ""] [--out FILE]     # NRT_FIRST_PIPE=0 build
+    python tools/nerfle_first_pipe_check.py --base sp0 [--new ""] [--out FILE]     # NRT_SECOND_PIPE=0 build
 
 Each build (build_native.py with NRT_BUILD_TAG, selected with NRT_LIB_TAG) renders, in a process of its own:
   * the 4K leg of bench.py: 3840 x 2160 rays, one uniform pass of 64 samples, f16;
