@@ -381,6 +381,61 @@ int nrt_nerfle_render_camera_host(const nrt_mlp_t* first, const nrt_mlp_t* secon
                                   const nrt_nerf_sampling_t* sampling, const float* light_code, int light_dim,
                                   float* out_rgb_host, void* stream);
 
+/* ---- occupancy grid: empty-space skipping for the gradient-free NeRFLE render (extension; the reference has none) --------
+ * Grid: a cube of res^3 cells over [bbox_min, bbox_max] (NRT_OCC_MIN_RES <= res <= NRT_OCC_MAX_RES; the box finite with
+ * bbox_max > bbox_min per axis).  Cell (i,j,k) has the linear index c = (i * res + j) * res + k (C order, z fastest, torch's
+ * [res,res,res]).  bits [ceil(res^3 / 32)] uint32: bit c & 31 of word c >> 5 is set iff density[c] > threshold.
+ * Update (nrt_occupancy_update): point q of cell c is at lo + (idx + u) * h per axis, h = (hi - lo) / res computed in double
+ * and rounded to float once, every operation rounded in fp32 (no contraction); u = the render's counter hash of
+ * (seed, c, 3 q + axis), or 0.5 (the cell centre) when seed = 0.  The points go through nrt_mlp_forward(first, prec) (fp32 at
+ * NRT_PREC_F32, the tensor cores otherwise), and density[c] = max(decay * density[c], max_q relu(sigma_raw(q))) with
+ * sigma_raw = column 0 of first's output (a NaN output counts as 0), then the bits are rewritten.  decay = 0 rebuilds the
+ * grid (density must then be finite, e.g. zeros); 0 <= decay <= 1, threshold finite and >= 0,
+ * 1 <= points_per_cell <= NRT_OCC_MAX_POINTS_PER_CELL.  workspace: nrt_occupancy_update_workspace bytes.
+ * Cull (nrt_occupancy_mask, the render below): the sample point p = o + t d (the expression of the render's first kernel), its
+ * cell floor((p - lo) * inv) per axis with inv = res / (hi - lo) computed in double and rounded to float once.  A sample is
+ * culled iff every axis lands in [0, res) and the cell's bit is clear: samples outside the box and non-finite points are kept.
+ * nrt_occupancy_mask writes keep [R,S] uint8 (1 = kept), ray-major, from the same device function the render uses. */
+#define NRT_OCC_MIN_RES 16
+#define NRT_OCC_MAX_RES 512
+#define NRT_OCC_MAX_POINTS_PER_CELL 4096
+typedef struct nrt_occupancy {
+  int32_t res;
+  float bbox_min[3], bbox_max[3];
+  const uint32_t* bits;     /* device; may be NULL for nrt_occupancy_update, which writes bits_out */
+} nrt_occupancy_t;
+size_t nrt_occupancy_update_workspace(const nrt_mlp_t* first, int prec, int32_t res, int points_per_cell);
+int nrt_occupancy_update(const nrt_mlp_t* first, int prec, const nrt_occupancy_t* grid, int points_per_cell, float decay,
+                         float threshold, uint64_t seed, float* density, uint32_t* bits_out, void* workspace,
+                         size_t workspace_bytes, void* stream);
+int nrt_occupancy_mask(const nrt_occupancy_t* grid, const float* rays, int64_t R, const float* ts, const float* ts_per_ray,
+                       int S, uint8_t* keep, void* stream);
+/* The render (nrt_nerfle_render / nrt_nerfle_render_camera) and its per-sample pass (nrt_nerfle_render_samples) with the
+ * grid's cull: exactly one of rays [R,6] / cam (R = the camera's ray count; a camera frame takes its rays from the ray
+ * generator kernel whatever nrt_set_camera_rays_mode says).  Every pass (the coarse and, with n_fine > 0, the fine one)
+ * writes sigma_raw = 0 and rgb = 0 at its culled samples and runs both tensor-core MLPs on the kept ones only, compacted
+ * (MMA rows are independent: a kept sample gets the bits of the unculled render).  With relu(sigma) = 0 a culled sample
+ * has alpha 0 and contributes exactly +0, so the image is the unculled render's with sigma_raw = rgb = 0 at culled samples;
+ * with every bit set it is the unculled render, bit for bit.  grid NULL: the call without a grid.  Tensor-core precisions
+ * only (NRT_PREC_F32 with a grid: NRT_E_UNSUPPORTED), with the 16-bit latent hand-off.  samples_done (optional, device
+ * uint64): the kept samples of every pass are added to it.  Asynchronous like the calls without a grid.
+ * workspace: the *_occupancy_workspace bytes (the plain workspace + a keep list of 4 B and a flag of 1 B per sample of the
+ * larger pass, the kept count and CUB's selection storage). */
+size_t nrt_nerfle_render_occupancy_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, int64_t R,
+                                             const nrt_camera_t* cam, const nrt_nerf_sampling_t* sampling);
+int nrt_nerfle_render_occupancy(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                const nrt_camera_t* cam, int64_t R, const float* ts, const nrt_nerf_sampling_t* sampling,
+                                const float* light_code, int light_dim, const int32_t* view_of_ray,
+                                const nrt_occupancy_t* grid, unsigned long long* samples_done, float* out_rgb,
+                                void* workspace, size_t workspace_bytes, void* stream);
+size_t nrt_nerfle_render_samples_occupancy_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, int64_t R,
+                                                     int S, const nrt_camera_t* cam);
+int nrt_nerfle_render_samples_occupancy(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                        const nrt_camera_t* cam, int64_t R, const float* ts, const float* ts_per_ray, int S,
+                                        const float* light_code, int light_dim, const int32_t* view_of_ray,
+                                        const nrt_occupancy_t* grid, unsigned long long* samples_done, float* out_sigma,
+                                        float* out_rgb, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- meshes: a SphereSDF on a lattice, and the isosurface of a lattice (extension; the reference has no mesh output) ----
  * Lattice: values[i][j][k] fp32 in C order (z fastest, torch's [nx, ny, nz]); point (i,j,k) is at origin + (i,j,k) * spacing,
  * per axis one rounded product and one rounded sum (no FMA contraction).  Dimensions are in [2, NRT_MAX_LATTICE_DIM]; origin

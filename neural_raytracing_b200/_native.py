@@ -53,6 +53,10 @@ class NrtLattice(ctypes.Structure):
     _fields_ = [("nx", c_i64), ("ny", c_i64), ("nz", c_i64), ("origin", c_f32 * 3), ("spacing", c_f32 * 3)]
 
 
+class NrtOccupancy(ctypes.Structure):
+    _fields_ = [("res", ctypes.c_int32), ("bbox_min", c_f32 * 3), ("bbox_max", c_f32 * 3), ("bits", c_vp)]
+
+
 class NrtLight(ctypes.Structure):
     _fields_ = [("mode", ctypes.c_int32), ("n_views", ctypes.c_int32), ("location", c_vp), ("amp", c_vp), ("coef", c_vp),
                 ("view_of_hit", c_vp), ("v", c_vp), ("sig_color", c_vp)]
@@ -71,6 +75,7 @@ _PM, _PS, _PN = ctypes.POINTER(NrtMlp), ctypes.POINTER(NrtSphereSdf), ctypes.POI
 _PL, _PB = ctypes.POINTER(NrtLight), ctypes.POINTER(NrtBlend)
 _PC = ctypes.POINTER(NrtCamera)
 _PG = ctypes.POINTER(NrtLattice)
+_PO = ctypes.POINTER(NrtOccupancy)
 
 # every symbol declared in include/nrt_b200.h: name -> (restype, argtypes)
 SIGNATURES = {
@@ -127,6 +132,15 @@ SIGNATURES = {
     "nrt_nerfle_render_samples": (c_int, [_PM, _PM, c_int, c_vp, _PC, c_i64, c_vp, c_vp, c_int, c_vp, c_int, c_vp, c_vp, c_vp,
                                           c_vp, c_sz, c_vp]),
     "nrt_nerfle_render_camera_host":(c_int, [_PM, _PM, c_int, _PC, c_vp, c_int, _PN, c_vp, c_int, c_vp, c_vp]),
+    "nrt_occupancy_update_workspace": (c_sz, [_PM, c_int, ctypes.c_int32, c_int]),
+    "nrt_occupancy_update": (c_int, [_PM, c_int, _PO, c_int, c_f32, c_f32, ctypes.c_uint64, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "nrt_occupancy_mask": (c_int, [_PO, c_vp, c_i64, c_vp, c_vp, c_int, c_vp, c_vp]),
+    "nrt_nerfle_render_occupancy_workspace": (c_sz, [_PM, _PM, c_int, c_i64, _PC, _PN]),
+    "nrt_nerfle_render_occupancy": (c_int, [_PM, _PM, c_int, c_vp, _PC, c_i64, c_vp, _PN, c_vp, c_int, c_vp, _PO, c_vp, c_vp,
+                                            c_vp, c_sz, c_vp]),
+    "nrt_nerfle_render_samples_occupancy_workspace": (c_sz, [_PM, _PM, c_int, c_i64, c_int, _PC]),
+    "nrt_nerfle_render_samples_occupancy": (c_int, [_PM, _PM, c_int, c_vp, _PC, c_i64, c_vp, c_vp, c_int, c_vp, c_int, c_vp,
+                                                    _PO, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "nrt_sdf_lattice_eval_workspace": (c_i64, [_PG]),
     "nrt_sdf_lattice_eval": (c_int, [_PS, c_int, _PG, c_vp, c_vp, c_sz, c_vp]),
     "nrt_isosurface_workspace": (c_i64, [_PG]),

@@ -169,7 +169,7 @@ int nrt_build_sdf_dev(const nrt_sphere_sdf_t* s, SdfDev* out) {
 static const char* kTagNames[TAG_COUNT] = {
     "mlp_fwd_f32", "sdf_eval_f32", "sdf_march_f32", "sdf_shadow_f32", "sdf_min_scan_f32", "nerfle_fused_f32",
     "composite_fwd", "composite_bwd", "mlp_tc_nerf_first", "mlp_tc_nerf_second", "mlp_tc_generic", "mlp_tc_pack",
-    "stratified_ts", "sample_pdf", "merge_composite", "mlp_bwd_f32", "sdf_value_grad_f32", "shade",
+    "stratified_ts", "sample_pdf", "merge_composite", "occupancy_cull", "occupancy_update", "mlp_bwd_f32", "sdf_value_grad_f32", "shade",
     "sdf_eval_tc", "sdf_march_tc", "sdf_shadow_tc", "sdf_min_scan_tc", "mlp_tc_train_fwd", "mlp_tc_dgrad",
     "mlp_tc_wgrad", "mlp_tc_wide", "camera_rays", "merge_ts", "composite_ts_fwd", "composite_ts_bwd",
     "lattice_points", "iso_count", "iso_scan", "iso_emit"};

@@ -72,11 +72,12 @@ int nrt_next_counter(cudaStream_t st, unsigned long long** out);
 int nrt_host_scratch(NrtDeviceState* s, int slot, size_t bytes, void** out);
 #endif
 
-// launch accounting / optional per-kernel event timing (nrt_profile_* in the C ABI)
+// launch accounting / optional per-kernel event timing (nrt_profile_* in the C ABI).  Tags are looked up by name; the mesh
+// tags stay last, after composite_ts_bwd, so the occupancy tags sit with the other render kernels.
 enum NrtTag {
   TAG_MLP_F32 = 0, TAG_SDF_EVAL_F32, TAG_MARCH_F32, TAG_SHADOW_F32, TAG_MIN_SCAN_F32, TAG_NERFLE_F32,
   TAG_COMPOSITE_FWD, TAG_COMPOSITE_BWD, TAG_TC_NERF_FIRST, TAG_TC_NERF_SECOND, TAG_TC_MLP, TAG_TC_PACK,
-  TAG_STRATIFIED_TS, TAG_SAMPLE_PDF, TAG_MERGE_COMPOSITE, TAG_MLP_BWD_F32, TAG_SDF_GRAD_F32, TAG_SHADE,
+  TAG_STRATIFIED_TS, TAG_SAMPLE_PDF, TAG_MERGE_COMPOSITE, TAG_OCCUPANCY_CULL, TAG_OCCUPANCY_UPDATE, TAG_MLP_BWD_F32, TAG_SDF_GRAD_F32, TAG_SHADE,
   TAG_TC_SDF_EVAL, TAG_TC_MARCH, TAG_TC_SHADOW, TAG_TC_MIN_SCAN, TAG_TC_TRAIN_FWD, TAG_TC_DGRAD, TAG_TC_WGRAD, TAG_TC_MLP_WIDE,
   TAG_CAMERA_RAYS, TAG_MERGE_TS, TAG_COMPOSITE_TS_FWD, TAG_COMPOSITE_TS_BWD,
   TAG_LATTICE_POINTS, TAG_ISO_COUNT, TAG_ISO_SCAN, TAG_ISO_EMIT, TAG_COUNT
@@ -88,5 +89,18 @@ struct NrtProfScope {
   NrtProfScope(int t, cudaStream_t s) : tag(t), st(s) { nrt_prof_begin(tag, st); }
   ~NrtProfScope() { nrt_prof_end(tag, st); }
 };
+
+// counter hash -> uniform [0,1) with 24 bits: the jitter of the stratified and fine distances (nrt_render.cu) and of the
+// occupancy grid's update points (nrt_occupancy.cu).  32-bit arithmetic: the 64-bit splitmix of round 1 cost ~25 integer
+// instructions per sample in kernels that should be HBM-bound; oracle/port.py restates the same recipe.
+#ifdef __CUDACC__
+__device__ __forceinline__ float hash_u01(uint64_t seed, uint64_t a, uint64_t b) {
+  uint32_t h = (uint32_t)seed ^ ((uint32_t)(seed >> 32) * 0x9E3779B1u);
+  h = (h ^ (uint32_t)a) * 0x85EBCA77u;
+  h = (h ^ (uint32_t)b) * 0xC2B2AE3Du;
+  h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
+  return (float)(h >> 8) * (1.0f / 16777216.0f);
+}
+#endif
 
 static inline int nrt_cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }

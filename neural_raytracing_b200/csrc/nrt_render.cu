@@ -17,6 +17,12 @@ int nrt_nerfle_pass_tc(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
                        cudaStream_t st, const nrt_camera_t* cam = nullptr, int64_t cam_r0 = 0);
 bool nrt_nerfle_pass_tc_camera_ok(const nrt_mlp_t* first, const nrt_mlp_t* second, int light_dim);
 size_t nrt_nerfle_pass_tc_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int64_t R, int S);
+size_t nrt_occupancy_pass_workspace(int64_t C, int S);
+int nrt_occupancy_pass(const nrt_occupancy_t* grid, unsigned long long* samples_done, const nrt_mlp_t* first,
+                       const nrt_mlp_t* second, int prec, const float* rays, int64_t n, const float* ts,
+                       const float* ts_per_ray, int S, const float* light_code, int light_dim, const int32_t* view_of_ray,
+                       float* out_sigma, float* out_srgb, void* tcws, size_t tcws_bytes, void* occws, size_t occws_bytes,
+                       cudaStream_t st);
 
 static int nerf_pass(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays, int64_t R,
                      const float* ts, const float* ts_per_ray, int S, const float* light_code, int light_dim,
@@ -56,15 +62,7 @@ extern "C" int nrt_set_camera_rays_mode(int fused) {
 // ---- stratified sample distances -------------------------------------------------------------
 // ts[r][s] = near + (s + u)/S * (far-near), u = hash(seed, r, s) in [0,1)  (extension; the
 // reference uses the same ts for every ray, nerf.py:178).
-// (32-bit arithmetic: the 64-bit splitmix of round 1 cost ~25 integer instructions per sample in kernels that should
-//  be HBM-bound; oracle/port.py restates the same recipe)
-__device__ __forceinline__ float hash_u01(uint64_t seed, uint64_t a, uint64_t b) {
-  uint32_t h = (uint32_t)seed ^ ((uint32_t)(seed >> 32) * 0x9E3779B1u);
-  h = (h ^ (uint32_t)a) * 0x85EBCA77u;
-  h = (h ^ (uint32_t)b) * 0xC2B2AE3Du;
-  h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15; h *= 0x846CA68Bu; h ^= h >> 16;
-  return (float)(h >> 8) * (1.0f / 16777216.0f);
-}
+// (hash_u01: nrt_common.cuh)
 
 // four consecutive samples of one ray per thread (S % 4 == 0: one 16-byte store per thread, coalesced), else one.
 // seed_dev (training under CUDA graphs, nrt_nerfle_sample_hierarchical): when not NULL the seed is read from device memory
@@ -389,8 +387,17 @@ int nrt_check_camera(const nrt_camera_t* cam, int64_t* total);
 int nrt_camera_rays_dev(const nrt_camera_t* cam, int64_t r0, int64_t n, float* out_rays, int32_t* out_view,
                         cudaStream_t st);
 
+// workspace of the occupancy-culled render on top of nrt_nerfle_render_workspace (nrt_occupancy.cu)
+static size_t occ_scratch_bytes(int64_t R, const nrt_nerf_sampling_t* sampling) {
+  const int64_t C = std::min<int64_t>(R, kRayChunk);
+  const int S = sampling ? std::max(sampling->n_coarse, sampling->n_fine) : 64;
+  return align256(nrt_occupancy_pass_workspace(C, S));
+}
+
 // the render of R rays given either as an array (rays) or as a camera (cam: every chunk's rays are generated into the
 // tail of the workspace right before its first pass; SURVEY f4).
+// Occupancy grid (occ not NULL, nrt_occupancy.cu): every pass is k_occupancy_cull -> NeRFLE.first -> NeRFLE.second on the
+// kept samples (nrt_occupancy_pass) in place of nerf_pass; camera rays come from k_camera_rays (mode 0).
 // Per-sample mode (nrt_nerfle_render_samples): smp_sigma [R,Sc] / smp_rgb [R,Sc,3] not NULL, n_fine = 0 -- every chunk's
 // pass stores its per-sample values there instead of the workspace and nothing is composited; ts_per_ray [R,Sc], when not
 // NULL, gives every ray its own distances in place of ts / the stratified ones.
@@ -398,8 +405,13 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
                        const nrt_camera_t* cam, int64_t R, const float* ts, const nrt_nerf_sampling_t* sampling,
                        const float* light_code, int light_dim, const int32_t* view_of_ray,
                        float* out_rgb, void* workspace, size_t workspace_bytes, cudaStream_t st,
-                       const float* ts_per_ray = nullptr, float* smp_sigma = nullptr, float* smp_rgb = nullptr) {
+                       const float* ts_per_ray = nullptr, float* smp_sigma = nullptr, float* smp_rgb = nullptr,
+                       const nrt_occupancy_t* occ = nullptr, unsigned long long* samples_done = nullptr) {
   NRT_REQUIRE(R >= 0, "nrt_nerfle_render: negative R");
+  if (occ != nullptr && prec == NRT_PREC_F32) {
+    nrt_set_error("nrt_nerfle_render_occupancy: the occupancy grid culls on the tensor-core precisions (f16, bf16) only");
+    return NRT_E_UNSUPPORTED;
+  }
   if (R == 0) return NRT_OK;
   const bool samples = smp_sigma != nullptr;
   NRT_REQUIRE((rays != nullptr || cam != nullptr) && (out_rgb != nullptr || (samples && smp_rgb != nullptr)),
@@ -413,11 +425,12 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
   NRT_REQUIRE(!samples || Sf == 0, "nrt_nerfle_render: per-sample outputs of a single pass only");
   NRT_REQUIRE(Sf == 0 || Sc >= 3, "hierarchical sampling needs n_coarse >= 3");
   const int64_t C = std::min<int64_t>(R, kRayChunk);
-  const size_t need = nrt_nerfle_render_workspace(first, second, prec, R, sampling) + (cam ? cam_scratch_bytes(C) : 0);
+  const size_t need = nrt_nerfle_render_workspace(first, second, prec, R, sampling) + (cam ? cam_scratch_bytes(C) : 0) +
+                      (occ ? occ_scratch_bytes(R, sampling) : 0);
   NRT_REQUIRE(workspace != nullptr && workspace_bytes >= need,
               "nrt_nerfle_render: workspace of %zu bytes required, got %zu", need, workspace_bytes);
   float* cam_rays = nullptr; int32_t* cam_view = nullptr;
-  const bool fused = cam && prec != NRT_PREC_F32 && camera_fused_default() &&
+  const bool fused = cam && !occ && prec != NRT_PREC_F32 && camera_fused_default() &&
                      nrt_nerfle_pass_tc_camera_ok(first, second, light_dim);
   if (cam) {
     char* tail = (char*)workspace + (need - cam_scratch_bytes(C));
@@ -439,6 +452,20 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
     tcws_bytes = nrt_nerfle_pass_tc_workspace(first, second, C, std::max(Sc, Sf));
     tcws = take(tcws_bytes);
   }
+  void* occws = nullptr; size_t occws_bytes = 0;
+  if (occ) {
+    occws_bytes = occ_scratch_bytes(R, sampling);
+    occws = take(occws_bytes);
+  }
+  // one pass over a chunk that stores its per-sample sigma / rgb: the plain pass, or the culled one
+  auto pass = [&](const float* c_rays, int64_t n, const float* ts_s, const float* ts_r, int S, const int32_t* c_view,
+                  float* o_sig, float* o_srgb, const nrt_camera_t* kcam, int64_t r0) {
+    if (occ)
+      return nrt_occupancy_pass(occ, samples_done, first, second, prec, c_rays, n, ts_s, ts_r, S, light_code, light_dim,
+                                c_view, o_sig, o_srgb, tcws, tcws_bytes, occws, occws_bytes, st);
+    return nerf_pass(first, second, prec, c_rays, n, ts_s, ts_r, S, light_code, light_dim, c_view, nullptr, o_sig, o_srgb,
+                     tcws, tcws_bytes, st, kcam, r0);
+  };
   const int warps = 4;
   const size_t merge_smem = (size_t)warps * 5 * (Sc + Sf) * sizeof(float);
   NRT_REQUIRE(merge_smem <= 48 * 1024, "too many samples per ray for the merge kernel");
@@ -466,8 +493,7 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
     }
     int rc;
     if (samples) {
-      rc = nerf_pass(first, second, prec, c_rays, n, ts_shared, ts_pr, Sc, light_code, light_dim, c_view, nullptr,
-                     smp_sigma + r0 * Sc, smp_rgb + r0 * Sc * 3, tcws, tcws_bytes, st, kcam, r0);
+      rc = pass(c_rays, n, ts_shared, ts_pr, Sc, c_view, smp_sigma + r0 * Sc, smp_rgb + r0 * Sc * 3, kcam, r0);
       if (rc != NRT_OK) return rc;
       continue;
     }
@@ -478,14 +504,12 @@ static int render_impl(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
       continue;
     }
     // coarse pass keeps per-sample sigma / rgb
-    rc = nerf_pass(first, second, prec, c_rays, n, ts_shared, ts_pr, Sc, light_code, light_dim, c_view, nullptr,
-                   sig_c, rgb_c, tcws, tcws_bytes, st, kcam, r0);
+    rc = pass(c_rays, n, ts_shared, ts_pr, Sc, c_view, sig_c, rgb_c, kcam, r0);
     if (rc != NRT_OK) return rc;
     if (Sf > 0) {
       rc = launch_sample_pdf(prec, sig_c, ts_shared, ts_pr, Sc, Sf, n, r0, sampling->jitter_seed, nullptr, ts_f, st);
       if (rc != NRT_OK) return rc;
-      rc = nerf_pass(first, second, prec, c_rays, n, nullptr, ts_f, Sf, light_code, light_dim, c_view, nullptr,
-                     sig_f, rgb_f, tcws, tcws_bytes, st, kcam, r0);
+      rc = pass(c_rays, n, nullptr, ts_f, Sf, c_view, sig_f, rgb_f, kcam, r0);
       if (rc != NRT_OK) return rc;
     }
     { NrtProfScope _ps(TAG_MERGE_COMPOSITE, st);
@@ -629,6 +653,68 @@ extern "C" int nrt_nerfle_render_samples(const nrt_mlp_t* first, const nrt_mlp_t
   const nrt_nerf_sampling_t samp{S, 0, 0.0f, 0.0f, 0};
   return render_impl(first, second, prec, rays, cam, R, ts, &samp, light_code, light_dim, view_of_ray, nullptr, workspace,
                      workspace_bytes, (cudaStream_t)stream, ts_per_ray, out_sigma, out_rgb);
+}
+
+// ---- the same three renders with an occupancy grid (nrt_occupancy.cu; NULL grid: the calls above) ------------------------
+extern "C" size_t nrt_nerfle_render_occupancy_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, int64_t R,
+                                                        const nrt_camera_t* cam, const nrt_nerf_sampling_t* sampling) {
+  if (cam) {
+    if (nrt_check_camera(cam, &R) != NRT_OK) return 0;
+  }
+  if (R < 0 || sampling == nullptr) return 0;
+  return nrt_nerfle_render_workspace(first, second, prec, R, sampling) +
+         (cam ? cam_scratch_bytes(std::min<int64_t>(R, kRayChunk)) : 0) + occ_scratch_bytes(R, sampling);
+}
+
+extern "C" int nrt_nerfle_render_occupancy(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays,
+                                           const nrt_camera_t* cam, int64_t R, const float* ts,
+                                           const nrt_nerf_sampling_t* sampling, const float* light_code, int light_dim,
+                                           const int32_t* view_of_ray, const nrt_occupancy_t* grid,
+                                           unsigned long long* samples_done, float* out_rgb, void* workspace,
+                                           size_t workspace_bytes, void* stream) {
+  NRT_REQUIRE(R >= 0, "nrt_nerfle_render_occupancy: negative R");
+  NRT_REQUIRE((rays != nullptr) != (cam != nullptr), "nrt_nerfle_render_occupancy: exactly one of rays / cam must be given");
+  if (cam) {
+    int64_t Rc = 0;
+    const int rc = nrt_check_camera(cam, &Rc);
+    if (rc != NRT_OK) return rc;
+    NRT_REQUIRE(R == Rc, "nrt_nerfle_render_occupancy: R = %lld but the camera has %lld rays", (long long)R, (long long)Rc);
+    NRT_REQUIRE(view_of_ray == nullptr, "nrt_nerfle_render_occupancy: a camera gives every ray its view; view_of_ray must be NULL");
+  }
+  return render_impl(first, second, prec, rays, cam, R, ts, sampling, light_code, light_dim, view_of_ray, out_rgb, workspace,
+                     workspace_bytes, (cudaStream_t)stream, nullptr, nullptr, nullptr, grid, samples_done);
+}
+
+extern "C" size_t nrt_nerfle_render_samples_occupancy_workspace(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
+                                                                int64_t R, int S, const nrt_camera_t* cam) {
+  if (R < 0 || S < 1) return 0;
+  const nrt_nerf_sampling_t samp{S, 0, 0.0f, 0.0f, 0};
+  return nrt_nerfle_render_samples_workspace(first, second, prec, R, S, cam) + occ_scratch_bytes(R, &samp);
+}
+
+extern "C" int nrt_nerfle_render_samples_occupancy(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec,
+                                                   const float* rays, const nrt_camera_t* cam, int64_t R, const float* ts,
+                                                   const float* ts_per_ray, int S, const float* light_code, int light_dim,
+                                                   const int32_t* view_of_ray, const nrt_occupancy_t* grid,
+                                                   unsigned long long* samples_done, float* out_sigma, float* out_rgb,
+                                                   void* workspace, size_t workspace_bytes, void* stream) {
+  NRT_REQUIRE(R >= 0, "nrt_nerfle_render_samples_occupancy: negative R");
+  NRT_REQUIRE((rays != nullptr) != (cam != nullptr), "nrt_nerfle_render_samples_occupancy: exactly one of rays / cam must be given");
+  if (cam) {
+    int64_t Rc = 0;
+    const int rc = nrt_check_camera(cam, &Rc);
+    if (rc != NRT_OK) return rc;
+    NRT_REQUIRE(R == Rc, "nrt_nerfle_render_samples_occupancy: R = %lld but the camera has %lld rays", (long long)R, (long long)Rc);
+    NRT_REQUIRE(view_of_ray == nullptr, "nrt_nerfle_render_samples_occupancy: a camera gives every ray its view; view_of_ray must be NULL");
+  }
+  NRT_REQUIRE(S >= 1, "nrt_nerfle_render_samples_occupancy: bad sample count %d", S);
+  NRT_REQUIRE((ts != nullptr) != (ts_per_ray != nullptr),
+              "nrt_nerfle_render_samples_occupancy: exactly one of ts / ts_per_ray must be given");
+  if (R == 0) return NRT_OK;
+  NRT_REQUIRE(out_sigma != nullptr && out_rgb != nullptr, "nrt_nerfle_render_samples_occupancy: null out_sigma/out_rgb");
+  const nrt_nerf_sampling_t samp{S, 0, 0.0f, 0.0f, 0};
+  return render_impl(first, second, prec, rays, cam, R, ts, &samp, light_code, light_dim, view_of_ray, nullptr, workspace,
+                     workspace_bytes, (cudaStream_t)stream, ts_per_ray, out_sigma, out_rgb, grid, samples_done);
 }
 
 // The host-buffer entry point keeps grow-only device scratch PER DEVICE (a stream-ordered pool would hand the memory

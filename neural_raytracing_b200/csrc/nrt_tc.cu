@@ -97,6 +97,9 @@ struct IoNerfFirst {
   }
   __device__ __forceinline__ void store(int64_t m, const float* o) const {
     sigma[m] = o[0];
+    store_latent(m, o);
+  }
+  __device__ __forceinline__ void store_latent(int64_t m, const float* o) const {
     if (lat32) {
       float4* dst = reinterpret_cast<float4*>(latent) + (m >> 7) * (int64_t)(NLAT / 4 * 128) + (m & 127);
 #pragma unroll
@@ -203,6 +206,50 @@ struct IoNerfSecond {
       rgb[m * 3 + j] = v;
     }
   }
+};
+
+// The occupancy-culled passes (render_impl with a grid): the kernels evaluate only the samples k_occupancy_cull kept.
+// Row m of the launch is sample keep[m] (= ray * S + s within the chunk, ascending), and *rows of them exist (a device
+// count, kDeviceRows): sigma and rgb go to the kept sample's own slot, the latent hand-off stays in compacted tile order,
+// so the bulk copy of NRT_SECOND_PIPE reads whole tiles as before.  The keep load is one more dependent load in front of
+// the ray's, issued a tile ahead with it (fetch / load_dir_code).  MMA rows are independent: a kept sample's outputs are
+// the bits the full layout gives it.
+template <int NLAT>
+struct IoNerfFirstKeep : IoNerfFirst<NLAT> {
+  const int32_t* keep; const int32_t* rows;
+  static constexpr bool kDeviceRows = true;
+  using Fetch = typename IoNerfFirst<NLAT>::Fetch;
+  __device__ __forceinline__ void fetch(int64_t m, Fetch& f) const { IoNerfFirst<NLAT>::fetch(__ldg(keep + m), f); }
+  __device__ __forceinline__ void load(int64_t m, float* v) const {
+    Fetch f;
+    fetch(m, f);
+    IoNerfFirst<NLAT>::point(f, v);
+  }
+  __device__ __forceinline__ void store(int64_t m, const float* o) const {
+    this->sigma[__ldg(keep + m)] = o[0];
+    this->store_latent(m, o);
+  }
+};
+template <int NLAT, int LD>
+struct IoNerfSecondKeep : IoNerfSecond<NLAT, LD, true> {
+  const int32_t* keep; const int32_t* rows;
+  static constexpr bool kDeviceRows = true;
+  __device__ __forceinline__ int64_t ray_of_row(int64_t m) const { return ray_of(__ldg(keep + m), this->S, this->s_shift); }
+  __device__ __forceinline__ void load_packed(int64_t m, uint32_t* w, float* v) const {
+    const uint4* src = reinterpret_cast<const uint4*>(this->latent) + (m >> 7) * (int64_t)(NLAT / 8 * 128) + (m & 127);
+#pragma unroll
+    for (int j = 0; j < NLAT / 8; ++j) {
+      const uint4 q = __ldg(src + j * 128);
+      w[4 * j] = q.x; w[4 * j + 1] = q.y; w[4 * j + 2] = q.z; w[4 * j + 3] = q.w;
+    }
+    load_dir_code(m, v + NLAT);
+  }
+  __device__ __forceinline__ void load_dir_code(int64_t m, float* v) const {
+    const int view = this->dir_and_view(ray_of_row(m), v);
+#pragma unroll
+    for (int j = 0; j < LD; ++j) v[3 + j] = __ldg(this->light_code + (int64_t)view * LD + j);
+  }
+  __device__ __forceinline__ void store(int64_t m, const float* o) const { IoNerfSecond<NLAT, LD, true>::store(__ldg(keep + m), o); }
 };
 
 static long long* g_dbg_timeline = nullptr;   // development only, see tools/tc_timeline.py
@@ -733,6 +780,49 @@ int nrt_nerfle_pass_tc(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec
                     : launch<NetNerfSecondLE, decltype(io2), 1>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND);
   }
   IoNerfSecond<64, 48> io2{rays, lat, light_code, view_of_ray, S, out_srgb, fmt, second_out_act, lat32, s_shift};
+  return fmt == 0 ? launch<NetNerfSecondLE, decltype(io2), 0>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND)
+                  : launch<NetNerfSecondLE, decltype(io2), 1>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND);
+}
+
+// the pass of an occupancy-culled render (nrt_render.cu, render_impl with a grid): the same two kernels on the rows that
+// k_occupancy_cull kept.  R * S is the capacity the persistent grids are sized from; *rows (device) is how many exist.
+int nrt_nerfle_pass_tc_keep(const nrt_mlp_t* first, const nrt_mlp_t* second, int prec, const float* rays, int64_t R,
+                            const float* ts, const float* ts_per_ray, int S, const float* light_code, int light_dim,
+                            const int32_t* view_of_ray, const int32_t* keep, const int32_t* rows, float* out_sigma,
+                            float* out_srgb, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  MlpDev d1, d2;
+  int rc = nrt_build_mlp_dev(first, &d1);
+  if (rc != NRT_OK) return rc;
+  rc = nrt_build_mlp_dev(second, &d2);
+  if (rc != NRT_OK) return rc;
+  NRT_REQUIRE(first->params_tc && second->params_tc, "params_tc is NULL: call nrt_mlp_pack_tc first");
+  NRT_REQUIRE(matches<NetNerfFirst>(d1), "tensor-core NeRF path: first MLP must be NeRFLE.first (3->65, 5x128)");
+  const bool pt = matches<NetNerfSecondPT>(d2) && light_dim == 3;
+  const bool le = matches<NetNerfSecondLE>(d2) && light_dim == 48;
+  NRT_REQUIRE(pt || le, "tensor-core NeRF path: second MLP must be NeRFLE.second (70->3 with a point light, or 115->3 with "
+                        "the 48-float environment code; 8x64)");
+  NRT_REQUIRE(rays != nullptr && keep != nullptr && rows != nullptr && out_sigma != nullptr && out_srgb != nullptr,
+              "occupancy-culled NeRF pass: null rays/keep/rows/outputs");
+  NRT_REQUIRE((ts != nullptr) != (ts_per_ray != nullptr), "exactly one of ts / ts_per_ray must be given");
+  if (nerf_latent32()) {
+    nrt_set_error("occupancy-culled NeRF pass: the 16-bit latent hand-off only (NRT_NERF_LATENT=f32 is not combined with a grid)");
+    return NRT_E_UNSUPPORTED;
+  }
+  const int64_t M = R * S;
+  NRT_REQUIRE(workspace != nullptr && workspace_bytes >= (size_t)((M + 127) / 128 * 128) * 64 * 2, "workspace too small");
+  void* lat = workspace;
+  const int fmt = fmt_of(prec);
+  const int s_shift = pow2_shift(S);
+  IoNerfFirstKeep<64> io1{{rays, ts, ts_per_ray, S, out_sigma, lat, fmt, 0, s_shift}, keep, rows};
+  rc = fmt == 0 ? launch<NetNerfFirstR, decltype(io1), 0>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST)
+                : launch<NetNerfFirstR, decltype(io1), 1>(first->params_tc, io1, M, st, TAG_TC_NERF_FIRST);
+  if (rc != NRT_OK) return rc;
+  if (pt) {
+    IoNerfSecondKeep<64, 3> io2{{rays, lat, light_code, view_of_ray, S, out_srgb, fmt, NRT_OUT_SIGMOID, 0, s_shift}, keep, rows};
+    return fmt == 0 ? launch<NetNerfSecondPT, decltype(io2), 0>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND)
+                    : launch<NetNerfSecondPT, decltype(io2), 1>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND);
+  }
+  IoNerfSecondKeep<64, 48> io2{{rays, lat, light_code, view_of_ray, S, out_srgb, fmt, NRT_OUT_SIGMOID, 0, s_shift}, keep, rows};
   return fmt == 0 ? launch<NetNerfSecondLE, decltype(io2), 0>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND)
                   : launch<NetNerfSecondLE, decltype(io2), 1>(second->params_tc, io2, M, st, TAG_TC_NERF_SECOND);
 }

@@ -1174,6 +1174,11 @@ template <class T, class D, class = void> struct FetchOf { using type = D; };
 template <class T, class D> struct FetchOf<T, D, std::void_t<typename T::Fetch>> { using type = typename T::Fetch; };
 template <class T, class = void> struct HasCtaInit : std::false_type {};
 template <class T> struct HasCtaInit<T, std::void_t<decltype(&T::cta_init)>> : std::true_type {};
+// tile policies with `static constexpr bool kDeviceRows = true` carry `const int32_t* rows`: the kernel evaluates
+// min(M, *rows) samples, a count written on the device by an earlier kernel of the stream (occupancy-culled NeRFLE
+// passes: M is the capacity the persistent grid was sized from, *rows the samples kept by k_occupancy_cull)
+template <class T, class = void> struct DeviceRowsOf { static constexpr bool value = false; };
+template <class T> struct DeviceRowsOf<T, std::void_t<decltype(T::kDeviceRows)>> { static constexpr bool value = T::kDeviceRows; };
 template <class T, class = void> struct IsIterative : std::false_type {};
 template <class T> struct IsIterative<T, std::void_t<typename T::State>> : std::true_type {};
 struct NoState {};
@@ -1287,6 +1292,10 @@ k_mlp_tc(const uint8_t* __restrict__ blob, IO io, int64_t M, long long* __restri
   const int mma_id = SELF ? -1 : warp - NET::NWG * WPS;   // >= 0: MMA-issuing warp
   const bool is_mma_warp = SELF ? warp == 0 : mma_id == 0;   // the one that also owns TMEM allocation and the weight load
   __shared__ uint32_t s_issue_lock;                  // self-issue: one slot's MMA batch at a time
+  if constexpr (DeviceRowsOf<IO>::value) {   // read once, before anything depends on M
+    const int64_t rows = *io.rows;
+    if (rows < M) M = rows;
+  }
   const int64_t ntiles = (M + 127) / 128;
   // IO policies that keep per-CTA tables in shared memory (the sphere set of the SDF policies) fill them here; the
   // __syncthreads() below publishes them

@@ -659,9 +659,13 @@ _ws_cache = {}
 
 def nerfle_render(first: PackedMLP, second: PackedMLP, rays: torch.Tensor, ts: Optional[torch.Tensor],
                   light_code: torch.Tensor, view_of_ray: Optional[torch.Tensor] = None, prec=PREC_F32,
-                  n_coarse: Optional[int] = None, n_fine=0, t_near=0.0, t_far=0.0, jitter_seed=0) -> torch.Tensor:
+                  n_coarse: Optional[int] = None, n_fine=0, t_near=0.0, t_far=0.0, jitter_seed=0, occupancy=None,
+                  samples_done: Optional[torch.Tensor] = None) -> torch.Tensor:
     """NeRFLE.forward (nerf.py:175-214): rays [...,6] -> rgb [...,3].
-    With n_fine == 0 and jitter_seed == 0 this is the reference's single uniform pass over `ts`."""
+    With n_fine == 0 and jitter_seed == 0 this is the reference's single uniform pass over `ts`.
+    `occupancy` (an OccupancyGrid, or any object with res / bbox_min / bbox_max / bits): cull the samples in empty cells
+    before both MLPs (nrt_nerfle_render_occupancy; f16 / bf16 only); `samples_done` (one int64 on the device) then
+    accumulates the kept samples.  None: the call without a grid."""
     prec = prec_id(prec)
     batch = rays.shape[:-1]
     r2 = _chk(rays, "rays").reshape(-1, 6)
@@ -676,6 +680,9 @@ def nerfle_render(first: PackedMLP, second: PackedMLP, rays: torch.Tensor, ts: O
     vor = _chk(view_of_ray.reshape(-1), "view_of_ray", torch.int32) if view_of_ray is not None else None
     out = torch.empty((R, 3), dtype=torch.float32, device=rays.device)
     samp = N.NrtNerfSampling(int(n_coarse), int(n_fine), float(t_near), float(t_far), int(jitter_seed))
+    if occupancy is not None or samples_done is not None:
+        return _render_occupancy(first, second, prec, r2, None, R, t, samp, lc, vor, occupancy, samples_done,
+                                 out).reshape(batch + (3,))
     with torch.cuda.device(rays.device):
         c1, c2 = first.c_struct(prec), second.c_struct(prec)
         nbytes = N.lib().nrt_nerfle_render_workspace(ctypes.byref(c1), ctypes.byref(c2), prec, R, ctypes.byref(samp))
@@ -812,9 +819,11 @@ def set_camera_rays_mode(fused: bool):
 
 def nerfle_render_camera(first: PackedMLP, second: PackedMLP, cam: CameraDesc, ts: Optional[torch.Tensor],
                          light_code: torch.Tensor, prec=PREC_F32, n_coarse: Optional[int] = None, n_fine=0,
-                         t_near=0.0, t_far=0.0, jitter_seed=0) -> torch.Tensor:
+                         t_near=0.0, t_far=0.0, jitter_seed=0, occupancy=None,
+                         samples_done: Optional[torch.Tensor] = None) -> torch.Tensor:
     """The frame of a volumetric shape from its camera in one call: rays are generated on the device inside the
-    library (f4; replaces the tile loop of pathtrace, main.py:57-88).  -> rgb [n_views, nx, ny, bundle, 3]."""
+    library (f4; replaces the tile loop of pathtrace, main.py:57-88).  -> rgb [n_views, nx, ny, bundle, 3].
+    `occupancy` / `samples_done`: as in nerfle_render (the rays then always come from the ray generator kernel)."""
     prec = prec_id(prec)
     t = _chk(ts, "ts").reshape(-1) if ts is not None else None
     if n_coarse is None:
@@ -827,6 +836,10 @@ def nerfle_render_camera(first: PackedMLP, second: PackedMLP, cam: CameraDesc, t
         raise NrtError("light_code has %d rows for %d views" % (lc.shape[0], cam.n_views))
     out = torch.empty((cam.n_views, cam.nx, cam.ny, cam.bundle, 3), dtype=torch.float32, device=cam.device)
     samp = N.NrtNerfSampling(int(n_coarse), int(n_fine), float(t_near), float(t_far), int(jitter_seed))
+    if occupancy is not None or samples_done is not None:
+        _render_occupancy(first, second, prec, None, cam, cam.n_rays, t, samp, lc, None, occupancy, samples_done,
+                          out.view(-1, 3))
+        return out
     with torch.cuda.device(cam.device):
         c1, c2 = first.c_struct(prec), second.c_struct(prec)
         nbytes = N.lib().nrt_nerfle_render_camera_workspace(ctypes.byref(c1), ctypes.byref(c2), prec,
@@ -843,11 +856,13 @@ def nerfle_render_camera(first: PackedMLP, second: PackedMLP, cam: CameraDesc, t
 
 
 def nerfle_render_samples(first: PackedMLP, second: PackedMLP, rays_or_cam, ts: torch.Tensor, light_code: torch.Tensor,
-                          view_of_ray: Optional[torch.Tensor] = None, prec=PREC_F32):
+                          view_of_ray: Optional[torch.Tensor] = None, prec=PREC_F32, occupancy=None,
+                          samples_done: Optional[torch.Tensor] = None):
     """The per-sample values the render composites (nrt_nerfle_render_samples: the render's own chunks and kernels):
     rays [...,6] or a CameraDesc, ts [S] (shared) or [R,S] (per ray) -> sigma [R,S] (pre-relu), rgb [R,S,3] (sigmoid),
     ray-major.  A camera picks the light-code row of every ray from its view and takes the camera-fed kernels when
-    set_camera_rays_mode(True) selected them, as nerfle_render_camera does."""
+    set_camera_rays_mode(True) selected them, as nerfle_render_camera does.  `occupancy` / `samples_done`: as in
+    nerfle_render; culled samples come out as sigma = 0, rgb = 0."""
     prec = prec_id(prec)
     cam = rays_or_cam if isinstance(rays_or_cam, CameraDesc) else None
     if cam is not None:
@@ -868,6 +883,17 @@ def nerfle_render_samples(first: PackedMLP, second: PackedMLP, rays_or_cam, ts: 
     sigma = torch.empty((R, S), dtype=torch.float32, device=dev)
     rgb = torch.empty((R, S, 3), dtype=torch.float32, device=dev)
     cs = ctypes.byref(cam.struct) if cam is not None else None
+    if occupancy is not None or samples_done is not None:
+        with torch.cuda.device(dev):
+            c1, c2 = first.c_struct(prec), second.c_struct(prec)
+            g, sd = _occ_args(occupancy, samples_done)
+            ws = _cached_ws(_ws_cache, dev, N.lib().nrt_nerfle_render_samples_occupancy_workspace(
+                ctypes.byref(c1), ctypes.byref(c2), prec, R, S, cs))
+            N.check(N.lib().nrt_nerfle_render_samples_occupancy(
+                ctypes.byref(c1), ctypes.byref(c2), prec, _ptr(r2), cs, R, None if per_ray else _ptr(t),
+                _ptr(t) if per_ray else None, S, _ptr(lc), lc.shape[-1], _ptr(vor), g, _ptr(sd), _ptr(sigma), _ptr(rgb),
+                _ptr(ws), ws.numel(), _stream()))
+        return sigma, rgb
     with torch.cuda.device(dev):
         c1, c2 = first.c_struct(prec), second.c_struct(prec)
         ws = _cached_ws(_ws_cache, dev, N.lib().nrt_nerfle_render_samples_workspace(ctypes.byref(c1), ctypes.byref(c2), prec,
@@ -897,6 +923,117 @@ def nerfle_render_camera_host(first: PackedMLP, second: PackedMLP, cam: CameraDe
             ctypes.c_void_p(ts_host.data_ptr()) if ts_host is not None else None, S, ctypes.byref(samp), _ptr(lc),
             lc.shape[-1], ctypes.c_void_p(out_host.data_ptr()), _stream()))
     return out_host
+
+
+# ---- occupancy grid: empty-space skipping for the gradient-free NeRFLE render (nrt_occupancy_*) ----------------------
+OCC_MIN_RES, OCC_MAX_RES, OCC_MAX_POINTS_PER_CELL = 16, 512, 4096   # NRT_OCC_MIN_RES, NRT_OCC_MAX_RES, ..._POINTS_PER_CELL
+
+
+def occupancy_words(res: int) -> int:
+    """Length of the bit words of a res^3 grid: ceil(res^3 / 32)."""
+    return (int(res) ** 3 + 31) // 32
+
+
+def check_occupancy_args(res, bbox_min, bbox_max, threshold=0.0, decay=0.0, points_per_cell=1):
+    """The grid's argument checks, on the host (the library repeats them)."""
+    import math
+    if isinstance(res, bool) or not isinstance(res, int) or not OCC_MIN_RES <= res <= OCC_MAX_RES:
+        raise NrtError("occupancy resolution must be an int in [%d, %d], got %r" % (OCC_MIN_RES, OCC_MAX_RES, res))
+    lo, hi = [float(v) for v in bbox_min], [float(v) for v in bbox_max]
+    if len(lo) != 3 or len(hi) != 3:
+        raise NrtError("bbox_min / bbox_max must have 3 entries")
+    for a in range(3):
+        if not (math.isfinite(lo[a]) and math.isfinite(hi[a]) and hi[a] > lo[a]):
+            raise NrtError("the occupancy box must be finite with bbox_max > bbox_min (axis %d: [%r, %r])" % (a, lo[a], hi[a]))
+    if not (math.isfinite(float(threshold)) and float(threshold) >= 0.0):
+        raise NrtError("threshold must be finite and >= 0, got %r" % (threshold,))
+    if not (0.0 <= float(decay) <= 1.0):
+        raise NrtError("decay must be in [0, 1], got %r" % (decay,))
+    if isinstance(points_per_cell, bool) or not isinstance(points_per_cell, int) or \
+            not 1 <= points_per_cell <= OCC_MAX_POINTS_PER_CELL:
+        raise NrtError("points_per_cell must be an int in [1, %d], got %r" % (OCC_MAX_POINTS_PER_CELL, points_per_cell))
+    return lo, hi
+
+
+def occupancy_struct(res, bbox_min, bbox_max, bits: Optional[torch.Tensor]) -> N.NrtOccupancy:
+    """nrt_occupancy_t of a res^3 grid over [bbox_min, bbox_max] with its bit words (int32 / uint32 CUDA tensor)."""
+    lo, hi = check_occupancy_args(res, bbox_min, bbox_max)
+    if bits is not None:
+        if not bits.is_cuda:
+            raise NrtError("occupancy bits must be a CUDA tensor (there is no CPU path)")
+        if bits.dtype not in (torch.int32, torch.uint32) or not bits.is_contiguous() or bits.numel() != occupancy_words(res):
+            raise NrtError("occupancy bits must be a contiguous int32 tensor of %d words" % occupancy_words(res))
+    return N.NrtOccupancy(int(res), (ctypes.c_float * 3)(*lo), (ctypes.c_float * 3)(*hi), _ptr(bits))
+
+
+def _occ_args(occupancy, samples_done):
+    g = None
+    if occupancy is not None:
+        g = ctypes.byref(occupancy_struct(occupancy.res, occupancy.bbox_min, occupancy.bbox_max, occupancy.bits))
+    sd = None
+    if samples_done is not None:
+        sd = _chk(samples_done, "samples_done", torch.int64)
+        if sd.numel() != 1:
+            raise NrtError("samples_done must hold one int64")
+    return g, sd
+
+
+def _render_occupancy(first, second, prec, r2, cam, R, t, samp, lc, vor, occupancy, samples_done, out):
+    dev = out.device
+    cs = ctypes.byref(cam.struct) if cam is not None else None
+    with torch.cuda.device(dev):
+        c1, c2 = first.c_struct(prec), second.c_struct(prec)
+        g, sd = _occ_args(occupancy, samples_done)
+        ws = _cached_ws(_ws_cache, dev, N.lib().nrt_nerfle_render_occupancy_workspace(
+            ctypes.byref(c1), ctypes.byref(c2), prec, R, cs, ctypes.byref(samp)))
+        N.check(N.lib().nrt_nerfle_render_occupancy(
+            ctypes.byref(c1), ctypes.byref(c2), prec, _ptr(r2), cs, R, _ptr(t), ctypes.byref(samp), _ptr(lc), lc.shape[-1],
+            _ptr(vor), g, _ptr(sd), _ptr(out), _ptr(ws), ws.numel(), _stream()))
+    return out
+
+
+_occ_ws_cache = {}
+
+
+def occupancy_update(first: PackedMLP, res: int, bbox_min, bbox_max, density: torch.Tensor, bits: torch.Tensor,
+                     points_per_cell=4, decay=0.0, threshold=0.01, seed=0, prec=PREC_F32):
+    """In place: density [res^3] = max(decay * density, max over points_per_cell points of every cell of relu(sigma_raw)),
+    bits [ceil(res^3 / 32)] = density > threshold (nrt_occupancy_update; sigma_raw = column 0 of `first` at `prec`).
+    seed 0 evaluates the cell centres, another seed jittered points."""
+    prec = prec_id(prec)
+    check_occupancy_args(res, bbox_min, bbox_max, threshold, decay, points_per_cell)
+    d = _chk(density, "density")
+    if density.numel() != int(res) ** 3 or not density.is_contiguous():
+        raise NrtError("density must be a contiguous float32 tensor of res^3 = %d cells" % int(res) ** 3)
+    g = occupancy_struct(res, bbox_min, bbox_max, bits)
+    if not isinstance(seed, int) or not 0 <= seed < 2 ** 64:
+        raise NrtError("seed must be an int in [0, 2^64)")
+    with torch.cuda.device(d.device):
+        c = first.c_struct(prec)
+        nbytes = N.lib().nrt_occupancy_update_workspace(ctypes.byref(c), prec, int(res), int(points_per_cell))
+        ws = _cached_ws(_occ_ws_cache, d.device, nbytes)
+        N.check(N.lib().nrt_occupancy_update(ctypes.byref(c), prec, ctypes.byref(g), int(points_per_cell), float(decay),
+                                             float(threshold), int(seed), _ptr(d), _ptr(bits), _ptr(ws), ws.numel(),
+                                             _stream()))
+    return density, bits
+
+
+def occupancy_mask(occupancy, rays: torch.Tensor, ts: torch.Tensor) -> torch.Tensor:
+    """The cull decision alone (nrt_occupancy_mask, the device function the render uses): rays [...,6], ts [S] (shared)
+    or [R,S] (per ray) -> keep [R,S] bool, True = kept (outside the box, non-finite, or in an occupied cell)."""
+    r2 = _chk(rays, "rays").reshape(-1, 6)
+    R = r2.shape[0]
+    t = _chk(ts, "ts")
+    per_ray = t.dim() == 2
+    if per_ray and t.shape[0] != R:
+        raise NrtError("ts [R,S] has %d rows for %d rays" % (t.shape[0], R))
+    S = t.shape[-1] if per_ray else t.numel()
+    keep = torch.empty((R, S), dtype=torch.uint8, device=r2.device)
+    with torch.cuda.device(r2.device):
+        g, _ = _occ_args(occupancy, None)
+        N.check(N.lib().nrt_occupancy_mask(g, _ptr(r2), R, None if per_ray else _ptr(t), _ptr(t) if per_ray else None, S,
+                                           _ptr(keep), _stream()))
+    return keep.bool()
 
 
 # ---- meshes: a SphereSDF on a lattice, isosurface extraction (nrt_sdf_lattice_eval, nrt_isosurface_*) --------------

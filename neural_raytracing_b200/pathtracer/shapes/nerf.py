@@ -111,6 +111,74 @@ class HierarchicalSampling:
             self.n_coarse, self.n_fine, self.t_near, self.t_far, self.jitter)
 
 
+class OccupancyGrid:
+    """Empty-space skipping for NeRFLE's gradient-free renders (an extension; the reference evaluates both MLPs at every
+    sample).  A cube of res^3 cells over [bbox_min, bbox_max]; cell (i,j,k) is entry (i * res + j) * res + k of `density`
+    (fp32 [res^3], i.e. a torch [res,res,res] tensor in C order) and bit c & 31 of word c >> 5 of `bits` (int32
+    [ceil(res^3 / 32)], the library's uint32 words) is set iff density[c] > threshold.
+
+    `update(model)` evaluates model.first at `points_per_cell` points of every cell (seed 0: the cell centres; otherwise
+    jittered by the library's counter hash) at the current config.precision and sets
+    density = max(decay * density, max over the points of relu(sigma_raw)), then the bits (decay = 0 rebuilds).
+
+    Assign the grid to `NeRFLE.occupancy`.  Gradient-free renders (forward under no_grad, render_camera, pathtrace's
+    frames) then write sigma = 0, rgb = 0 at every sample whose point lies in the box and in a cell with a clear bit, and
+    run both MLPs on the other samples only; samples outside the box are always evaluated.  Because the compositing
+    uses relu(sigma), such a sample contributes exactly nothing: with every bit set the image is bit-identical to the
+    render without a grid.  Training (the differentiable forward) ignores the grid.  Culling runs on the tensor-core
+    precisions (f16 / bf16): a render at "f32" with a grid raises NrtError.
+
+    The grid remembers which weights of model.first it was built from (the packed blob's data_ptr and version); a render
+    after they changed raises until `update` is called again.  training.GraphedStep replays do not bump tensor versions:
+    call `update` after them.  The grid is not part of state_dict: rebuilding it is one `update` call."""
+
+    def __init__(self, resolution=128, bbox_min=(-1.5, -1.5, -1.5), bbox_max=(1.5, 1.5, 1.5), threshold=0.01,
+                 device="cuda"):
+        res = resolution
+        if isinstance(res, bool) or not isinstance(res, int):
+            raise ValueError("OccupancyGrid: resolution must be an int, got %r" % (res,))
+        try:
+            lo, hi = ops.check_occupancy_args(res, bbox_min, bbox_max, threshold)
+        except ops.NrtError as e:
+            raise ValueError("OccupancyGrid: %s" % e) from None
+        self.res, self.bbox_min, self.bbox_max, self.threshold = res, tuple(lo), tuple(hi), float(threshold)
+        self.density = torch.zeros(res ** 3, dtype=torch.float32, device=device)
+        self.bits = torch.zeros(ops.occupancy_words(res), dtype=torch.int32, device=device)
+        self._key = None      # model.first's pack key at the last update
+
+    def update(self, model, points_per_cell=4, decay=0.0, seed=1):
+        """Re-evaluates the density of every cell with model.first (see the class docstring).  Returns self."""
+        if isinstance(seed, bool) or not isinstance(seed, int) or not 0 <= seed < 2 ** 64:
+            raise ValueError("OccupancyGrid.update: seed must be an int in [0, 2^64), got %r" % (seed,))
+        try:
+            ops.check_occupancy_args(self.res, self.bbox_min, self.bbox_max, self.threshold, decay, points_per_cell)
+        except ops.NrtError as e:
+            raise ValueError("OccupancyGrid.update: %s" % e) from None
+        first = model.first
+        prec = config.precision if first.precision() != "f32" else "f32"
+        with torch.no_grad():
+            ops.occupancy_update(first.packed(), self.res, self.bbox_min, self.bbox_max, self.density, self.bits,
+                                 points_per_cell=points_per_cell, decay=float(decay), threshold=self.threshold,
+                                 seed=seed, prec=prec)
+        self._key = first._pack_key
+        return self
+
+    def check_current(self, first):
+        """Raises NrtError unless the grid was built from first's current weights (call after first.packed())."""
+        if self._key is None:
+            raise ops.NrtError("OccupancyGrid: never updated -- call grid.update(model) before rendering with it")
+        if first._pack_key != self._key:
+            raise ops.NrtError("OccupancyGrid: model.first changed since the last update -- call grid.update(model)")
+
+    def occupied_fraction(self) -> float:
+        """Share of the cells whose bit is set."""
+        return float((self.density > self.threshold).sum().item()) / self.res ** 3
+
+    def __repr__(self):
+        return "OccupancyGrid(resolution=%d, bbox_min=%r, bbox_max=%r, threshold=%g)" % (
+            self.res, self.bbox_min, self.bbox_max, self.threshold)
+
+
 class _NerfleFused(torch.autograd.Function):
     """first MLP -> [latent | r_d | light] -> second MLP -> sigmoid on the tensor-core training kernels, nothing but
     sigma [S,...] and rgb [S,...,3] materialised in fp32 (ops.nerfle_train_forward / _backward).  Gradients reach the
@@ -163,6 +231,9 @@ class NeRFLE(nn.Module):
         # optional HierarchicalSampling (not a constructor argument: the constructor keeps the reference's signature;
         # not in state_dict).  None: the reference's 64 shared uniform distances.
         self.sampling = None
+        # optional OccupancyGrid: gradient-free renders skip the samples in its empty cells (not a constructor argument,
+        # not in state_dict; training ignores it)
+        self.occupancy = None
 
     def _sample_ts(self, device):
         if getattr(self, "far_jitter", None) is not None:
@@ -205,6 +276,15 @@ class NeRFLE(nn.Module):
         s = self.sampling
         return dict(n_coarse=s.n_coarse, n_fine=s.n_fine, t_near=s.t_near, t_far=s.t_far, jitter_seed=s.render_seed)
 
+    def _render_occupancy(self):
+        """nerfle_render keyword argument of `occupancy` for a gradient-free render (checked against first's weights)."""
+        grid = getattr(self, "occupancy", None)
+        if grid is None:
+            return {}
+        self.first.packed()
+        grid.check_current(self.first)
+        return dict(occupancy=grid)
+
     def render_camera(self, cam, lights):
         """The frame of `cam` (ops.CameraDesc) in one library call, rays generated on the device inside it (f4):
         what pathtrace's tile loop + sample_positions + forward compute for an inference render (main.py:57-88,
@@ -216,10 +296,10 @@ class NeRFLE(nn.Module):
         prec = config.precision if self.first.precision() != "f32" and self.second.precision() != "f32" else "f32"
         if getattr(self, "sampling", None) is not None:
             return ops.nerfle_render_camera(self.first.packed(), self.second.packed(), cam, None, code.detach().float(),
-                                            prec=prec, **self._render_sampling())
+                                            prec=prec, **self._render_sampling(), **self._render_occupancy())
         ts = self._sample_ts(device)
         return ops.nerfle_render_camera(self.first.packed(), self.second.packed(), cam, ts, code.detach().float(),
-                                        prec=prec)
+                                        prec=prec, **self._render_occupancy())
 
     def forward(self, rays, lights):
         """nerf.py:175-214.  With `sampling` (a HierarchicalSampling) set, the samples are its stratified coarse +
@@ -227,7 +307,8 @@ class NeRFLE(nn.Module):
         random.random() is used: a gradient-free forward renders with sampling.render_seed; a differentiable one takes
         the merged distances from a no-grad coarse pass (at the train precision) seeded by the device tensor
         sampling.train_seed(), advances that seed by one, and trains both MLPs on all n_coarse + n_fine samples (the
-        light code is a constant there, as on the fused path)."""
+        light code is a constant there, as on the fused path).  With `occupancy` (an OccupancyGrid) set, a gradient-free
+        forward skips the samples in its empty cells; the differentiable forward ignores it, so training is unchanged."""
         if getattr(self, "sampling", None) is not None:
             return self._forward_hierarchical(rays, lights)
         r_o, r_d = rays.split([3, 3], dim=-1)
@@ -241,7 +322,7 @@ class NeRFLE(nn.Module):
             # other shape keeps the exact fp32 kernel (SkipConnMLP.precision() knows which shapes are instantiated)
             prec = config.precision if self.first.precision() != "f32" and self.second.precision() != "f32" else "f32"
             return ops.nerfle_render(self.first.packed(), self.second.packed(), rays.detach().float(), ts,
-                                     code.detach().float(), view, prec=prec)
+                                     code.detach().float(), view, prec=prec, **self._render_occupancy())
         # differentiable path: fused MLP kernels where available + CUDA compositing
         tprec = self.first.train_precision()
         if rays.is_cuda and tprec != "f32" and self.second.train_precision() == tprec and not rays.requires_grad \
@@ -270,7 +351,7 @@ class NeRFLE(nn.Module):
         if not self._needs_grad(rays):
             prec = config.precision if self.first.precision() != "f32" and self.second.precision() != "f32" else "f32"
             return ops.nerfle_render(self.first.packed(), self.second.packed(), rays.detach().float(), None, code, view,
-                                     prec=prec, **self._render_sampling())
+                                     prec=prec, **self._render_sampling(), **self._render_occupancy())
         tprec = self.first.train_precision()
         fused = tprec != "f32" and self.second.train_precision() == tprec and not rays.requires_grad
         seed = s.train_seed(rays.device)

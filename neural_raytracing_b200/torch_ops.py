@@ -320,16 +320,35 @@ def _(rays, centers, radii, tfs, params, basis, arch, step, n_steps, prec):
 
 
 # ---- a18: NeRFLE volumetric render ------------------------------------------------------------------------------
+class _Grid:
+    """The occupancy grid of an operator's trailing arguments (occ_bits None: no grid)."""
+
+    def __init__(self, bits, res, bbox_min, bbox_max):
+        self.bits, self.res, self.bbox_min, self.bbox_max = bits, int(res), bbox_min, bbox_max
+
+
+def _grid(occ_bits: Optional[Tensor], occ_res: int, occ_bbox_min: Optional[List[float]], occ_bbox_max: Optional[List[float]]):
+    if occ_bits is None:
+        return None
+    if occ_bbox_min is None or occ_bbox_max is None:
+        raise ops.NrtError("an occupancy grid needs occ_bbox_min and occ_bbox_max")
+    return _Grid(occ_bits, occ_res, occ_bbox_min, occ_bbox_max)
+
+
 @torch.library.custom_op(NS + "::nerfle_render", mutates_args=())
 def nerfle_render(rays: Tensor, ts: Tensor, light_code: Tensor, params1: Tensor, basis1: Tensor, arch1: List[int],
-                  params2: Tensor, basis2: Tensor, arch2: List[int], prec: int) -> Tensor:
-    """NeRFLE.forward (nerf.py:175-214) for one view / light code: rays [R,6], ts [S] -> rgb [R,3] (gradient-free)."""
+                  params2: Tensor, basis2: Tensor, arch2: List[int], prec: int, occ_bits: Optional[Tensor] = None,
+                  occ_res: int = 0, occ_bbox_min: Optional[List[float]] = None,
+                  occ_bbox_max: Optional[List[float]] = None) -> Tensor:
+    """NeRFLE.forward (nerf.py:175-214) for one view / light code: rays [R,6], ts [S] -> rgb [R,3] (gradient-free).
+    occ_bits (int32 words of a res^3 grid over [occ_bbox_min, occ_bbox_max]): cull the samples in empty cells (f16 / bf16)."""
     return ops.nerfle_render(_mlp(params1, basis1, arch1), _mlp(params2, basis2, arch2), rays, ts, light_code,
-                             prec=prec).reshape(-1, 3)
+                             prec=prec, occupancy=_grid(occ_bits, occ_res, occ_bbox_min, occ_bbox_max)).reshape(-1, 3)
 
 
 @nerfle_render.register_fake
-def _(rays, ts, light_code, params1, basis1, arch1, params2, basis2, arch2, prec):
+def _(rays, ts, light_code, params1, basis1, arch1, params2, basis2, arch2, prec, occ_bits=None, occ_res=0, occ_bbox_min=None,
+      occ_bbox_max=None):
     return rays.new_empty((rays.reshape(-1, 6).shape[0], 3))
 
 
@@ -375,17 +394,39 @@ def _(kind, a, b, focal, size, x0, y0, nx, ny, bundle, positions, jitter, jitter
 def nerfle_render_camera(kind: int, a: Tensor, b: Optional[Tensor], focal: float, size: float, x0: int, y0: int, nx: int,
                          ny: int, bundle: int, jitter: float, jitter_seed: int, ts: Tensor, light_code: Tensor,
                          params1: Tensor, basis1: Tensor, arch1: List[int], params2: Tensor, basis2: Tensor,
-                         arch2: List[int], prec: int) -> Tensor:
+                         arch2: List[int], prec: int, occ_bits: Optional[Tensor] = None, occ_res: int = 0,
+                         occ_bbox_min: Optional[List[float]] = None, occ_bbox_max: Optional[List[float]] = None) -> Tensor:
     """The frame of a NeRFLE from its camera in one call, rays generated on the device inside the library (f4; what pathtrace
-    + NeRFReproduce compute, main.py:57-88 + nerf.py:175-214) -> rgb [n_views, nx, ny, bundle, 3] (gradient-free)."""
+    + NeRFReproduce compute, main.py:57-88 + nerf.py:175-214) -> rgb [n_views, nx, ny, bundle, 3] (gradient-free).
+    occ_*: an occupancy grid, as in nerfle_render."""
     cam = _cam(kind, a, b, focal, size, x0, y0, nx, ny, bundle, None, jitter, jitter_seed)
-    return ops.nerfle_render_camera(_mlp(params1, basis1, arch1), _mlp(params2, basis2, arch2), cam, ts, light_code, prec=prec)
+    return ops.nerfle_render_camera(_mlp(params1, basis1, arch1), _mlp(params2, basis2, arch2), cam, ts, light_code, prec=prec,
+                                    occupancy=_grid(occ_bits, occ_res, occ_bbox_min, occ_bbox_max))
 
 
 @nerfle_render_camera.register_fake
 def _(kind, a, b, focal, size, x0, y0, nx, ny, bundle, jitter, jitter_seed, ts, light_code, params1, basis1, arch1, params2,
-      basis2, arch2, prec):
+      basis2, arch2, prec, occ_bits=None, occ_res=0, occ_bbox_min=None, occ_bbox_max=None):
     return a.new_empty((a.shape[0], nx, ny, bundle, 3))
+
+
+# ---- occupancy grid of a NeRFLE density network (extension; nrt_occupancy_update) -----------------------------------
+@torch.library.custom_op(NS + "::occupancy_update", mutates_args=())
+def occupancy_update(density: Tensor, bits: Tensor, params1: Tensor, basis1: Tensor, arch1: List[int], res: int,
+                     bbox_min: List[float], bbox_max: List[float], points_per_cell: int, decay: float, threshold: float,
+                     seed: int, prec: int) -> Tuple[Tensor, Tensor]:
+    """The grid after one update with NeRFLE.first (gradient-free): density [res^3] -> max(decay * density, max over
+    points_per_cell points of every cell of relu(sigma_raw)), bits [ceil(res^3 / 32)] int32 = density > threshold.
+    Returns new tensors; the inputs are not modified."""
+    d, b = density.clone(), bits.clone()
+    ops.occupancy_update(_mlp(params1, basis1, arch1), res, bbox_min, bbox_max, d, b, points_per_cell=points_per_cell,
+                         decay=decay, threshold=threshold, seed=seed, prec=prec)
+    return d, b
+
+
+@occupancy_update.register_fake
+def _(density, bits, params1, basis1, arch1, res, bbox_min, bbox_max, points_per_cell, decay, threshold, seed, prec):
+    return torch.empty_like(density), torch.empty_like(bits)
 
 
 # ---- meshes: isosurface of a lattice (extension; the reference has no mesh output) ----------------------------------
@@ -405,4 +446,4 @@ def _(values, origin, spacing, level):
 
 OPERATORS = ["camera_rays", "nerfle_render_camera", "mlp_forward", "mlp_backward", "mlp_forward_train_tc", "mlp_backward_tc", "composite", "composite_backward", "mlp_value_jac", "mlp_value_jac_backward",
              "sdf_eval", "sdf_sphere_trace", "sdf_shadow_test", "sdf_min_scan", "nerfle_render", "composite_ts",
-             "composite_ts_backward", "nerfle_sample_hierarchical", "isosurface"]
+             "composite_ts_backward", "nerfle_sample_hierarchical", "isosurface", "occupancy_update"]
